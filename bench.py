@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # native arm (this repo's CUDA path), config c2
     python bench.py --impl reference --gpus N --steps K ...  # reference arm: CPU port of the reference loop
     python bench.py --config {c1,c2,c3,c4,sweep} ...         # the other BASELINE.json configs (same JSON contract)
+    python bench.py ... --dump-outputs DIR                    # also write the last timed step's outputs as DIR/<name>.npy
 
 One "step" = one pass of the hot path over the population of the chosen config on each GPU:
 act (actor forward) -> OU noise + clip -> Platoon.step -> ReplayBuffer.add for every agent -> replay sample (64 per ring) ->
@@ -181,11 +182,17 @@ def build_trainer(cfg, rank, world, precision, pg, ring_cap=None):
         # (trainer.py:640-641: 10 x 600 steps), far beyond a benchmark run, and are covered by tests/test_gpu_ddpg.py
         kw.update(fed_method="interfrl", weighted_average_enabled=False)
     conf = Config(**kw)
-    free, _ = torch.cuda.mem_get_info()
+    # sized from the device's total memory, not from what happens to be free, so that the same arguments give the same ring (and the
+    # same sampled inputs) on every run; a ring above half of the device's memory is shrunk to 35 % of it (the JSON line reports it)
+    total = torch.cuda.get_device_properties(torch.cuda.current_device()).total_memory
     cap = RING_CAP if ring_cap is None else ring_cap
     per_slot = M * G * E * 40
-    if cap * per_slot > 0.5 * free:      # never drive the box out of memory: shrink the ring and say so
-        cap = int(0.35 * free / per_slot)
+    if cap * per_slot > 0.5 * total:
+        cap = int(0.35 * total / per_slot)
+    free, _ = torch.cuda.mem_get_info()
+    if cap * per_slot > free:
+        raise RuntimeError(f"the {cap}-slot replay ring needs {cap * per_slot / 1e9:.1f} GB, but only {free / 1e9:.1f} GB of device memory "
+                           "are free (the ring is sized for a device the benchmark has to itself)")
     tr = BatchedTrainer(conf, num_groups=G, envs_per_group=E, ring_capacity=cap, rank=rank, world=world,
                         process_group=pg if cfg["fed"] else None, precision=precision)
     if E >= 64:
@@ -270,6 +277,27 @@ def env_host_leg(M, P, steps):
             "reward + done, stream sync) on pinned host buffers"}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(tr, out_dir):
+    """Write what the last training step handed its caller to out_dir/<name>.npy (float32): the observations, rewards and done flags
+    of every platoon, the applied (OU-perturbed, clipped) actions, the learn losses and local gradients, and the weights of the four
+    networks of every agent.  Two builds run with the same arguments see the same inputs, so their files compare one to one."""
+    import numpy as np
+    env, pop = tr.env, tr.pop
+    arrays = {"obs": env.obs, "reward": env.reward, "done": env.done, "action": env.action_out.t(), "loss": pop.loss,
+              "actor_grad": pop.actor.grad, "critic_grad": pop.critic.grad, "actor": pop.actor.flat, "critic": pop.critic.flat,
+              "target_actor": pop.t_actor.flat, "target_critic": pop.t_critic.flat}
+    arrays = {k: v.float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total / 2**20:.1f} MB of outputs exceed the {DUMP_LIMIT_BYTES >> 20} MB limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def run_native(args):
     import torch
     rank, world, local = _dist_setup()
@@ -294,7 +322,7 @@ def run_native(args):
     graph = (cfg["graph"] or args.graph) and not args.eager and (tr.fed is None or tr.fed.graph_safe)
     if graph:
         tr.capture(warmup=1)
-    K = max(1, args.steps)
+    K = args.steps
 
     def run_steps():                 # EXACTLY K steps: K // 2 replays (+ one eager step when K is odd)
         if graph:
@@ -316,6 +344,8 @@ def run_native(args):
     if graph:      # replays do not pass through the launch sites: kernels per captured step x replayed steps (+ the eager one)
         launches += (K // 2) * 2 * tr.kernels_per_step
     value = world * P * M / (ms_step * 1e-3)
+    if args.dump_outputs and rank == 0:      # before the legs below move the state on
+        dump_outputs(tr, args.dump_outputs)
 
     # ---- attribution: env part (act + env step + replay add), learn part (sample + learn), FRL round (reduce + fused consumer)
     def env_part():
@@ -490,7 +520,7 @@ def run_sweep(args, rank, world, local):
             for train in (False, True):
                 if train and P * M > (1 << 25):      # 4-slot ring = 160 B per vehicle: keep the sweep far from the HBM capacity
                     continue
-                rl = time_env_roofline(P, M, train, steps=max(10, min(args.steps, 30)), warmup=max(3, args.warmup))
+                rl = time_env_roofline(P, M, train, steps=args.steps, warmup=max(3, args.warmup))
                 ms = _max_over_ranks(rl["avg_ms"], world)
                 gbs = rl["alg_bytes"] / (ms * 1e-3) / 1e9
                 pts.append({"platoons_per_gpu": P, "followers": M, "mode": "train" if train else "plain", "us": ms * 1e3,
@@ -504,7 +534,7 @@ def run_sweep(args, rank, world, local):
                           "vs_baseline": None, "dtype": "f32", "data": "synthetic", "impl": "native",
                           "config": {"workload": "sweep: env-step kernel, 2^10..2^24 platoons x {4, 8} followers per GPU, plain (48 B/vehicle-step) "
                                                  "and training launch (112 B/vehicle-step) vs the HBM roofline"},
-                          "clocks": clk.summary(), "gpu_launches": len(pts) * (max(10, min(args.steps, 30)) + max(3, args.warmup)),
+                          "clocks": clk.summary(), "gpu_launches": len(pts) * (args.steps + max(3, args.warmup)),
                           "roofline": {"bound": "hbm", "kernel": "env_step_kernel (training launch, best point)", "achieved": best["alg_GBps_per_gpu"],
                                        "peak": pk["hbm"], "unit": "GB/s", "frac": best["frac_of_hbm"], "traffic": None, "peak_source": pk["src"]},
                           "best_plain": bestp, "best_train": best, "points": pts, "e2e": None, "cpu_baseline": None}))
@@ -523,7 +553,7 @@ def run_reference(args):
         return
     from oracle import cpu_baseline
     cfg = CONFIGS[args.config if args.config in CONFIGS else "c2"]
-    total = max(1, args.steps)
+    total = args.steps
     budget = max(0.25, min(args.cpu_seconds, 150.0 / (total + args.warmup)))
     pool = cpu_baseline.EnvLoopPool(M=cfg["M"], with_learn=True)
     vals, steps, slowest = [], 0, 0.0
@@ -558,7 +588,14 @@ def main():
                     help="learn kernels: 0 fp32 SIMT (parity mode), 1 bf16 tcgen05, 2 fp16 tcgen05 (default; DESIGN.md section 4)")
     ap.add_argument("--graph", action="store_true", help="replay a captured CUDA graph of the training step (the default of every config)")
     ap.add_argument("--eager", action="store_true", help="launch the training step kernel by kernel instead of replaying its CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (observations, rewards, done flags, actions, losses, "
+                         "gradients, weights) to DIR/<name>.npy (rank 0; configs c1-c4)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.config == "sweep"):
+        ap.error("--dump-outputs needs the native training step (configs c1-c4)")
     if args.impl == "reference":
         run_reference(args)
     else:
