@@ -11,7 +11,7 @@ import os
 
 AVD_MAX_FOLLOWERS = 16
 RING_RECORD_FLOATS = 10
-ABI_VERSION = 2
+ABI_VERSION = 3
 
 RNG_RESET_VEHICLE, RNG_RESET_PLATOON, RNG_OU, RNG_LEADER_EXOG, RNG_REPLAY, RNG_INIT = range(6)
 
@@ -135,6 +135,7 @@ SIGNATURES = {
     "avd_replay_fill_synthetic": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_uint64, C.c_void_p]),
     "avd_ddpg_param_counts": (C.c_int, [C.POINTER(NetDims), C.POINTER(C.c_int64)]),
     "avd_ddpg_workspace_bytes": (C.c_int64, [C.POINTER(NetDims), C.c_int32, C.c_int64, C.c_int32]),
+    "avd_forward_workspace_bytes": (C.c_int64, [C.POINTER(NetDims), C.c_int32, C.c_int64, C.c_int32, C.c_int32]),
     "avd_ddpg_learn": (C.c_int, [C.POINTER(LearnIO), C.c_void_p]),
     "avd_actor_forward": (C.c_int, [C.POINTER(NetDims), C.c_int32, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64,
                                     C.c_float, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p]),
@@ -163,6 +164,8 @@ SIGNATURES = {
                                 C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p]),
     "avd_gemm_f16kind": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64,
                                    C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "avd_gemm_bf16x3": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64,
+                                  C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p]),
     "avd_rng_words": (C.c_int, [C.c_void_p, C.c_int64, C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint64, C.c_void_p]),
     "avd_rng_normals": (C.c_int, [C.c_void_p, C.c_int64, C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint64, C.c_void_p]),
 }

@@ -11,7 +11,8 @@
 // The three big contractions (forward, wgrad, dgrad on the l1 x l2 and (l1+la) x l2 layers, 97% of the FLOPs)
 // go through `gemm_batched`, which dispatches on io->precision: 0 = fp32 SIMT tiles (parity mode, this
 // file), 1 = bf16 tcgen05/TMEM tensor-core kernels, 2 = the same kernels with fp16 layer-2 operands (11-bit significand;
-// the backward tile stays bf16) and the T formulation of the critic-action pass (avd_fused3.cu).  Everything else (K=ns and K=1 layers,
+// the backward tile stays bf16) and the T formulation of the critic-action pass (avd_fused3.cu), 3 = the unfused tcgen05 GEMMs on
+// three-way split bf16 operands (umma::gemm_bf16x3: hi / mid / lo planes, fp32-accurate).  Everything else (K=ns and K=1 layers,
 // heads with N=1, BatchNorm affine, reductions for bias/BN gradients, TD target, losses) is fused into the
 // layer1 / head kernels below.
 //
@@ -58,10 +59,36 @@ int run(bool f16, int A, int64_t R, int F, const bf16* DZ, const bf16* W2b, cons
 namespace umma {   // avd_umma.cu
 int gemm_bf16(int layout, int batch, int M, int N, int K, const void* A, int64_t lda, int64_t a_batch, const void* B, int64_t ldb,
               int64_t b_batch, float* C, int64_t ldc, int64_t c_batch, int splitk, cudaStream_t st);
+int gemm_bf16x3(int layout, int batch, int M, int N, int K, const void* A, int64_t lda, int64_t a_batch, const void* B, int64_t ldb,
+                int64_t b_batch, float* C, int64_t ldc, int64_t c_batch, int splitk, cudaStream_t st);
+}
+
+// GEMM operand written as three bf16 planes (precision 3): element i is hi at p[i], mid at p[plane + i], lo at p[2 plane + i],
+// hi = bf16(x), mid = bf16(x - hi), lo = bf16(x - hi - mid).  Both differences are exact in fp32, so hi + mid + lo keeps 24 bits of x.
+// Behaves like an output pointer (offset, null test) so that the producers take it in place of float* / bf16*.
+struct Planes3 {
+    bf16* p;
+    int64_t plane;
+    __host__ __device__ Planes3 operator+(int64_t i) const { return Planes3{p + i, plane}; }
+    __host__ __device__ explicit operator bool() const { return p != nullptr; }
+};
+
+__device__ __forceinline__ void split3(float x, bf16& hi, bf16& mid, bf16& lo) {
+    hi = __float2bfloat16_rn(x);
+    const float r = x - __bfloat162float(hi);
+    mid = __float2bfloat16_rn(r);
+    lo = __float2bfloat16_rn(r - __bfloat162float(mid));
 }
 
 __device__ __forceinline__ void store_out(float* p, float v) { *p = v; }
 __device__ __forceinline__ void store_out(bf16* p, float v) { *p = __float2bfloat16_rn(v); }
+__device__ __forceinline__ void store_out(Planes3 o, float v) {
+    bf16 h, m, l;
+    split3(v, h, m, l);
+    o.p[0] = h;
+    o.p[o.plane] = m;
+    o.p[2 * o.plane] = l;
+}
 
 // ------------------------------------------------------------------------------------------------
 // layer 1: H[n][f] = bn(relu(x[n] . W[:,f] + b[f]))   (state columns, then -- critic -- action columns)
@@ -73,13 +100,21 @@ __device__ __forceinline__ void store_pair(float* p, float v0, float v1) { *rein
 __device__ __forceinline__ void store_pair(bf16* p, float v0, float v1) {
     *reinterpret_cast<__nv_bfloat162*>(p) = __floats2bfloat162_rn(v0, v1);
 }
+__device__ __forceinline__ void store_pair(Planes3 o, float v0, float v1) {
+    bf16 h0, m0, l0, h1, m1, l1;
+    split3(v0, h0, m0, l0);
+    split3(v1, h1, m1, l1);
+    *reinterpret_cast<__nv_bfloat162*>(o.p) = __halves2bfloat162(h0, h1);
+    *reinterpret_cast<__nv_bfloat162*>(o.p + o.plane) = __halves2bfloat162(m0, m1);
+    *reinterpret_cast<__nv_bfloat162*>(o.p + 2 * o.plane) = __halves2bfloat162(l0, l1);
+}
 
 // One thread owns a PAIR of adjacent columns (packed 4/8-byte stores, a warp writes 128/256 contiguous bytes per row);
-// l1 and la must be even so that a pair never straddles the state/action boundary.
+// l1 and la must be even so that a pair never straddles the state/action boundary.  TOut: float*, bf16* or Planes3.
 template <bool CRITIC, typename TOut>
 __global__ void __launch_bounds__(128) l1_forward_kernel(avd_net_dims d, const float* __restrict__ params, int64_t pstride,
                                                          const float* __restrict__ s, int64_t s_rs, int64_t s_cs,
-                                                         const float* __restrict__ act, int64_t R, TOut* __restrict__ H) {
+                                                         const float* __restrict__ act, int64_t R, TOut H) {
     const int agent = blockIdx.y;
     const float* P = params + (int64_t)agent * pstride;
     const int F = CRITIC ? d.l1 + d.la : d.l1;
@@ -290,13 +325,17 @@ struct HeadArgs {
     const float* y;        // CRITIC_BWD
     const float* dpi;      // ACTOR_BWD
     float* out;            // ACTOR_FWD: action, TARGET: y, Q/BWD: q (nullable for BWD)
-    void* DZ;              // BWD modes: float* (precision 0) or bf16* (precision 1)
+    void* DZ;              // BWD modes: float* (precision 0), bf16* (precision 1 / 2) or three bf16 planes (precision 3)
+    int64_t dz_plane;      // precision 3: elements per plane of DZ (all agents' rows)
     float* grads;          // [A][gstride] (BWD, ACTOR_BWD)
     int64_t gstride;
     float* loss;           // [A][2] nullable
 };
 
-template <int MODE, int CPL, typename TDZ>   // CPL = columns per lane (l2 = 32*CPL)
+template <typename T> __device__ __forceinline__ T dz_out(void* p, int64_t) { return reinterpret_cast<T>(p); }
+template <> __device__ __forceinline__ Planes3 dz_out<Planes3>(void* p, int64_t plane) { return Planes3{reinterpret_cast<bf16*>(p), plane}; }
+
+template <int MODE, int CPL, typename TDZ>   // CPL = columns per lane (l2 = 32*CPL); TDZ: float*, bf16* or Planes3
 __global__ void __launch_bounds__(256) head_kernel(HeadArgs h) {
     constexpr int L2 = 32 * CPL;
     constexpr int ROWS = 64;
@@ -359,7 +398,7 @@ __global__ void __launch_bounds__(256) head_kernel(HeadArgs h) {
             for (int j = 0; j < CPL; ++j) {
                 const float dh = dq * w3[j];
                 const float dz = z[j] > 0.0f ? dh * ginv[j] : 0.0f;
-                store_out(reinterpret_cast<TDZ*>(h.DZ) + n * L2 + lane + 32 * j, dz);
+                store_out(dz_out<TDZ>(h.DZ, h.dz_plane) + n * L2 + lane + 32 * j, dz);
                 if (BWD) {
                     aW3[j] = fmaf(hh[j], dq, aW3[j]);
                     aG[j] = fmaf(dh, (fmaxf(z[j], 0.0f) - mu[j]) * inv[j], aG[j]);
@@ -695,18 +734,19 @@ __global__ void __launch_bounds__(256) fed_broadcast_kernel(float* __restrict__ 
 
 // ------------------------------------------------------------------------------------------------
 // bf16 copies of the layer-2 kernels for the tensor-core path: W2b [F][l2] (dgrad B operand, K-major) and
-// W2T [l2][F] (forward B operand, K-major)
+// W2T [l2][F] (forward B operand, K-major); TOut = bf16* (precision 1 / 2) or Planes3 (precision 3)
 // ------------------------------------------------------------------------------------------------
+template <typename TOut>
 __global__ void __launch_bounds__(256) pack_w2_kernel(const float* __restrict__ params, int64_t pstride, int64_t oW2, int F, int l2,
-                                                      bf16* __restrict__ W2b, bf16* __restrict__ W2T) {
+                                                      TOut W2b, TOut W2T) {
     const int agent = blockIdx.y;
     const float* W = params + (int64_t)agent * pstride + oW2;
     const int n = F * l2;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
         const int f = i / l2, c = i - f * l2;
-        const bf16 v = __float2bfloat16_rn(W[i]);
-        if (W2b) W2b[(int64_t)agent * n + i] = v;
-        W2T[(int64_t)agent * n + (int64_t)c * F + f] = v;
+        const float v = W[i];
+        if (W2b) store_out(W2b + ((int64_t)agent * n + i), v);
+        store_out(W2T + ((int64_t)agent * n + (int64_t)c * F + f), v);
     }
 }
 
@@ -1139,7 +1179,7 @@ __global__ void __launch_bounds__(32 * kUnfoldWarps) unfold_kernel(const float* 
 // ------------------------------------------------------------------------------------------------
 struct Workspace {
     float *H, *H1a, *Z, *Za, *DZ, *DH, *a2, *y, *q, *dpi;
-    bf16 *cW2b, *cW2T, *tcW2T, *aW2b, *aW2T, *taW2T;   // packed weights (precision 1: bf16; precision 2: fp16)
+    bf16 *cW2b, *cW2T, *tcW2T, *aW2b, *aW2T, *taW2T;   // packed weights (precision 1: bf16; precision 2: fp16; precision 3: three bf16 planes)
     float* vtab;               // [A][fused3::vtab_floats()] V table + breakpoints of the critic-action pass
     float* wscale;             // precision 2: [2][A] 1 / s of the critic [0] and actor [1] W2'' / T packs
     uint32_t* mask2;           // [N][4] sign bits of the actor's z2 + b2' (MODE_ACTOR_SAVE -> actor_dm_kernel)
@@ -1159,36 +1199,40 @@ struct Workspace {
     static constexpr int kMaskWords = 10, kFp = 320, kG2Rows = 384;
     // fused: the persistent tensor-core kernels keep every activation on chip -- only the dz2 tile (DZ) of the fp32 activation
     // buffers exists then (C2: 0.9 GB instead of 5.4 GB of workspace, C4: 3.5 GB instead of 21 GB)
-    static int64_t bytes(const avd_net_dims& d, int64_t A, int64_t N, bool fused) {
+    // planes = 3 (precision 3): the GEMM operands H, H1a, DZ and the six weight packs hold three bf16 planes, 6 B per element
+    static int64_t bytes(const avd_net_dims& d, int64_t A, int64_t N, bool fused, int planes) {
         const int64_t F = d.l1 + d.la;
-        const int64_t acts = N * (fused ? (int64_t)d.l2 : 2 * F + d.l1 + 3 * (int64_t)d.l2) * (int64_t)sizeof(float);
-        const int64_t packed = A * (3 * F + 3 * (int64_t)d.l1) * d.l2 * (int64_t)sizeof(bf16) + (2 * A + 4 + A * (int64_t)fused3::vtab_floats()) * (int64_t)sizeof(float);
+        int64_t acts = N * (fused ? (int64_t)d.l2 : 2 * F + d.l1 + 3 * (int64_t)d.l2) * (int64_t)sizeof(float);
+        if (planes == 3) acts += N * (F + d.l1 + d.l2) * 2;
+        const int64_t packed = planes * A * (3 * F + 3 * (int64_t)d.l1) * d.l2 * (int64_t)sizeof(bf16) + (2 * A + 4 + A * (int64_t)fused3::vtab_floats()) * (int64_t)sizeof(float);
         const int64_t vecs = (5 + 4) * ((N + 3) / 4 * 4) * (int64_t)sizeof(float);
         const int64_t slices = std::max<int64_t>(A, sm_count());
         const int64_t fold = N * ((kMaskWords + 8) * 4 + 16 * 2) + A * (8 * (int64_t)d.l2 + 16) * (int64_t)sizeof(float) + A * 16 * 64 * 2 +
                              2 * slices * (kFp * 16 + kG2Rows * (int64_t)d.l2) * (int64_t)sizeof(float);
         return acts + packed + vecs + fold + 1024;
     }
-    void carve(void* base_, const avd_net_dims& d, int64_t A, int64_t N, bool fused) {
+    void carve(void* base_, const avd_net_dims& d, int64_t A, int64_t N, bool fused, int planes) {
         const int64_t F = d.l1 + d.la;
         float* p = reinterpret_cast<float*>(((uintptr_t)base_ + 255) & ~(uintptr_t)255);
+        // floats taken by a GEMM-operand buffer of n elements: fp32 / one 16-bit copy (planes = 1) or three bf16 planes
+        auto opnd = [planes](int64_t n) { return planes == 3 ? n * 3 / 2 : n; };
         H = DH = H1a = Z = Za = nullptr;
         if (!fused) {
-            H = p; p += N * F;
+            H = p; p += opnd(N * F);
             DH = p; p += N * F;
-            H1a = p; p += N * d.l1;
+            H1a = p; p += opnd(N * d.l1);
             Z = p; p += N * d.l2;
             Za = p; p += N * d.l2;
         }
-        DZ = p; p += N * d.l2;
+        DZ = p; p += opnd(N * d.l2);
         DZa = reinterpret_cast<bf16*>(DZ) + N * d.l2;
         bf16* b = reinterpret_cast<bf16*>(p);
-        cW2b = b; b += A * F * d.l2;
-        cW2T = b; b += A * F * d.l2;
-        tcW2T = b; b += A * F * d.l2;
-        aW2b = b; b += A * (int64_t)d.l1 * d.l2;
-        aW2T = b; b += A * (int64_t)d.l1 * d.l2;
-        taW2T = b; b += A * (int64_t)d.l1 * d.l2;
+        cW2b = b; b += planes * A * F * d.l2;
+        cW2T = b; b += planes * A * F * d.l2;
+        tcW2T = b; b += planes * A * F * d.l2;
+        aW2b = b; b += planes * A * (int64_t)d.l1 * d.l2;
+        aW2T = b; b += planes * A * (int64_t)d.l1 * d.l2;
+        taW2T = b; b += planes * A * (int64_t)d.l1 * d.l2;
         p = reinterpret_cast<float*>(((uintptr_t)b + 15) & ~(uintptr_t)15);
         wscale = p; p += (2 * A + 3) / 4 * 4;
         vtab = p; p += A * (int64_t)fused3::vtab_floats();
@@ -1223,35 +1267,40 @@ static int check_dims(const avd_net_dims* d, int precision = 0) {
     AVD_REQUIRE(d->ns >= 1 && d->ns <= 8, "ns=%d outside 1..8", d->ns);
     AVD_REQUIRE(d->l1 >= 4 && d->la >= 4 && d->l1 % 4 == 0 && d->la % 4 == 0 && d->la <= 64,
                 "layer sizes must be multiples of 4 and la <= 64 (l1=%d, la=%d)", d->l1, d->la);
-    AVD_REQUIRE(precision >= 0 && precision <= 2, "precision must be 0 (fp32 SIMT), 1 (bf16 tcgen05) or 2 (fp16 tcgen05)");
+    AVD_REQUIRE(precision >= 0 && precision <= 3, "precision must be 0 (fp32 SIMT), 1 (bf16 tcgen05), 2 (fp16 tcgen05) or 3 (split bf16 tcgen05)");
     if (d->l2 != 32 && d->l2 != 64 && d->l2 != 96 && d->l2 != 128) {
         set_error("layer2 size %d not supported (32, 64, 96 or 128)", d->l2);
         return AVD_ERR_UNSUPPORTED;
     }
     if (precision >= 1 && (d->l1 % 8 || d->la % 8 || d->l2 % 8)) {
-        set_error("precision 1 / 2 need layer sizes that are multiples of 8 (TMA 16-byte pitch)");
+        set_error("precision 1 / 2 / 3 need layer sizes that are multiples of 8 (TMA 16-byte pitch)");
         return AVD_ERR_UNSUPPORTED;
     }
     return AVD_OK;
 }
 
+template <int MODE, typename TDZ>
+static void launch_head_t(const HeadArgs& h, int l2, dim3 grid, cudaStream_t st) {
+    switch (l2 / 32) {
+        case 1: head_kernel<MODE, 1, TDZ><<<grid, 256, 0, st>>>(h); break;
+        case 2: head_kernel<MODE, 2, TDZ><<<grid, 256, 0, st>>>(h); break;
+        case 3: head_kernel<MODE, 3, TDZ><<<grid, 256, 0, st>>>(h); break;
+        default: head_kernel<MODE, 4, TDZ><<<grid, 256, 0, st>>>(h); break;
+    }
+}
+
+// prec: the learn step's precision, which decides the format of the backward tile DZ (fp32, one bf16 copy, or three bf16 planes)
 template <int MODE>
-static int launch_head(const HeadArgs& h, int l2, int A, cudaStream_t st, bool dz_bf16 = false) {
+static int launch_head(const HeadArgs& h, int l2, int A, cudaStream_t st, int prec = 0) {
     dim3 grid((unsigned)((h.R + 63) / 64), A);
-    if (dz_bf16) {
-        switch (l2 / 32) {
-            case 1: head_kernel<MODE, 1, bf16><<<grid, 256, 0, st>>>(h); break;
-            case 2: head_kernel<MODE, 2, bf16><<<grid, 256, 0, st>>>(h); break;
-            case 3: head_kernel<MODE, 3, bf16><<<grid, 256, 0, st>>>(h); break;
-            default: head_kernel<MODE, 4, bf16><<<grid, 256, 0, st>>>(h); break;
-        }
+    if (prec == 3) {
+        HeadArgs hp = h;
+        hp.dz_plane = (int64_t)A * h.R * l2;
+        launch_head_t<MODE, Planes3>(hp, l2, grid, st);
+    } else if (prec) {
+        launch_head_t<MODE, bf16*>(h, l2, grid, st);
     } else {
-        switch (l2 / 32) {
-            case 1: head_kernel<MODE, 1, float><<<grid, 256, 0, st>>>(h); break;
-            case 2: head_kernel<MODE, 2, float><<<grid, 256, 0, st>>>(h); break;
-            case 3: head_kernel<MODE, 3, float><<<grid, 256, 0, st>>>(h); break;
-            default: head_kernel<MODE, 4, float><<<grid, 256, 0, st>>>(h); break;
-        }
+        launch_head_t<MODE, float*>(h, l2, grid, st);
     }
     AVD_LAUNCH_OK();
     return AVD_OK;
@@ -1286,22 +1335,33 @@ struct Pass {
 
     dim3 l1_grid() const { return dim3((unsigned)((R + kL1Rows - 1) / kL1Rows), A); }
 
-    // layer 1 (+BN) of the actor (critic=false) or critic (true) into H ([N][F] fp32 or bf16)
+    // layer 1 (+BN) of the actor (critic=false) or critic (true) into H ([N][F] fp32, bf16, or three bf16 planes of N*F)
     int layer1(bool critic, const float* params, const float* s, int64_t s_rs, int64_t s_cs, const float* act, void* H) const {
         const int64_t ps = critic ? critic_off(d).total : actor_off(d).total;
-        if (prec) {
-            if (critic) l1_forward_kernel<true, bf16><<<l1_grid(), 128, 0, st>>>(d, params, ps, s, s_rs, s_cs, act, R, (bf16*)H);
-            else l1_forward_kernel<false, bf16><<<l1_grid(), 128, 0, st>>>(d, params, ps, s, s_rs, s_cs, act, R, (bf16*)H);
+        if (prec == 3) {
+            const Planes3 o{(bf16*)H, (int64_t)A * R * (critic ? d.l1 + d.la : d.l1)};
+            if (critic) l1_forward_kernel<true, Planes3><<<l1_grid(), 128, 0, st>>>(d, params, ps, s, s_rs, s_cs, act, R, o);
+            else l1_forward_kernel<false, Planes3><<<l1_grid(), 128, 0, st>>>(d, params, ps, s, s_rs, s_cs, act, R, o);
+        } else if (prec) {
+            if (critic) l1_forward_kernel<true, bf16*><<<l1_grid(), 128, 0, st>>>(d, params, ps, s, s_rs, s_cs, act, R, (bf16*)H);
+            else l1_forward_kernel<false, bf16*><<<l1_grid(), 128, 0, st>>>(d, params, ps, s, s_rs, s_cs, act, R, (bf16*)H);
         } else {
-            if (critic) l1_forward_kernel<true, float><<<l1_grid(), 128, 0, st>>>(d, params, ps, s, s_rs, s_cs, act, R, (float*)H);
-            else l1_forward_kernel<false, float><<<l1_grid(), 128, 0, st>>>(d, params, ps, s, s_rs, s_cs, act, R, (float*)H);
+            if (critic) l1_forward_kernel<true, float*><<<l1_grid(), 128, 0, st>>>(d, params, ps, s, s_rs, s_cs, act, R, (float*)H);
+            else l1_forward_kernel<false, float*><<<l1_grid(), 128, 0, st>>>(d, params, ps, s, s_rs, s_cs, act, R, (float*)H);
         }
         AVD_LAUNCH_OK();
         return AVD_OK;
     }
 
+    // 16-bit layer-2 kernels W2b / W2T of A agents (precision 3: three planes of A*F*l2 elements each)
     int pack(const float* params, int64_t pstride, int64_t oW2, int F, bf16* W2b, bf16* W2T) const {
-        pack_w2_kernel<<<dim3((unsigned)((F * d.l2 + 255) / 256), A), 256, 0, st>>>(params, pstride, oW2, F, d.l2, W2b, W2T);
+        const dim3 grid((unsigned)((F * d.l2 + 255) / 256), A);
+        if (prec == 3) {
+            const int64_t plane = (int64_t)A * F * d.l2;
+            pack_w2_kernel<Planes3><<<grid, 256, 0, st>>>(params, pstride, oW2, F, d.l2, Planes3{W2b, plane}, Planes3{W2T, plane});
+        } else {
+            pack_w2_kernel<bf16*><<<grid, 256, 0, st>>>(params, pstride, oW2, F, d.l2, W2b, W2T);
+        }
         AVD_LAUNCH_OK();
         return AVD_OK;
     }
@@ -1383,6 +1443,8 @@ struct Pass {
 
     // Z[a] (R x l2) = H[a] (R x F) . W2[a] (F x l2)
     int forward(const void* H, int F, const float* params, int64_t pstride, int64_t oW2, const bf16* W2T, float* Z) const {
+        if (prec == 3)
+            return umma::gemm_bf16x3(0, A, (int)R, d.l2, F, H, F, R * F, W2T, F, (int64_t)d.l2 * F, Z, d.l2, R * d.l2, 1, st);
         if (prec)
             return umma::gemm_bf16(0, A, (int)R, d.l2, F, H, F, R * F, W2T, F, (int64_t)d.l2 * F, Z, d.l2, R * d.l2, 1, st);
         GemmArgs g = {};
@@ -1399,6 +1461,8 @@ struct Pass {
         const int64_t chunk = prec ? 64 : 256;
         int split = (int)std::min<int64_t>((R + chunk - 1) / chunk, std::max(1, 4 * sm_count() / std::max(1, tiles)));
         split = std::max(1, split);
+        if (prec == 3)
+            return umma::gemm_bf16x3(1, A, F, d.l2, (int)R, H, F, R * F, DZ, d.l2, R * d.l2, grads + oW2, d.l2, gstride, split, st);
         if (prec)
             return umma::gemm_bf16(1, A, F, d.l2, (int)R, H, F, R * F, DZ, d.l2, R * d.l2, grads + oW2, d.l2, gstride, split, st);
         GemmArgs g = {};
@@ -1411,6 +1475,9 @@ struct Pass {
 
     // DH[a] (R x Fsub) = DZ[a] (R x l2) . W2[a][f0:f0+Fsub, :]^T
     int dgrad(const void* DZ, const float* params, int64_t pstride, int64_t oW2, const bf16* W2b, int F, int f0, int Fsub, float* DH) const {
+        if (prec == 3)
+            return umma::gemm_bf16x3(0, A, (int)R, Fsub, d.l2, DZ, d.l2, R * d.l2, W2b + (int64_t)f0 * d.l2, d.l2, (int64_t)F * d.l2, DH, Fsub,
+                                     R * Fsub, 1, st);
         if (prec)
             return umma::gemm_bf16(0, A, (int)R, Fsub, d.l2, DZ, d.l2, R * d.l2, W2b + (int64_t)f0 * d.l2, d.l2, (int64_t)F * d.l2, DH, Fsub,
                                    R * Fsub, 1, st);
@@ -1436,9 +1503,21 @@ extern "C" int avd_ddpg_param_counts(const avd_net_dims* dims, int64_t* out4) {
     return AVD_OK;
 }
 
+// the persistent fused kernels (avd_fused3.cu and friends) serve precision 1 and 2 at the dims they support
+static bool fused_path(const avd_net_dims& d, int precision) { return (precision == 1 || precision == 2) && fused3::supported(d); }
+
 extern "C" int64_t avd_ddpg_workspace_bytes(const avd_net_dims* dims, int32_t A, int64_t rows_per_agent, int32_t precision) {
     if (!dims || A < 0 || rows_per_agent < 0) return -1;
-    return Workspace::bytes(*dims, A, (int64_t)A * rows_per_agent, precision != 0 && fused3::supported(*dims));
+    return Workspace::bytes(*dims, A, (int64_t)A * rows_per_agent, fused_path(*dims, precision), precision == 3 ? 3 : 1);
+}
+
+// [H | Z | W2T]: layer-1 output (fp32, or three bf16 planes at precision 3), layer-2 output (fp32), packed layer-2 kernel (16-bit, 3 planes)
+extern "C" int64_t avd_forward_workspace_bytes(const avd_net_dims* dims, int32_t A, int64_t rows_per_agent, int32_t critic, int32_t precision) {
+    if (!dims || A < 0 || rows_per_agent < 0) return -1;
+    const int64_t N = (int64_t)A * rows_per_agent, F = critic ? dims->l1 + dims->la : dims->l1;
+    const int64_t planes = precision == 3 ? 3 : 1;
+    const int64_t h = precision == 3 ? N * F * 3 * (int64_t)sizeof(bf16) : N * F * (int64_t)sizeof(float);
+    return h + N * dims->l2 * (int64_t)sizeof(float) + planes * A * F * dims->l2 * (int64_t)sizeof(bf16) + 512;
 }
 
 #define AVD_TRY(expr)             \
@@ -1455,15 +1534,15 @@ extern "C" int avd_actor_forward(const avd_net_dims* dims, int32_t A, int64_t R,
     AVD_REQUIRE(A >= 0 && R >= 0, "bad sizes");
     const avd_net_dims d = *dims;
     const int64_t N = (int64_t)A * R;
-    const int64_t need = N * (d.l1 + d.l2) * (int64_t)sizeof(float) + (int64_t)A * d.l1 * d.l2 * (int64_t)sizeof(bf16) + 512;
+    const int64_t need = avd_forward_workspace_bytes(dims, A, R, 0, precision);
     AVD_REQUIRE(workspace_bytes >= need, "workspace too small (%lld < %lld)", (long long)workspace_bytes, (long long)need);
     if (N == 0) return AVD_OK;
     const Pass p{d, A, precision, R, (cudaStream_t)stream};
     const ActorOff o = actor_off(d);
     float* H = reinterpret_cast<float*>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
-    float* Z = H + N * d.l1;
+    float* Z = H + (precision == 3 ? N * d.l1 * 3 / 2 : N * d.l1);
     bf16* W2T = reinterpret_cast<bf16*>(Z + N * d.l2);
-    if (precision && fused3::supported(d)) {   // fused kernel: H / Z are never materialised, their space holds the folded bias
+    if (fused_path(d, precision)) {   // fused kernel: H / Z are never materialised, their space holds the folded bias
         AVD_TRY(p.pack_fold(false, actor_params, nullptr, W2T, H));
         return fused3::run(fused3::MODE_ACTOR_OUT, p.f16(), d, A, R, actor_params, o.total, W2T, H, nullptr, s, s_rs, s_cs, nullptr, nullptr, 0.f,
                            action_high, nullptr, nullptr, out, nullptr, nullptr, 1.0f, nullptr, nullptr, p.st);
@@ -1485,15 +1564,15 @@ extern "C" int avd_critic_forward(const avd_net_dims* dims, int32_t A, int64_t R
     const avd_net_dims d = *dims;
     const int64_t N = (int64_t)A * R;
     const int F = d.l1 + d.la;
-    const int64_t need = N * (F + d.l2) * (int64_t)sizeof(float) + (int64_t)A * F * d.l2 * (int64_t)sizeof(bf16) + 512;
+    const int64_t need = avd_forward_workspace_bytes(dims, A, R, 1, precision);
     AVD_REQUIRE(workspace_bytes >= need, "workspace too small (%lld < %lld)", (long long)workspace_bytes, (long long)need);
     if (N == 0) return AVD_OK;
     const Pass p{d, A, precision, R, (cudaStream_t)stream};
     const CriticOff o = critic_off(d);
     float* H = reinterpret_cast<float*>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
-    float* Z = H + N * F;
+    float* Z = H + (precision == 3 ? (int64_t)N * F * 3 / 2 : N * F);
     bf16* W2T = reinterpret_cast<bf16*>(Z + N * d.l2);
-    if (precision && fused3::supported(d)) {
+    if (fused_path(d, precision)) {
         AVD_TRY(p.pack_fold(true, critic_params, nullptr, W2T, H));
         return fused3::run(fused3::MODE_Q, p.f16(), d, A, R, critic_params, o.total, W2T, H, nullptr, s, d.ns, 1, a, nullptr, 0.f, 0.f, nullptr,
                            nullptr, q, nullptr, nullptr, 1.0f, nullptr, nullptr, p.st);
@@ -1861,8 +1940,8 @@ extern "C" int avd_ddpg_learn(const avd_learn_io* io, void* stream) {
     const CriticOff co = critic_off(d);
     const int F = d.l1 + d.la;
     Workspace w;
-    const bool fz = tc && fused3::supported(d);   // persistent fused pass / dgrad / wgrad kernels
-    w.carve(io->workspace, d, A, N, fz);
+    const bool fz = fused_path(d, io->precision);   // persistent fused pass / dgrad / wgrad kernels
+    w.carve(io->workspace, d, A, N, fz, io->precision == 3 ? 3 : 1);
     const dim3 gl1b((unsigned)((R + kL1BwdRows - 1) / kL1BwdRows), A);
     const int64_t srs = io->s_stride ? io->s_stride : d.ns;      // row pitch of the state batches
     AVD_REQUIRE(srs >= d.ns, "s_stride %d is smaller than the state width %d", (int)io->s_stride, d.ns);
@@ -1871,7 +1950,7 @@ extern "C" int avd_ddpg_learn(const avd_learn_io* io, void* stream) {
     AVD_CUDA_OK(cudaMemsetAsync(io->critic_grad, 0, (size_t)A * co.n_train * sizeof(float), st));
     if (io->loss) AVD_CUDA_OK(cudaMemsetAsync(io->loss, 0, (size_t)A * 2 * sizeof(float), st));
     if (fz) return learn_fused3(io, p, w, st);
-    if (tc) {   // bf16 copies of the four layer-2 kernels (K-major for forward, and for dgrad on the online nets)
+    if (tc) {   // 16-bit copies (precision 3: split planes) of the four layer-2 kernels (K-major for forward, and for dgrad on the online nets)
         AVD_TRY(p.pack(io->t_actor, ao.total, ao.W2, d.l1, nullptr, w.taW2T));
         AVD_TRY(p.pack(io->t_critic, co.total, co.W2, F, nullptr, w.tcW2T));
         AVD_TRY(p.pack(io->critic, co.total, co.W2, F, w.cW2b, w.cW2T));
@@ -1898,7 +1977,7 @@ extern "C" int avd_ddpg_learn(const avd_learn_io* io, void* stream) {
     {
         HeadArgs h = critic_head(d, io->critic, w.Z, R);
         h.y = w.y; h.out = w.q; h.DZ = w.DZ; h.grads = io->critic_grad; h.gstride = co.n_train; h.loss = io->loss;
-        AVD_TRY(launch_head<HEAD_CRITIC_BWD>(h, d.l2, A, st, tc));
+        AVD_TRY(launch_head<HEAD_CRITIC_BWD>(h, d.l2, A, st, io->precision));
     }
     AVD_TRY(p.wgrad(w.H, F, w.DZ, io->critic_grad, co.n_train, co.W2));
     AVD_TRY(p.dgrad(w.DZ, io->critic, co.total, co.W2, w.cW2b, F, 0, F, w.DH));
@@ -1917,7 +1996,7 @@ extern "C" int avd_ddpg_learn(const avd_learn_io* io, void* stream) {
     {
         HeadArgs h = critic_head(d, io->critic, w.Z, R);
         h.DZ = w.DZ; h.loss = io->loss;
-        AVD_TRY(launch_head<HEAD_CRITIC_BWD_ACTION>(h, d.l2, A, st, tc));
+        AVD_TRY(launch_head<HEAD_CRITIC_BWD_ACTION>(h, d.l2, A, st, io->precision));
     }
     AVD_TRY(p.dgrad(w.DZ, io->critic, co.total, co.W2, w.cW2b, F, d.l1, d.la, w.DH));   // action columns only
     action_grad_kernel<<<dim3((unsigned)std::min<int64_t>((R + 255) / 256, 2048), A), 256, 0, st>>>(d, io->critic, co.total, w.a2, R, w.DH, w.dpi);
@@ -1925,7 +2004,7 @@ extern "C" int avd_ddpg_learn(const avd_learn_io* io, void* stream) {
     {
         HeadArgs h = actor_head(d, io->actor, w.Za, R, io->action_high);
         h.dpi = w.dpi; h.DZ = w.DZ; h.grads = io->actor_grad; h.gstride = ao.n_train;
-        AVD_TRY(launch_head<HEAD_ACTOR_BWD>(h, d.l2, A, st, tc));
+        AVD_TRY(launch_head<HEAD_ACTOR_BWD>(h, d.l2, A, st, io->precision));
     }
     AVD_TRY(p.wgrad(w.H1a, d.l1, w.DZ, io->actor_grad, ao.n_train, ao.W2));
     AVD_TRY(p.dgrad(w.DZ, io->actor, ao.total, ao.W2, w.aW2b, d.l1, 0, d.l1, w.DH));

@@ -68,7 +68,7 @@ class DDPGPopulation:
         if M != self.M or P != self.G * envs_per_group:
             raise ValueError("state batch does not match the population")
         rows = envs_per_group
-        need = self.A * rows * (d.l1 + d.l2) * 4 + self.A * d.l1 * d.l2 * 2 + 1024
+        need = self.lib.avd_forward_workspace_bytes(C.byref(d), self.A, rows, 0, self.precision)
         if self._act_ws is None or self._act_ws.numel() < need:
             self._act_ws = torch.empty(need, dtype=torch.uint8, device=self.device)
         _lib.check(self.lib.avd_actor_forward(C.byref(d), self.A, rows, _lib.ptr(self.actor.flat), _lib.ptr(native_state), 1,

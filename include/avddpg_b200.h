@@ -31,7 +31,7 @@ extern "C" {
 
 #define AVD_MAX_FOLLOWERS 16
 #define AVD_RING_RECORD_FLOATS 10
-#define AVD_ABI_VERSION 2
+#define AVD_ABI_VERSION 3
 
 typedef enum avd_status {
     AVD_OK = 0,
@@ -240,13 +240,16 @@ typedef struct avd_learn_io {
     float* loss;                /* [A][2] nullable: critic_loss, actor_loss                            */
     void* workspace;            /* avd_ddpg_workspace_bytes(dims, A, rows_per_agent, precision) bytes  */
     int64_t workspace_bytes;
-    int32_t precision;          /* 0: fp32 SIMT kernels (parity mode); 1: bf16 tcgen05 tensor-core GEMMs; 2: fp16 tcgen05 (DESIGN.md 4) */
+    int32_t precision;          /* 0: fp32 SIMT kernels (parity mode); 1: bf16 tcgen05 tensor-core GEMMs; 2: fp16 tcgen05;
+                                   3: tcgen05 on three-way split bf16 operands, fp32-accurate (avd_gemm_bf16x3; DESIGN.md 4) */
     int32_t s_stride;           /* row pitch of s / s2 in floats: 4 for the replay gather output (avd_replay_gather), 0 = dims.ns */
 } avd_learn_io;
 
 /* sizes of the flat parameter vectors: out4 = {actor_trainable, actor_total, critic_trainable, critic_total} */
 int avd_ddpg_param_counts(const avd_net_dims* dims, int64_t* out4);
 int64_t avd_ddpg_workspace_bytes(const avd_net_dims* dims, int32_t A, int64_t rows_per_agent, int32_t precision);
+/* workspace of avd_actor_forward (critic = 0) / avd_critic_forward (critic = 1) for A agents x rows_per_agent rows; -1 on bad arguments */
+int64_t avd_forward_workspace_bytes(const avd_net_dims* dims, int32_t A, int64_t rows_per_agent, int32_t critic, int32_t precision);
 
 /* Trainer.learn (workers/trainer.py:472-508) for all agents at once: TD target from the target nets,
  * critic MSE gradient, actor -mean(Q) gradient (both on the pre-update weights); then, if apply_updates,
@@ -388,6 +391,14 @@ int avd_gemm_bf16(int layout, int batch, int M, int N, int K, const void* A, int
  * descriptor has a format field per operand, but B200 traps on fp16 x bf16.                                                         */
 int avd_gemm_f16kind(int layout, int batch, int M, int N, int K, const void* A, int64_t lda, int64_t a_batch, const void* B,
                      int64_t ldb, int64_t b_batch, float* C, int64_t ldc, int64_t c_batch, int splitk, int a_fmt, int b_fmt, void* stream);
+
+/* The same GEMM on fp32-accurate split operands, the building block of precision = 3: every operand element x is given as three bf16
+ * planes hi = bf16(x), mid = bf16(x - hi), lo = bf16(x - hi - mid) (24 significand bits together), stored [plane][batch][rows][inner]:
+ * plane p of batch b starts at A_planes + (p * batch + b) * a_batch (likewise B), so a_batch / b_batch must be positive.  Each K block
+ * runs the six products hi.hi + hi.mid + mid.hi + hi.lo + mid.mid + lo.hi into one fp32 accumulator; the dropped ones are below
+ * 2^-27 |a||b|.  Layouts, pitches, split-K and alignment as avd_gemm_bf16.                                                         */
+int avd_gemm_bf16x3(int layout, int batch, int M, int N, int K, const void* A_planes, int64_t lda, int64_t a_batch, const void* B_planes,
+                    int64_t ldb, int64_t b_batch, float* C, int64_t ldc, int64_t c_batch, int splitk, void* stream);
 
 /* ---- raw RNG access (parity tests: bit-exact against oracle/philox_np.py) ------------------- */
 int avd_rng_words(uint32_t* out4 /*[n][4]*/, int64_t n, uint64_t id_base, uint32_t tick, uint32_t purpose,

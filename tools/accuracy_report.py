@@ -1,6 +1,6 @@
-"""Per-tensor error of the tensor-core learn step (precision 1 = bf16 operands, 2 = fp16 operands) against the fp32 oracle,
-for a few batch sizes.
-    python tools/accuracy_report.py > profiles/r02_tensor_core_accuracy.txt"""
+"""Per-tensor error of the tensor-core learn step (precision 1 = bf16 operands, 2 = fp16 operands, 3 = three-way split bf16
+operands) against the fp32 oracle, for a few batch sizes.
+    python tools/accuracy_report.py [precision ...] > profiles/r03_tensor_core_accuracy.txt      (default: 1 2 3)"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -12,7 +12,8 @@ from avddpg_b200.config import Config
 
 mods = dict(lib=_lib, trainer=trainer, Config=Config)
 print("# rel-L2 error of every gradient tensor, tcgen05 learn step vs oracle/ddpg_np.py (fp32 numpy); seed 50 of tests/test_gpu_ddpg.py")
-for prec, R in [(p, R) for p in (1, 2) for R in (64, 1024, 16384, 262144)]:
+precisions = [int(x) for x in sys.argv[1:]] or [1, 2, 3]
+for prec, R in [(p, R) for p in precisions for R in (64, 1024, 16384, 262144)]:
     conf, pop, nets, batches, (s, a, r, s2) = T.build_population(mods, 1, R, [50])
     pop.precision = prec
     pop.learn(s, a, r, s2, apply_updates=False)

@@ -5,6 +5,9 @@ float64 with the chosen sites rounded to the chosen format and reports the rel-L
 unrounded run.  Used to decide which operands need more than bf16 (DESIGN.md §4); runs without a GPU:
 
     python tools/precision_model.py                # table: one site at a time, R = 64 (worst of 20 seeds) and R = 16384
+    python tools/precision_model.py --split        # table: every site in one format (fp32, bf16x2, bf16x3, tf32x2), worst
+                                                   # per-tensor max-norm error over 40 seeds at R = 64, 4 at 1000, 2 at 16384
+                                                   # (the choice of three-way split bf16 operands for precision = 3)
 
 Sites (names follow csrc/avd_fused3.cu / avd_wgrad3.cu / avd_dgrad3.cu):
     r1    relu(z1) A tile of layer 2, all passes                    W2f   folded layer-2 kernel W2' (forward B operand)
@@ -37,9 +40,23 @@ def rnd(x, fmt):
         m = float(t.abs().max())
         k = 0 if m == 0 else 14 - int(np.ceil(np.log2(m)))
         return (t * 2.0 ** k).to(torch.float16).to(torch.float64).numpy() * 2.0 ** -k
+    if fmt == "fp32":      # operands only stored in fp32
+        return t.to(torch.float64).numpy()
     if fmt == "bf16x2":    # hi + lo split
         hi = t.to(torch.bfloat16).to(torch.float32)
         lo = (t - hi).to(torch.bfloat16).to(torch.float32)
+        return (hi.to(torch.float64) + lo.to(torch.float64)).numpy()
+    if fmt == "bf16x3":    # hi + mid + lo split of precision 3 (csrc/avd_ddpg.cu split3), products mid.lo, lo.mid, lo.lo dropped by
+        hi = t.to(torch.bfloat16).to(torch.float32)       # the GEMM are below 2^-27 relative and not modelled
+        mid = (t - hi).to(torch.bfloat16).to(torch.float32)
+        lo = (t - hi - mid).to(torch.bfloat16).to(torch.float32)
+        return (hi.to(torch.float64) + mid.to(torch.float64) + lo.to(torch.float64)).numpy()
+    if fmt == "tf32x2":    # hi + lo split into 10-bit-significand tf32 (round to nearest on the 13 dropped bits)
+        def tf32(v):
+            b = v.view(torch.int32)
+            return ((b + 0x1000) & ~0x1FFF).view(torch.float32)
+        hi = tf32(t.clone())
+        lo = tf32((t - hi).contiguous())
         return (hi.to(torch.float64) + lo.to(torch.float64)).numpy()
     raise ValueError(fmt)
 
@@ -192,7 +209,33 @@ def report(configs, Rs=(64, 16384), seeds64=20):
             print(f"{name:34s} R={R:6d} critic max {cmax:.1e} actor max {amax:.1e}  " + " ".join(f"{k}={worst[k]:.1e}" for k in keys), flush=True)
 
 
+SPLIT_SITES = ("r1", "W2f", "dm", "W2b", "dz1", "action_T")
+
+
+def report_split(fmts=("fp32", "bf16x2", "bf16x3", "tf32x2"), cases=((64, 40), (1000, 4), (16384, 2))):
+    """Every rounding site in one format; worst per-tensor max-norm error (max |got - ref| / max |ref|, the metric of the
+    precision-0 parity test) against the unrounded float64 run, over the seeds of each batch size."""
+    for fmt in fmts:
+        sites = {k: fmt for k in SPLIT_SITES}
+        row = []
+        for R, nseeds in cases:
+            worst, where = 0.0, None
+            for seed in range(nseeds):
+                nets, batch = make_case(100 + seed, R)
+                for (rc, ra), (gc, ga) in ((emulate(nets, batch, {}), emulate(nets, batch, sites)),):
+                    for tag, ref, got in (("c.", rc, gc), ("a.", ra, ga)):
+                        for k in ref:
+                            e = float(np.max(np.abs(got[k] - ref[k])) / max(np.max(np.abs(ref[k])), 1e-300))
+                            if e > worst:
+                                worst, where = e, f"{tag}{k} seed {seed}"
+            row.append(f"R={R:6d} ({nseeds:2d} seeds) {worst:.1e} [{where}]")
+        print(f"{fmt:7s} " + "  ".join(row), flush=True)
+
+
 if __name__ == "__main__":
+    if "--split" in sys.argv:
+        report_split()
+        sys.exit(0)
     one_at_a_time = [("round 1 (all bf16)", ROUND1)] + [(f"only {k}", {k: "bf16"}) for k in ("r1", "W2f", "dm", "W2b", "dz1")] + [
         ("only dza+W2a (critic-action)", {"dza": "bf16", "W2a": "bf16"})]
     report(one_at_a_time)
