@@ -12,7 +12,7 @@
 // go through `gemm_batched`, which dispatches on io->precision: 0 = fp32 SIMT tiles (parity mode, this
 // file), 1 = bf16 tcgen05/TMEM tensor-core kernels, 2 = the same kernels with fp16 layer-2 operands (11-bit significand;
 // the backward tile stays bf16) and the T formulation of the critic-action pass (avd_fused3.cu), 3 = the unfused tcgen05 GEMMs on
-// three-way split bf16 operands (umma::gemm_bf16x3: hi / mid / lo planes, fp32-accurate).  Everything else (K=ns and K=1 layers,
+// three-way split bf16 operands (umma::gemm_bf16 on hi / mid / lo planes, fp32-accurate).  Everything else (K=ns and K=1 layers,
 // heads with N=1, BatchNorm affine, reductions for bias/BN gradients, TD target, losses) is fused into the
 // layer1 / head kernels below.
 //
@@ -21,47 +21,17 @@
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>
+#include <type_traits>
 
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
 #include "avd_common.cuh"
 #include "avd_ddpg_layout.cuh"
+#include "avd_learn_kernels.cuh"
 #include "avd_umma.cuh"
 
 namespace avd {
-
-typedef __nv_bfloat16 bf16;
-
-namespace fused3 {  // avd_fused3.cu
-enum Mode { MODE_ACTOR_OUT = 0, MODE_TARGET = 1, MODE_Q = 2, MODE_CRITIC_BWD = 3, MODE_ACTOR_BWD = 4, MODE_CRITIC_ACTION = 5, MODE_ACTOR_SAVE = 6 };
-bool supported(const avd_net_dims& d);
-int vtab_rows();
-int vtab_stride();
-int vtab_floats();
-int run(int mode, bool f16, const avd_net_dims& d, int A, int64_t R, const float* params, int64_t pstride, const bf16* W2T, const float* b2f,
-        const float* vtab, const float* s, int64_t s_rs, int64_t s_cs, const float* act, const float* rew, float gamma, float high, const float* y,
-        const float* dpi, float* out, uint32_t* mask_out, bf16* DZ_out, float dm_scale, float* sdq, float* loss, cudaStream_t st,
-        uint32_t* mask2_out = nullptr, float* dact_out = nullptr);
-}
-
-namespace wgrad3 {  // avd_wgrad3.cu
-int ctas_per_agent(int A, int64_t R);
-int run(bool f16, const avd_net_dims& d, bool critic, int A, int64_t R, const float* params, int64_t pstride, const float* s, int64_t s_rs,
-        const float* act, const bf16* DZ, float* out, int64_t out_agent_stride, int64_t out_cta_stride, cudaStream_t st);
-}
-
-namespace dgrad3 {  // avd_dgrad3.cu
-int run(bool f16, int A, int64_t R, int F, const bf16* DZ, const bf16* W2b, const uint32_t* mask, int mask_words, const bf16* xextT, int64_t Rp,
-        float* G1, int Fp, float* db2, int64_t db2_stride, cudaStream_t st);
-}
-
-namespace umma {   // avd_umma.cu
-int gemm_bf16(int layout, int batch, int M, int N, int K, const void* A, int64_t lda, int64_t a_batch, const void* B, int64_t ldb,
-              int64_t b_batch, float* C, int64_t ldc, int64_t c_batch, int splitk, cudaStream_t st);
-int gemm_bf16x3(int layout, int batch, int M, int N, int K, const void* A, int64_t lda, int64_t a_batch, const void* B, int64_t ldb,
-                int64_t b_batch, float* C, int64_t ldc, int64_t c_batch, int splitk, cudaStream_t st);
-}
 
 // GEMM operand written as three bf16 planes (precision 3): element i is hi at p[i], mid at p[plane + i], lo at p[2 plane + i],
 // hi = bf16(x), mid = bf16(x - hi), lo = bf16(x - hi - mid).  Both differences are exact in fp32, so hi + mid + lo keeps 24 bits of x.
@@ -72,6 +42,29 @@ struct Planes3 {
     __host__ __device__ Planes3 operator+(int64_t i) const { return Planes3{p + i, plane}; }
     __host__ __device__ explicit operator bool() const { return p != nullptr; }
 };
+
+// Format of the GEMM operands of the unfused learn step and forward passes (H, H1a, DZ and the W2 packs), set by the precision:
+// fp32 (0), one bf16 copy (1 and 2) or three bf16 planes (3).  A bf16 copy is given as much workspace as fp32.
+enum OperandFormat { OPND_F32, OPND_BF16, OPND_BF16X3 };
+inline OperandFormat operand_format(int precision) { return precision == 0 ? OPND_F32 : precision == 3 ? OPND_BF16X3 : OPND_BF16; }
+inline int operand_planes(int precision) { return operand_format(precision) == OPND_BF16X3 ? 3 : 1; }
+inline int64_t operand_bytes(int precision, int64_t n) {     // workspace of an operand of n elements
+    return operand_format(precision) == OPND_BF16X3 ? n * 3 * (int64_t)sizeof(bf16) : n * (int64_t)sizeof(float);
+}
+
+// The operand at p as T: float*, bf16* or Planes3 (plane = elements per plane)
+template <typename T> __host__ __device__ __forceinline__ T as_operand(void* p, int64_t) { return reinterpret_cast<T>(p); }
+template <> __host__ __device__ __forceinline__ Planes3 as_operand<Planes3>(void* p, int64_t plane) { return Planes3{reinterpret_cast<bf16*>(p), plane}; }
+
+// Calls f with the operand at p typed by the precision's format; f picks the kernel instantiation from the argument's type
+template <class Fn>
+void with_operand(int precision, void* p, int64_t plane, Fn&& f) {
+    switch (operand_format(precision)) {
+        case OPND_F32: f(as_operand<float*>(p, plane)); break;
+        case OPND_BF16: f(as_operand<bf16*>(p, plane)); break;
+        case OPND_BF16X3: f(as_operand<Planes3>(p, plane)); break;
+    }
+}
 
 __device__ __forceinline__ void split3(float x, bf16& hi, bf16& mid, bf16& lo) {
     hi = __float2bfloat16_rn(x);
@@ -332,9 +325,6 @@ struct HeadArgs {
     float* loss;           // [A][2] nullable
 };
 
-template <typename T> __device__ __forceinline__ T dz_out(void* p, int64_t) { return reinterpret_cast<T>(p); }
-template <> __device__ __forceinline__ Planes3 dz_out<Planes3>(void* p, int64_t plane) { return Planes3{reinterpret_cast<bf16*>(p), plane}; }
-
 template <int MODE, int CPL, typename TDZ>   // CPL = columns per lane (l2 = 32*CPL); TDZ: float*, bf16* or Planes3
 __global__ void __launch_bounds__(256) head_kernel(HeadArgs h) {
     constexpr int L2 = 32 * CPL;
@@ -398,7 +388,7 @@ __global__ void __launch_bounds__(256) head_kernel(HeadArgs h) {
             for (int j = 0; j < CPL; ++j) {
                 const float dh = dq * w3[j];
                 const float dz = z[j] > 0.0f ? dh * ginv[j] : 0.0f;
-                store_out(dz_out<TDZ>(h.DZ, h.dz_plane) + n * L2 + lane + 32 * j, dz);
+                store_out(as_operand<TDZ>(h.DZ, h.dz_plane) + n * L2 + lane + 32 * j, dz);
                 if (BWD) {
                     aW3[j] = fmaf(hh[j], dq, aW3[j]);
                     aG[j] = fmaf(dh, (fmaxf(z[j], 0.0f) - mu[j]) * inv[j], aG[j]);
@@ -536,38 +526,6 @@ __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ params, i
         Mm[i] = mi;
         Vv[i] = vi;
         P[i] -= lr_t * mi / (sqrtf(vi) + eps);
-    }
-}
-
-// Adam on the trainable prefix and the Polyak update of the target vector in one pass over an agent's parameters
-// (trainer.py:348-349 then 352-356 / ddpgagent.py:44-55: the target sees the freshly updated online weights).
-__global__ void __launch_bounds__(256) adam_polyak_kernel(float* __restrict__ params, float* __restrict__ target, int64_t pstride,
-                                                          const float* __restrict__ grads, int64_t gstride, float* __restrict__ m,
-                                                          float* __restrict__ v, const int32_t* __restrict__ step,
-                                                          const uint8_t* __restrict__ mask, int64_t n_train, int64_t total, float lr, float b1,
-                                                          float b2, float eps, float tau) {
-    const int agent = blockIdx.y;
-    if (mask && !mask[agent]) return;
-    const float t = (float)(step[agent] + 1);
-    const float lr_t = lr * sqrtf(1.0f - powf(b2, t)) / (1.0f - powf(b1, t));
-    float* P = params + (int64_t)agent * pstride;
-    float* T = target + (int64_t)agent * pstride;
-    const float* G = grads + (int64_t)agent * gstride;
-    float* Mm = m + (int64_t)agent * n_train;
-    float* Vv = v + (int64_t)agent * n_train;
-    const float omt = 1.0f - tau;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
-        float p = P[i];
-        if (i < n_train) {
-            const float g = G[i];
-            const float mi = Mm[i] + (g - Mm[i]) * (1.0f - b1);
-            const float vi = Vv[i] + (g * g - Vv[i]) * (1.0f - b2);
-            Mm[i] = mi;
-            Vv[i] = vi;
-            p -= lr_t * mi / (sqrtf(vi) + eps);
-            P[i] = p;
-        }
-        T[i] = p * tau + T[i] * omt;
     }
 }
 
@@ -1289,19 +1247,13 @@ static void launch_head_t(const HeadArgs& h, int l2, dim3 grid, cudaStream_t st)
     }
 }
 
-// prec: the learn step's precision, which decides the format of the backward tile DZ (fp32, one bf16 copy, or three bf16 planes)
+// prec: the learn step's precision, which decides the operand format of the backward tile DZ
 template <int MODE>
 static int launch_head(const HeadArgs& h, int l2, int A, cudaStream_t st, int prec = 0) {
     dim3 grid((unsigned)((h.R + 63) / 64), A);
-    if (prec == 3) {
-        HeadArgs hp = h;
-        hp.dz_plane = (int64_t)A * h.R * l2;
-        launch_head_t<MODE, Planes3>(hp, l2, grid, st);
-    } else if (prec) {
-        launch_head_t<MODE, bf16*>(h, l2, grid, st);
-    } else {
-        launch_head_t<MODE, float*>(h, l2, grid, st);
-    }
+    HeadArgs hp = h;
+    hp.dz_plane = (int64_t)A * h.R * l2;
+    with_operand(prec, h.DZ, hp.dz_plane, [&](auto dz) { launch_head_t<MODE, decltype(dz)>(hp, l2, grid, st); });
     AVD_LAUNCH_OK();
     return AVD_OK;
 }
@@ -1333,35 +1285,38 @@ struct Pass {
 
     bool f16() const { return prec == 2; }     // fp16 layer-2 operands in the fused tensor-core kernels
 
+    // the fields every fused pass sets; the caller adds those of its mode
+    fused3::RunArgs fused_args(fused3::Mode mode, const float* params, const bf16* W2T, const float* b2f, const float* s, int64_t s_rs) const {
+        const bool actor = mode == fused3::MODE_ACTOR_OUT || mode == fused3::MODE_ACTOR_SAVE;
+        fused3::RunArgs a;
+        a.mode = mode; a.f16 = f16(); a.d = d; a.A = A; a.R = R;
+        a.params = params; a.pstride = actor ? actor_off(d).total : critic_off(d).total;
+        a.W2T = W2T; a.b2f = b2f; a.s = s; a.s_rs = s_rs;
+        return a;
+    }
+
     dim3 l1_grid() const { return dim3((unsigned)((R + kL1Rows - 1) / kL1Rows), A); }
 
-    // layer 1 (+BN) of the actor (critic=false) or critic (true) into H ([N][F] fp32, bf16, or three bf16 planes of N*F)
+    // layer 1 (+BN) of the actor (critic=false) or critic (true) into H ([N][F] in the operand format)
     int layer1(bool critic, const float* params, const float* s, int64_t s_rs, int64_t s_cs, const float* act, void* H) const {
         const int64_t ps = critic ? critic_off(d).total : actor_off(d).total;
-        if (prec == 3) {
-            const Planes3 o{(bf16*)H, (int64_t)A * R * (critic ? d.l1 + d.la : d.l1)};
-            if (critic) l1_forward_kernel<true, Planes3><<<l1_grid(), 128, 0, st>>>(d, params, ps, s, s_rs, s_cs, act, R, o);
-            else l1_forward_kernel<false, Planes3><<<l1_grid(), 128, 0, st>>>(d, params, ps, s, s_rs, s_cs, act, R, o);
-        } else if (prec) {
-            if (critic) l1_forward_kernel<true, bf16*><<<l1_grid(), 128, 0, st>>>(d, params, ps, s, s_rs, s_cs, act, R, (bf16*)H);
-            else l1_forward_kernel<false, bf16*><<<l1_grid(), 128, 0, st>>>(d, params, ps, s, s_rs, s_cs, act, R, (bf16*)H);
-        } else {
-            if (critic) l1_forward_kernel<true, float*><<<l1_grid(), 128, 0, st>>>(d, params, ps, s, s_rs, s_cs, act, R, (float*)H);
-            else l1_forward_kernel<false, float*><<<l1_grid(), 128, 0, st>>>(d, params, ps, s, s_rs, s_cs, act, R, (float*)H);
-        }
+        with_operand(prec, H, (int64_t)A * R * (critic ? d.l1 + d.la : d.l1), [&](auto o) {
+            if (critic) l1_forward_kernel<true, decltype(o)><<<l1_grid(), 128, 0, st>>>(d, params, ps, s, s_rs, s_cs, act, R, o);
+            else l1_forward_kernel<false, decltype(o)><<<l1_grid(), 128, 0, st>>>(d, params, ps, s, s_rs, s_cs, act, R, o);
+        });
         AVD_LAUNCH_OK();
         return AVD_OK;
     }
 
-    // 16-bit layer-2 kernels W2b / W2T of A agents (precision 3: three planes of A*F*l2 elements each)
+    // 16-bit layer-2 kernels W2b / W2T of A agents in the operand format of precision 1, 2 or 3 (planes of A*F*l2 elements)
     int pack(const float* params, int64_t pstride, int64_t oW2, int F, bf16* W2b, bf16* W2T) const {
         const dim3 grid((unsigned)((F * d.l2 + 255) / 256), A);
-        if (prec == 3) {
-            const int64_t plane = (int64_t)A * F * d.l2;
-            pack_w2_kernel<Planes3><<<grid, 256, 0, st>>>(params, pstride, oW2, F, d.l2, Planes3{W2b, plane}, Planes3{W2T, plane});
-        } else {
-            pack_w2_kernel<bf16*><<<grid, 256, 0, st>>>(params, pstride, oW2, F, d.l2, W2b, W2T);
-        }
+        const int64_t plane = (int64_t)A * F * d.l2;
+        with_operand(prec, W2T, plane, [&](auto o) {
+            using T = decltype(o);
+            if constexpr (!std::is_same<T, float*>::value)
+                pack_w2_kernel<T><<<grid, 256, 0, st>>>(params, pstride, oW2, F, d.l2, as_operand<T>(W2b, plane), o);
+        });
         AVD_LAUNCH_OK();
         return AVD_OK;
     }
@@ -1420,7 +1375,7 @@ struct Pass {
     int unfold(bool critic, const float* params, int F, int Fp, float* G1, const float* G2part, float* grads, float* dbm, const float* b2f, float* U,
                const float* sdq, int* ticket, const float* wscale, float dm_scale) const {
         const int64_t gs = critic ? critic_off(d).n_train : actor_off(d).n_train;
-        const int ncta = wgrad3::ctas_per_agent(A, R);
+        const int ncta = ctas_per_agent(A, R);
         UnfoldOff u;
         u.f = fold_off(critic);
         int64_t ps;
@@ -1443,10 +1398,8 @@ struct Pass {
 
     // Z[a] (R x l2) = H[a] (R x F) . W2[a] (F x l2)
     int forward(const void* H, int F, const float* params, int64_t pstride, int64_t oW2, const bf16* W2T, float* Z) const {
-        if (prec == 3)
-            return umma::gemm_bf16x3(0, A, (int)R, d.l2, F, H, F, R * F, W2T, F, (int64_t)d.l2 * F, Z, d.l2, R * d.l2, 1, st);
-        if (prec)
-            return umma::gemm_bf16(0, A, (int)R, d.l2, F, H, F, R * F, W2T, F, (int64_t)d.l2 * F, Z, d.l2, R * d.l2, 1, st);
+        if (operand_format(prec) != OPND_F32)
+            return umma::gemm_bf16(operand_planes(prec), 0, A, (int)R, d.l2, F, H, F, R * F, W2T, F, (int64_t)d.l2 * F, Z, d.l2, R * d.l2, 1, st);
         GemmArgs g = {};
         g.A = (const float*)H; g.a_m = F; g.a_k = 1; g.a_batch = R * F;
         g.B = params + oW2; g.b_k = d.l2; g.b_n = 1; g.b_batch = pstride;
@@ -1461,10 +1414,8 @@ struct Pass {
         const int64_t chunk = prec ? 64 : 256;
         int split = (int)std::min<int64_t>((R + chunk - 1) / chunk, std::max(1, 4 * sm_count() / std::max(1, tiles)));
         split = std::max(1, split);
-        if (prec == 3)
-            return umma::gemm_bf16x3(1, A, F, d.l2, (int)R, H, F, R * F, DZ, d.l2, R * d.l2, grads + oW2, d.l2, gstride, split, st);
-        if (prec)
-            return umma::gemm_bf16(1, A, F, d.l2, (int)R, H, F, R * F, DZ, d.l2, R * d.l2, grads + oW2, d.l2, gstride, split, st);
+        if (operand_format(prec) != OPND_F32)
+            return umma::gemm_bf16(operand_planes(prec), 1, A, F, d.l2, (int)R, H, F, R * F, DZ, d.l2, R * d.l2, grads + oW2, d.l2, gstride, split, st);
         GemmArgs g = {};
         g.A = (const float*)H; g.a_m = 1; g.a_k = F; g.a_batch = R * F;
         g.B = (const float*)DZ; g.b_k = d.l2; g.b_n = 1; g.b_batch = R * d.l2;
@@ -1475,12 +1426,9 @@ struct Pass {
 
     // DH[a] (R x Fsub) = DZ[a] (R x l2) . W2[a][f0:f0+Fsub, :]^T
     int dgrad(const void* DZ, const float* params, int64_t pstride, int64_t oW2, const bf16* W2b, int F, int f0, int Fsub, float* DH) const {
-        if (prec == 3)
-            return umma::gemm_bf16x3(0, A, (int)R, Fsub, d.l2, DZ, d.l2, R * d.l2, W2b + (int64_t)f0 * d.l2, d.l2, (int64_t)F * d.l2, DH, Fsub,
-                                     R * Fsub, 1, st);
-        if (prec)
-            return umma::gemm_bf16(0, A, (int)R, Fsub, d.l2, DZ, d.l2, R * d.l2, W2b + (int64_t)f0 * d.l2, d.l2, (int64_t)F * d.l2, DH, Fsub,
-                                   R * Fsub, 1, st);
+        if (operand_format(prec) != OPND_F32)
+            return umma::gemm_bf16(operand_planes(prec), 0, A, (int)R, Fsub, d.l2, DZ, d.l2, R * d.l2, W2b + (int64_t)f0 * d.l2, d.l2,
+                                   (int64_t)F * d.l2, DH, Fsub, R * Fsub, 1, st);
         GemmArgs g = {};
         g.A = (const float*)DZ; g.a_m = d.l2; g.a_k = 1; g.a_batch = R * d.l2;
         g.B = params + oW2 + (int64_t)f0 * d.l2; g.b_k = 1; g.b_n = d.l2; g.b_batch = pstride;
@@ -1508,16 +1456,31 @@ static bool fused_path(const avd_net_dims& d, int precision) { return (precision
 
 extern "C" int64_t avd_ddpg_workspace_bytes(const avd_net_dims* dims, int32_t A, int64_t rows_per_agent, int32_t precision) {
     if (!dims || A < 0 || rows_per_agent < 0) return -1;
-    return Workspace::bytes(*dims, A, (int64_t)A * rows_per_agent, fused_path(*dims, precision), precision == 3 ? 3 : 1);
+    return Workspace::bytes(*dims, A, (int64_t)A * rows_per_agent, fused_path(*dims, precision), operand_planes(precision));
 }
 
-// [H | Z | W2T]: layer-1 output (fp32, or three bf16 planes at precision 3), layer-2 output (fp32), packed layer-2 kernel (16-bit, 3 planes)
+// Workspace of the forward entry points, [H | Z | W2T]: layer-1 output in the operand format, layer-2 output (fp32), packed layer-2
+// kernel (16-bit, one copy or three planes), from `base` rounded up to 256 bytes.
+struct ForwardWorkspace {
+    float *H, *Z;
+    bf16* W2T;
+    int64_t bytes;
+};
+static ForwardWorkspace forward_workspace(const avd_net_dims& d, int64_t A, int64_t R, bool critic, int precision, void* base) {
+    const int64_t N = A * R, F = critic ? d.l1 + d.la : d.l1;
+    const int64_t h = operand_bytes(precision, N * F), z = N * d.l2 * (int64_t)sizeof(float);
+    const uintptr_t p = ((uintptr_t)base + 255) & ~(uintptr_t)255;
+    ForwardWorkspace w;
+    w.H = reinterpret_cast<float*>(p);
+    w.Z = reinterpret_cast<float*>(p + h);
+    w.W2T = reinterpret_cast<bf16*>(p + h + z);
+    w.bytes = h + z + operand_planes(precision) * A * F * d.l2 * (int64_t)sizeof(bf16) + 512;
+    return w;
+}
+
 extern "C" int64_t avd_forward_workspace_bytes(const avd_net_dims* dims, int32_t A, int64_t rows_per_agent, int32_t critic, int32_t precision) {
     if (!dims || A < 0 || rows_per_agent < 0) return -1;
-    const int64_t N = (int64_t)A * rows_per_agent, F = critic ? dims->l1 + dims->la : dims->l1;
-    const int64_t planes = precision == 3 ? 3 : 1;
-    const int64_t h = precision == 3 ? N * F * 3 * (int64_t)sizeof(bf16) : N * F * (int64_t)sizeof(float);
-    return h + N * dims->l2 * (int64_t)sizeof(float) + planes * A * F * dims->l2 * (int64_t)sizeof(bf16) + 512;
+    return forward_workspace(*dims, A, rows_per_agent, critic != 0, precision, nullptr).bytes;
 }
 
 #define AVD_TRY(expr)             \
@@ -1533,24 +1496,21 @@ extern "C" int avd_actor_forward(const avd_net_dims* dims, int32_t A, int64_t R,
     AVD_REQUIRE(actor_params && s && out && workspace, "null buffer");
     AVD_REQUIRE(A >= 0 && R >= 0, "bad sizes");
     const avd_net_dims d = *dims;
-    const int64_t N = (int64_t)A * R;
-    const int64_t need = avd_forward_workspace_bytes(dims, A, R, 0, precision);
-    AVD_REQUIRE(workspace_bytes >= need, "workspace too small (%lld < %lld)", (long long)workspace_bytes, (long long)need);
-    if (N == 0) return AVD_OK;
+    const ForwardWorkspace w = forward_workspace(d, A, R, false, precision, workspace);
+    AVD_REQUIRE(workspace_bytes >= w.bytes, "workspace too small (%lld < %lld)", (long long)workspace_bytes, (long long)w.bytes);
+    if ((int64_t)A * R == 0) return AVD_OK;
     const Pass p{d, A, precision, R, (cudaStream_t)stream};
     const ActorOff o = actor_off(d);
-    float* H = reinterpret_cast<float*>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
-    float* Z = H + (precision == 3 ? N * d.l1 * 3 / 2 : N * d.l1);
-    bf16* W2T = reinterpret_cast<bf16*>(Z + N * d.l2);
     if (fused_path(d, precision)) {   // fused kernel: H / Z are never materialised, their space holds the folded bias
-        AVD_TRY(p.pack_fold(false, actor_params, nullptr, W2T, H));
-        return fused3::run(fused3::MODE_ACTOR_OUT, p.f16(), d, A, R, actor_params, o.total, W2T, H, nullptr, s, s_rs, s_cs, nullptr, nullptr, 0.f,
-                           action_high, nullptr, nullptr, out, nullptr, nullptr, 1.0f, nullptr, nullptr, p.st);
+        AVD_TRY(p.pack_fold(false, actor_params, nullptr, w.W2T, w.H));
+        fused3::RunArgs f = p.fused_args(fused3::MODE_ACTOR_OUT, actor_params, w.W2T, w.H, s, s_rs);
+        f.s_cs = s_cs; f.high = action_high; f.out = out;
+        return fused3::run(f, p.st);
     }
-    if (precision) AVD_TRY(p.pack(actor_params, o.total, o.W2, d.l1, nullptr, W2T));
-    AVD_TRY(p.layer1(false, actor_params, s, s_rs, s_cs, nullptr, H));
-    AVD_TRY(p.forward(H, d.l1, actor_params, o.total, o.W2, W2T, Z));
-    HeadArgs h = actor_head(d, actor_params, Z, R, action_high);
+    if (precision) AVD_TRY(p.pack(actor_params, o.total, o.W2, d.l1, nullptr, w.W2T));
+    AVD_TRY(p.layer1(false, actor_params, s, s_rs, s_cs, nullptr, w.H));
+    AVD_TRY(p.forward(w.H, d.l1, actor_params, o.total, o.W2, w.W2T, w.Z));
+    HeadArgs h = actor_head(d, actor_params, w.Z, R, action_high);
     h.out = out;
     return launch_head<HEAD_ACTOR_FWD>(h, d.l2, A, p.st);
 }
@@ -1562,25 +1522,22 @@ extern "C" int avd_critic_forward(const avd_net_dims* dims, int32_t A, int64_t R
     AVD_REQUIRE(critic_params && s && a && q && workspace, "null buffer");
     AVD_REQUIRE(A >= 0 && R >= 0, "bad sizes");
     const avd_net_dims d = *dims;
-    const int64_t N = (int64_t)A * R;
     const int F = d.l1 + d.la;
-    const int64_t need = avd_forward_workspace_bytes(dims, A, R, 1, precision);
-    AVD_REQUIRE(workspace_bytes >= need, "workspace too small (%lld < %lld)", (long long)workspace_bytes, (long long)need);
-    if (N == 0) return AVD_OK;
+    const ForwardWorkspace w = forward_workspace(d, A, R, true, precision, workspace);
+    AVD_REQUIRE(workspace_bytes >= w.bytes, "workspace too small (%lld < %lld)", (long long)workspace_bytes, (long long)w.bytes);
+    if ((int64_t)A * R == 0) return AVD_OK;
     const Pass p{d, A, precision, R, (cudaStream_t)stream};
     const CriticOff o = critic_off(d);
-    float* H = reinterpret_cast<float*>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
-    float* Z = H + (precision == 3 ? (int64_t)N * F * 3 / 2 : N * F);
-    bf16* W2T = reinterpret_cast<bf16*>(Z + N * d.l2);
     if (fused_path(d, precision)) {
-        AVD_TRY(p.pack_fold(true, critic_params, nullptr, W2T, H));
-        return fused3::run(fused3::MODE_Q, p.f16(), d, A, R, critic_params, o.total, W2T, H, nullptr, s, d.ns, 1, a, nullptr, 0.f, 0.f, nullptr,
-                           nullptr, q, nullptr, nullptr, 1.0f, nullptr, nullptr, p.st);
+        AVD_TRY(p.pack_fold(true, critic_params, nullptr, w.W2T, w.H));
+        fused3::RunArgs f = p.fused_args(fused3::MODE_Q, critic_params, w.W2T, w.H, s, d.ns);
+        f.act = a; f.out = q;
+        return fused3::run(f, p.st);
     }
-    if (precision) AVD_TRY(p.pack(critic_params, o.total, o.W2, F, nullptr, W2T));
-    AVD_TRY(p.layer1(true, critic_params, s, d.ns, 1, a, H));
-    AVD_TRY(p.forward(H, F, critic_params, o.total, o.W2, W2T, Z));
-    HeadArgs h = critic_head(d, critic_params, Z, R);
+    if (precision) AVD_TRY(p.pack(critic_params, o.total, o.W2, F, nullptr, w.W2T));
+    AVD_TRY(p.layer1(true, critic_params, s, d.ns, 1, a, w.H));
+    AVD_TRY(p.forward(w.H, F, critic_params, o.total, o.W2, w.W2T, w.Z));
+    HeadArgs h = critic_head(d, critic_params, w.Z, R);
     h.out = q;
     return launch_head<HEAD_CRITIC_Q>(h, d.l2, A, p.st);
 }
@@ -1847,31 +1804,38 @@ static int learn_fused3(const avd_learn_io* io, const Pass& p, const Workspace& 
     AVD_LAUNCH_OK();
     tm.mark("fold+xext");
     // ---- TD target: y = r + gamma * target_critic(s', target_actor(s'))            trainer.py:493-494
-    AVD_TRY(fused3::run(fused3::MODE_ACTOR_OUT, f16, d, A, R, io->t_actor, ao.total, w.taW2T, w.ta_b2f, nullptr, io->s2, srs, 1, nullptr, nullptr, 0.f,
-                        io->action_high, nullptr, nullptr, w.a2, nullptr, nullptr, 1.0f, nullptr, nullptr, st));
+    {
+        fused3::RunArgs f = p.fused_args(fused3::MODE_ACTOR_OUT, io->t_actor, w.taW2T, w.ta_b2f, io->s2, srs);
+        f.high = io->action_high; f.out = w.a2;
+        AVD_TRY(fused3::run(f, st));
+    }
     tm.mark("t_actor");
-    AVD_TRY(fused3::run(fused3::MODE_TARGET, f16, d, A, R, io->t_critic, co.total, w.tcW2T, w.tc_b2f, nullptr, io->s2, srs, 1, w.a2, io->r, io->gamma, 0.f,
-                        nullptr, nullptr, w.y, nullptr, nullptr, 1.0f, nullptr, nullptr, st));
+    {
+        fused3::RunArgs f = p.fused_args(fused3::MODE_TARGET, io->t_critic, w.tcW2T, w.tc_b2f, io->s2, srs);
+        f.act = w.a2; f.rew = io->r; f.gamma = io->gamma; f.out = w.y;
+        AVD_TRY(fused3::run(f, st));
+    }
     tm.mark("t_critic");
-    const int ncta = wgrad3::ctas_per_agent(A, R);
+    const int ncta = ctas_per_agent(A, R);
     const int64_t g2_cta = (int64_t)Workspace::kG2Rows * d.l2, g2_agent = (int64_t)ncta * g2_cta;
     float* const dbm_a = w.dbm + (int64_t)A * d.l2;
     // The actor's chain needs the critic's WEIGHTS, not its gradients, so its first half goes in front of the critic's backward pass: the
     // elementwise kernel that forms the actor's backward tile (HBM-bound, 55 us) then runs on the side stream beside the critic's
     // backward pass (tensor-bound), and the critic's unfold beside the actor's dgrad.  Both chains have their own tile / mask / slice buffers.
     // ---- actor loss gradient, first half: pi(s), d(-mean q)/d pi                    trainer.py:501-506
-    static const bool legacy_actor_bwd = getenv("AVD_ACTOR_BWD_PASS") != nullptr;     // diagnostic: the round-1 second forward pass
-    AVD_TRY(fused3::run(legacy_actor_bwd ? fused3::MODE_ACTOR_OUT : fused3::MODE_ACTOR_SAVE, f16, d, A, R, io->actor, ao.total, w.aW2T, w.a_b2f, nullptr,
-                        io->s, srs, 1, nullptr, nullptr, 0.f, io->action_high, nullptr, nullptr, w.a2, legacy_actor_bwd ? nullptr : w.mask_a, nullptr, 1.0f,
-                        nullptr, nullptr, st, w.mask2, w.dact));   // pi (+ the sign masks and d(action)/d(pre-activation) for the backward)
+    {   // pi, the sign masks and d(action)/d(pre-activation) for the backward
+        fused3::RunArgs f = p.fused_args(fused3::MODE_ACTOR_SAVE, io->actor, w.aW2T, w.a_b2f, io->s, srs);
+        f.high = io->action_high; f.out = w.a2; f.mask_out = w.mask_a; f.mask2_out = w.mask2; f.dact_out = w.dact;
+        AVD_TRY(fused3::run(f, st));
+    }
     tm.mark("actor_fwd");
-    AVD_TRY(fused3::run(fused3::MODE_CRITIC_ACTION, f16, d, A, R, io->critic, co.total, w.cW2T, w.c_b2f, w.vtab, io->s, srs, 1, w.a2,
-                        nullptr, 0.f, 0.f, nullptr, nullptr, w.dpi, nullptr, nullptr, 1.0f, nullptr, io->loss, st));          // d(-mean q)/d pi
+    {   // d(-mean q)/d pi
+        fused3::RunArgs f = p.fused_args(fused3::MODE_CRITIC_ACTION, io->critic, w.cW2T, w.c_b2f, io->s, srs);
+        f.act = w.a2; f.vtab = w.vtab; f.out = w.dpi; f.loss = io->loss;
+        AVD_TRY(fused3::run(f, st));
+    }
     tm.mark("critic_action");
-    if (legacy_actor_bwd) {
-        AVD_TRY(fused3::run(fused3::MODE_ACTOR_BWD, f16, d, A, R, io->actor, ao.total, w.aW2T, w.a_b2f, nullptr, io->s, srs, 1, nullptr, nullptr, 0.f,
-                            io->action_high, nullptr, w.dpi, nullptr, w.mask_a, w.DZa, dm_a, w.sdq + A, nullptr, st));
-    } else {
+    {
         cudaStream_t sd = st;
         if (side) {    // branch A: the actor's backward tile beside the critic's backward pass
             AVD_CUDA_OK(cudaEventRecord(side->fork, st));
@@ -1886,8 +1850,11 @@ static int learn_fused3(const avd_learn_io* io, const Pass& p, const Workspace& 
     }
     tm.mark("actor_bwd");
     // ---- critic loss gradient on (s, a)                                             trainer.py:495-498
-    AVD_TRY(fused3::run(fused3::MODE_CRITIC_BWD, f16, d, A, R, io->critic, co.total, w.cW2T, w.c_b2f, nullptr, io->s, srs, 1, io->a, nullptr, 0.f, 0.f,
-                        w.y, nullptr, w.q, w.mask, DZ, dm_c, w.sdq, io->loss, st));
+    {
+        fused3::RunArgs f = p.fused_args(fused3::MODE_CRITIC_BWD, io->critic, w.cW2T, w.c_b2f, io->s, srs);
+        f.act = io->a; f.y = w.y; f.out = w.q; f.mask_out = w.mask; f.DZ_out = DZ; f.dm_scale = dm_c; f.sdq = w.sdq; f.loss = io->loss;
+        AVD_TRY(fused3::run(f, st));
+    }
     tm.mark("critic_bwd");
     // dgrad first, wgrad second: the unfold kernel then finds the 23 MB of partial G2 slices the weight-gradient CTAs have just written
     // still in L2 (after a dgrad pass, which streams 340 MB, it read them back from HBM)
@@ -1907,7 +1874,7 @@ static int learn_fused3(const avd_learn_io* io, const Pass& p, const Workspace& 
     }
     tm.mark("critic_unfold");
     // ---- actor loss gradient, second half
-    if (side && !legacy_actor_bwd) AVD_CUDA_OK(cudaStreamWaitEvent(st, side->join, 0));      // join A: the actor's backward tile is complete
+    if (side) AVD_CUDA_OK(cudaStreamWaitEvent(st, side->join, 0));      // join A: the actor's backward tile is complete
     AVD_TRY(p.dgrad3_only(w.DZa, w.aW2b, d.l1, Fp, w.mask_a, 8, w.xextT, w.G1a, dbm_a));
     tm.mark("actor_dgrad");
     AVD_TRY(wgrad3::run(f16, d, false, A, R, io->actor, ao.total, io->s, srs, nullptr, w.DZa, w.G2part_a, g2_agent, g2_cta, st));
@@ -1941,7 +1908,7 @@ extern "C" int avd_ddpg_learn(const avd_learn_io* io, void* stream) {
     const int F = d.l1 + d.la;
     Workspace w;
     const bool fz = fused_path(d, io->precision);   // persistent fused pass / dgrad / wgrad kernels
-    w.carve(io->workspace, d, A, N, fz, io->precision == 3 ? 3 : 1);
+    w.carve(io->workspace, d, A, N, fz, operand_planes(io->precision));
     const dim3 gl1b((unsigned)((R + kL1BwdRows - 1) / kL1BwdRows), A);
     const int64_t srs = io->s_stride ? io->s_stride : d.ns;      // row pitch of the state batches
     AVD_REQUIRE(srs >= d.ns, "s_stride %d is smaller than the state width %d", (int)io->s_stride, d.ns);

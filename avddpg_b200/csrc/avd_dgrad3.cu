@@ -13,18 +13,14 @@
 //
 // Warps: 0 issuer of the dR chunk MMAs, 18 issuer of the G1 / db2 MMAs, 1 TMA producer, 2..17 epilogue (TMEM lane quadrant = warp % 4, 32 of a chunk pair's 128 columns each).  TMEM: 3-slot ring of 128-column dR chunk pairs + 3 x 16 columns of G1 + 16 columns of
 // dz2^T xext, whose column 5 (xext's constant one) is the layer-2 bias gradient db2.
-#include <cudaTypedefs.h>
-
-#include <algorithm>
-
 #include "avd_common.cuh"
+#include "avd_learn_kernels.cuh"
 #include "avd_umma.cuh"
 
 namespace avd {
 namespace dgrad3 {
 
 using namespace umma;
-typedef __nv_bfloat16 bf16;
 
 constexpr int TILE_M = 128, L2N = 128, KB = 64, MAX_NC = 5, NRING = 3;
 constexpr int NUM_THREADS = 32 * 19;
@@ -288,38 +284,6 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) dgrad3_kernel(const __grid_con
     }
 }
 
-static PFN_cuTensorMapEncodeTiled encode_fn() {
-    static PFN_cuTensorMapEncodeTiled fn = nullptr;
-    if (!fn) {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<PFN_cuTensorMapEncodeTiled>(p);
-    }
-    return fn;
-}
-
-static int make_map(CUtensorMap* tm, const void* base, uint64_t inner, uint64_t rows, uint64_t batch, uint64_t pitch, uint64_t batch_stride,
-                    uint32_t box_rows) {
-    PFN_cuTensorMapEncodeTiled enc = encode_fn();
-    if (!enc) {
-        set_error("cuTensorMapEncodeTiled is not available from the driver");
-        return AVD_ERR_CUDA;
-    }
-    cuuint64_t dims[3] = {inner, rows, batch};
-    cuuint64_t strides[2] = {pitch * 2, batch_stride * 2};
-    cuuint32_t box[3] = {KB, box_rows, 1};
-    cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-        set_error("cuTensorMapEncodeTiled failed with %d (inner=%llu rows=%llu batch=%llu pitch=%llu)", (int)r, (unsigned long long)inner,
-                  (unsigned long long)rows, (unsigned long long)batch, (unsigned long long)pitch);
-        return AVD_ERR_CUDA;
-    }
-    return AVD_OK;
-}
-
 // DZ: 16-bit [A*R][128];  W2b: [A][F][128] folded layer-2 kernel W2'' = W2' diag(w3') (bf16, or with f16 = true everything fp16, W2b
 // scaled by a power of two s per agent and DZ by dm_scale: G1 / db2 then carry those factors, which the unfold kernel divides out);  mask: [A*R][mask_words];  xextT: bf16 [A][16][Rp]
 // (Rp = rows per agent rounded up to a multiple of 64);  G1: fp32 [A][ctas_per_agent][Fp][16] partial slices, one per CTA, plain
@@ -337,13 +301,13 @@ int run(bool f16, int A, int64_t R, int F, const bf16* DZ, const bf16* W2b, cons
         attr_set = true;
     }
     CUtensorMap tmW, tmDZ, tmXT;
-    if (int rc = make_map(&tmW, W2b, L2N, (uint64_t)F, (uint64_t)A, L2N, (uint64_t)F * L2N, 64)) return rc;
-    if (int rc = make_map(&tmDZ, DZ, L2N, (uint64_t)R, (uint64_t)A, L2N, (uint64_t)R * L2N, TILE_M)) return rc;
-    if (int rc = make_map(&tmXT, xextT, (uint64_t)R, 16, (uint64_t)A, (uint64_t)Rp, (uint64_t)16 * Rp, 16)) return rc;
+    if (int rc = make_tensor_map(&tmW, W2b, L2N, (uint64_t)F, (uint64_t)A, L2N, (uint64_t)F * L2N, KB, 64)) return rc;
+    if (int rc = make_tensor_map(&tmDZ, DZ, L2N, (uint64_t)R, (uint64_t)A, L2N, (uint64_t)R * L2N, KB, TILE_M)) return rc;
+    if (int rc = make_tensor_map(&tmXT, xextT, (uint64_t)R, 16, (uint64_t)A, (uint64_t)Rp, (uint64_t)16 * Rp, KB, 16)) return rc;
     Args g;
     g.A = A; g.F = F; g.NC = (F + 63) / 64; g.R = R; g.mask = mask; g.mask_words = mask_words; g.G1 = G1; g.Fp = Fp; g.db2 = db2; g.db2_stride = db2_stride;
     g.tiles_per_agent = (int)((R + TILE_M - 1) / TILE_M);
-    g.ctas_per_agent = std::max(1, std::min(g.tiles_per_agent, sm_count() / std::max(1, A)));      // == wgrad3::ctas_per_agent(A, R)
+    g.ctas_per_agent = ctas_per_agent(A, R);
     const unsigned grid = (unsigned)(g.ctas_per_agent * A);
     if (g.NC == 4 && !f16) AVD_CUDA_OK(launch_pdl(dgrad3_kernel<4, false>, dim3(grid), dim3(NUM_THREADS), SMEM_BYTES, st, tmW, tmDZ, tmXT, g));
     else if (!f16) AVD_CUDA_OK(launch_pdl(dgrad3_kernel<5, false>, dim3(grid), dim3(NUM_THREADS), SMEM_BYTES, st, tmW, tmDZ, tmXT, g));

@@ -19,19 +19,15 @@
 // warp % 4, column quarter = (warp - 1) / 4) running a software pipeline  convert(i+1) | pass2(i-1) | pass1(i)  so that
 // every MMA has a full stage of other work to hide behind.
 // Reference semantics: agent/model.py:19-37 (actor), 55-83 (critic); workers/trainer.py:489-506.
-#include <cudaTypedefs.h>
-
-#include <algorithm>
-
 #include "avd_common.cuh"
 #include "avd_ddpg_layout.cuh"
+#include "avd_learn_kernels.cuh"
 #include "avd_umma.cuh"
 
 namespace avd {
 namespace fused3 {
 
 using namespace umma;
-typedef __nv_bfloat16 bf16;
 
 constexpr int TILE_M = 128, L2N = 128, KB = 64, MAX_KB = 5, L1N = 256;
 constexpr int NCONS = 16;
@@ -56,11 +52,6 @@ constexpr int kVRows = 49, kVStride = 132, kVBrk = 64;
 static_assert((kVRows * kVStride + kVBrk) * 4 + 2 * 4 * TILE_M * 4 <= 2 * SLOT_BYTES, "V table + partial sums exceed the dz2-tile slots");
 static_assert(SMEM_BYTES <= 232448, "exceeds the 227 KB shared memory of an sm_100 CTA");
 
-// MODE_ACTOR_SAVE: the actor forward pass that ALSO keeps what its backward needs -- sign bits of z1 (40 B per row) and of
-// z2 + b2' (16 B), and d(action)/d(pre-activation) = high (1 - tanh^2) (4 B) -- so that the actor backward of the learn step is an
-// elementwise kernel (actor_dm_kernel, avd_ddpg.cu) instead of a second full forward pass (MODE_ACTOR_BWD, kept for reference).
-enum Mode { MODE_ACTOR_OUT = 0, MODE_TARGET = 1, MODE_Q = 2, MODE_CRITIC_BWD = 3, MODE_ACTOR_BWD = 4, MODE_CRITIC_ACTION = 5, MODE_ACTOR_SAVE = 6 };
-
 struct Args {
     avd_net_dims d;
     int A;
@@ -74,7 +65,6 @@ struct Args {
     const float* rew;           // MODE_TARGET
     float gamma, high;
     const float* y;             // MODE_CRITIC_BWD: TD targets
-    const float* dpi;           // MODE_ACTOR_BWD: d loss / d action
     float* out;                 // forward modes: [A*R]; MODE_CRITIC_ACTION: d loss / d action; MODE_CRITIC_BWD: q (nullable)
     uint32_t* mask_out;         // backward modes / MODE_ACTOR_SAVE: [A*R][mask_words] sign bits of z1 (column j of word w at bit 31-j)
     int mask_words;
@@ -122,9 +112,9 @@ __device__ __forceinline__ uint32_t pack2(bf16 a, bf16 b) {
 // 160 us, and a 0.5 % bias on every actor gradient from the two bf16 roundings); this is exact in fp32.
 template <int MODE, bool F16>
 __global__ void __launch_bounds__(NUM_THREADS, 1) fused3_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CUtensorMap tmDZ, Args g) {
-    constexpr bool CRITIC = MODE != MODE_ACTOR_OUT && MODE != MODE_ACTOR_BWD && MODE != MODE_ACTOR_SAVE;
+    constexpr bool CRITIC = MODE != MODE_ACTOR_OUT && MODE != MODE_ACTOR_SAVE;
     constexpr bool SAVE = MODE == MODE_ACTOR_SAVE;                               // forward pass that keeps its sign masks
-    constexpr bool BWD = MODE == MODE_CRITIC_BWD || MODE == MODE_ACTOR_BWD;      // full backward: masks, r1 / dz2 to HBM, U
+    constexpr bool BWD = MODE == MODE_CRITIC_BWD;                                // full backward: masks, r1 / dz2 to HBM, U
     constexpr bool ACTION = MODE == MODE_CRITIC_ACTION;                          // forward + d q / d action (V table)
     constexpr bool HAS_DZ = BWD;
     constexpr int NKB = CRITIC ? 5 : 4;
@@ -332,7 +322,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) fused3_kernel(const __grid_con
         // its use would put a full global-memory latency on the critical path of every tile.
         //   xs   : state row of the tile whose X buffer this thread's quarter writes at the end of its next convert()
         //   a_pf : action of the next tile whose action-branch columns this quarter converts
-        //   y_pf : reward / TD target / d loss/d action of the tile whose pass 2 comes next;  a_ag: action of the next pass1() (ACTION)
+        //   y_pf : reward / TD target of the tile whose pass 2 comes next;  a_ag: action of the next pass1() (ACTION)
         float xs[4] = {0.f, 0.f, 0.f, 0.f}, a_pf = 0.0f, y_pf = 0.0f, a_ag = 0.0f;
         auto xg_of = [&](int tc) { return CRITIC ? 2 * (1 - (tc & 1)) : (tc & 3); };      // quarter that stages tile tc + 2 during convert(tc)
         auto is_action_quarter = [&](int tc) { return CRITIC && (c4 >> 1) == (tc & 1); };   // quarters 2 (tc & 1), 2 (tc & 1) + 1
@@ -434,8 +424,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) fused3_kernel(const __grid_con
                 bool v0;
                 const int64_t n0 = rowinfo(tc, v0);
                 if (MODE == MODE_TARGET) { if (c4 == 0) y_pf = __ldg(g.rew + n0); }
-                else if (MODE == MODE_CRITIC_BWD) y_pf = __ldg(g.y + n0);
-                else y_pf = __ldg(g.dpi + n0);
+                else y_pf = __ldg(g.y + n0);
             }
             const float* vrow = vtab_s;          // ACTION: this row's V[k(a)] (its 32 columns), k(a) = breakpoints below the action
             if (ACTION) {
@@ -527,17 +516,11 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) fused3_kernel(const __grid_con
                 if (lane == 0) mbar_arrive(&acc_empty[buf]);
                 return;
             }
-            float dq = 0.0f;
-            if (MODE == MODE_CRITIC_BWD) {
-                const float diff = qv - yv;
-                dq = valid ? 2.0f * diff * invR : 0.0f;                              // d mean((y-q)^2) / dq      trainer.py:496
-                if (c4 == 0) {
-                    if (valid) loss_acc = fmaf(diff, diff * invR, loss_acc);
-                    if (valid && g.out) g.out[nrow] = qv;
-                }
-            } else if (MODE == MODE_ACTOR_BWD) {
-                const float t = tanhf(qv);
-                dq = valid ? yv * g.high * (1.0f - t * t) : 0.0f;                    // through high * tanh(.)    model.py:36-37
+            const float diff = qv - yv;
+            const float dq = valid ? 2.0f * diff * invR : 0.0f;                      // d mean((y-q)^2) / dq      trainer.py:496
+            if (c4 == 0) {
+                if (valid) loss_acc = fmaf(diff, diff * invR, loss_acc);
+                if (valid && g.out) g.out[nrow] = qv;
             }
             if (c4 == 0) sdq_acc += dq;
             float v[32];
@@ -589,7 +572,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) fused3_kernel(const __grid_con
         if ((HAS_DZ || ACTION) && c4 == 0) {
             const float sl = warp_sum(loss_acc), sd = warp_sum(sdq_acc);
             if (lane == 0) {
-                if (g.loss && MODE != MODE_ACTOR_BWD) atomicAdd(g.loss + 2 * agent + (MODE == MODE_CRITIC_BWD ? 0 : 1), sl);
+                if (g.loss) atomicAdd(g.loss + 2 * agent + (MODE == MODE_CRITIC_BWD ? 0 : 1), sl);
                 if (BWD) atomicAdd(g.sdq + agent, sd);
             }
         }
@@ -600,38 +583,6 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) fused3_kernel(const __grid_con
         tc_fence_after();
         tmem_dealloc(tmem_base, 512);
     }
-}
-
-static PFN_cuTensorMapEncodeTiled encode_fn() {
-    static PFN_cuTensorMapEncodeTiled fn = nullptr;
-    if (!fn) {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<PFN_cuTensorMapEncodeTiled>(p);
-    }
-    return fn;
-}
-
-// 3-D bf16 map {inner, rows, batch}, box {64, 128, 1}, 128-byte swizzle
-static int make_map(CUtensorMap* tm, const void* base, uint64_t inner, uint64_t rows, uint64_t batch, uint64_t pitch, uint64_t batch_stride) {
-    PFN_cuTensorMapEncodeTiled enc = encode_fn();
-    if (!enc) {
-        set_error("cuTensorMapEncodeTiled is not available from the driver");
-        return AVD_ERR_CUDA;
-    }
-    cuuint64_t dims[3] = {inner, rows, batch};
-    cuuint64_t strides[2] = {pitch * 2, batch_stride * 2};
-    cuuint32_t box[3] = {KB, TILE_M, 1};
-    cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-        set_error("cuTensorMapEncodeTiled failed with %d (inner=%llu rows=%llu batch=%llu pitch=%llu)", (int)r, (unsigned long long)inner,
-                  (unsigned long long)rows, (unsigned long long)batch, (unsigned long long)pitch);
-        return AVD_ERR_CUDA;
-    }
-    return AVD_OK;
 }
 
 bool supported(const avd_net_dims& d) {       // la <= 48: the V table of the critic-action pass has la + 1 <= kVRows rows
@@ -657,45 +608,44 @@ static int launch(bool f16, const CUtensorMap& tmW, const CUtensorMap& tmDZ, con
     return f16 ? launch2<MODE, true>(tmW, tmDZ, g, grid, st) : launch2<MODE, false>(tmW, tmDZ, g, grid, st);
 }
 
-// One pass.  W2T: 16-bit [A][128][F] folded layer-2 kernel (K-major; bf16, or fp16 with f16 = true), b2f: [A][128]
-// (pack_fold_kernel / pack_fold4_kernel).  MODE_CRITIC_ACTION: vtab [A][vtab_floats()] from critic_vtab_kernel.
-// Backward modes: mask_out [A*R][2*ceil(F/64)] sign masks of z1, DZ_out: 16-bit [A*R][128] = dm_scale * dq [z2 + b2' > 0], sdq [A] accumulated into.
-int run(int mode, bool f16, const avd_net_dims& d, int A, int64_t R, const float* params, int64_t pstride, const bf16* W2T, const float* b2f,
-        const float* vtab, const float* s, int64_t s_rs, int64_t s_cs, const float* act, const float* rew, float gamma, float high, const float* y,
-        const float* dpi, float* out, uint32_t* mask_out, bf16* DZ_out, float dm_scale, float* sdq, float* loss, cudaStream_t st,
-        uint32_t* mask2_out, float* dact_out) {
+// One pass (the buffers are described at RunArgs, avd_learn_kernels.cuh).
+int run(const RunArgs& a, cudaStream_t st) {
+    const avd_net_dims& d = a.d;
     if (!supported(d)) {
         set_error("fused pass kernel does not support these layer sizes");
         return AVD_ERR_UNSUPPORTED;
     }
-    const bool critic = mode != MODE_ACTOR_OUT && mode != MODE_ACTOR_BWD && mode != MODE_ACTOR_SAVE;
-    const bool bwd = mode == MODE_CRITIC_BWD || mode == MODE_ACTOR_BWD;
+    const int mode = a.mode;
+    const bool critic = mode != MODE_ACTOR_OUT && mode != MODE_ACTOR_SAVE;
+    const bool bwd = mode == MODE_CRITIC_BWD;
     const int F = critic ? d.l1 + d.la : d.l1;
-    AVD_REQUIRE(params && W2T && b2f && s, "null buffer");
-    AVD_REQUIRE(A >= 1 && R >= 1 && R < (int64_t)1 << 31, "rows per agent must fit the 32-bit TMA coordinates");
-    AVD_REQUIRE(!critic || act, "critic passes need actions");
-    AVD_REQUIRE(!bwd || (mask_out && DZ_out && sdq), "backward passes need mask / dz2 / sdq outputs");
-    AVD_REQUIRE(mode != MODE_CRITIC_ACTION || (vtab && d.la < kVRows), "the critic-action pass needs its V table (la <= %d)", kVRows - 1);
-    AVD_REQUIRE(bwd || out, "null output");
-    AVD_REQUIRE(mode != MODE_ACTOR_SAVE || (mask_out && mask2_out && dact_out), "MODE_ACTOR_SAVE needs the mask / d(action) outputs");
+    AVD_REQUIRE(a.params && a.W2T && a.b2f && a.s, "null buffer");
+    AVD_REQUIRE(a.A >= 1 && a.R >= 1 && a.R < (int64_t)1 << 31, "rows per agent must fit the 32-bit TMA coordinates");
+    AVD_REQUIRE(!critic || a.act, "critic passes need actions");
+    AVD_REQUIRE(!bwd || (a.mask_out && a.DZ_out && a.sdq), "backward passes need mask / dz2 / sdq outputs");
+    AVD_REQUIRE(mode != MODE_CRITIC_ACTION || (a.vtab && d.la < kVRows), "the critic-action pass needs its V table (la <= %d)", kVRows - 1);
+    AVD_REQUIRE(bwd || a.out, "null output");
+    AVD_REQUIRE(mode != MODE_ACTOR_SAVE || (a.mask_out && a.mask2_out && a.dact_out), "MODE_ACTOR_SAVE needs the mask / d(action) outputs");
+    const int A = a.A;
+    const int64_t R = a.R;
     CUtensorMap tmW, tmDZ;
-    if (int rc = make_map(&tmW, W2T, (uint64_t)F, L2N, (uint64_t)A, (uint64_t)F, (uint64_t)F * L2N)) return rc;
+    if (int rc = make_tensor_map(&tmW, a.W2T, (uint64_t)F, L2N, (uint64_t)A, (uint64_t)F, (uint64_t)F * L2N, KB, TILE_M)) return rc;
     tmDZ = tmW;
     if (bwd)
-        if (int rc = make_map(&tmDZ, DZ_out, L2N, (uint64_t)R, (uint64_t)A, L2N, (uint64_t)R * L2N)) return rc;
+        if (int rc = make_tensor_map(&tmDZ, a.DZ_out, L2N, (uint64_t)R, (uint64_t)A, L2N, (uint64_t)R * L2N, KB, TILE_M)) return rc;
     Args g;
-    g.d = d; g.A = A; g.R = R; g.params = params; g.pstride = pstride; g.b2f = b2f; g.s = s; g.s_rs = s_rs; g.s_cs = s_cs; g.act = act;
-    g.rew = rew; g.gamma = gamma; g.high = high; g.y = y; g.dpi = dpi; g.out = out; g.mask_out = mask_out; g.mask_words = 2 * ((F + KB - 1) / KB);
-    g.vtab = vtab; g.dm_scale = dm_scale; g.sdq = sdq; g.loss = loss; g.mask2_out = mask2_out; g.dact_out = dact_out;
+    g.d = d; g.A = A; g.R = R; g.params = a.params; g.pstride = a.pstride; g.b2f = a.b2f; g.s = a.s; g.s_rs = a.s_rs; g.s_cs = a.s_cs; g.act = a.act;
+    g.rew = a.rew; g.gamma = a.gamma; g.high = a.high; g.y = a.y; g.out = a.out; g.mask_out = a.mask_out; g.mask_words = 2 * ((F + KB - 1) / KB);
+    g.vtab = a.vtab; g.dm_scale = a.dm_scale; g.sdq = a.sdq; g.loss = a.loss; g.mask2_out = a.mask2_out; g.dact_out = a.dact_out;
     g.tiles_per_agent = (int)((R + TILE_M - 1) / TILE_M);
-    g.ctas_per_agent = std::max(1, std::min(g.tiles_per_agent, sm_count() / std::max(1, A)));
+    g.ctas_per_agent = ctas_per_agent(A, R);
     const dim3 grid((unsigned)(g.ctas_per_agent * A));
+    const bool f16 = a.f16;
     switch (mode) {
         case MODE_ACTOR_OUT: return launch<MODE_ACTOR_OUT>(f16, tmW, tmDZ, g, grid, st);
         case MODE_TARGET: return launch<MODE_TARGET>(f16, tmW, tmDZ, g, grid, st);
         case MODE_Q: return launch<MODE_Q>(f16, tmW, tmDZ, g, grid, st);
         case MODE_CRITIC_BWD: return launch<MODE_CRITIC_BWD>(f16, tmW, tmDZ, g, grid, st);
-        case MODE_ACTOR_BWD: return launch<MODE_ACTOR_BWD>(f16, tmW, tmDZ, g, grid, st);
         case MODE_CRITIC_ACTION: return launch<MODE_CRITIC_ACTION>(f16, tmW, tmDZ, g, grid, st);
         case MODE_ACTOR_SAVE: return launch<MODE_ACTOR_SAVE>(f16, tmW, tmDZ, g, grid, st);
     }

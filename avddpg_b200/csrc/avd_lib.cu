@@ -1,4 +1,5 @@
-// avd_lib.cu -- library-level entry points: ABI version, last-error text, device probe.
+// avd_lib.cu -- library-level entry points: ABI version, last-error text, device probe; the tensor-map encoder.
+#include <cudaTypedefs.h>
 #include <cstdlib>
 #include <stdarg.h>
 #include <string.h>
@@ -6,6 +7,7 @@
 #include <atomic>
 
 #include "avd_common.cuh"
+#include "avd_umma.cuh"
 
 namespace avd {
 
@@ -41,6 +43,34 @@ int sm_count() {
             return 148;  // B200; only reached when no device is visible (launches then fail loudly)
     }
     return cached;
+}
+
+int umma::make_tensor_map(CUtensorMap* map, const void* base, uint64_t inner, uint64_t rows, uint64_t batch, uint64_t pitch,
+                          uint64_t batch_stride, uint32_t box_inner, uint32_t box_rows) {
+    static PFN_cuTensorMapEncodeTiled enc = nullptr;
+    if (!enc) {
+        void* p = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
+            enc = reinterpret_cast<PFN_cuTensorMapEncodeTiled>(p);
+    }
+    if (!enc) {
+        set_error("cuTensorMapEncodeTiled is not available from the driver");
+        return AVD_ERR_CUDA;
+    }
+    cuuint64_t dims[3] = {inner, rows, batch};
+    cuuint64_t strides[2] = {pitch * 2, batch_stride * 2};
+    if (batch == 1 && strides[1] == 0) strides[1] = pitch * 2 * rows;
+    cuuint32_t box[3] = {box_inner, box_rows, 1};
+    cuuint32_t estr[3] = {1, 1, 1};
+    CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                     CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) {
+        set_error("cuTensorMapEncodeTiled failed with %d (inner=%llu rows=%llu batch=%llu pitch=%llu)", (int)r, (unsigned long long)inner,
+                  (unsigned long long)rows, (unsigned long long)batch, (unsigned long long)pitch);
+        return AVD_ERR_CUDA;
+    }
+    return AVD_OK;
 }
 
 }  // namespace avd

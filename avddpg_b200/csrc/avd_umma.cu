@@ -21,11 +21,10 @@
 // virtual K blocks, one (A plane, B plane) pair each, that stream through the 4-stage ring like ordinary K blocks.  hi.hi accumulates into one TMEM tile and the five correction products into a
 // second one, summed in the epilogue: the MMA's fp32 accumulation rounds once per instruction, and sharing one tile would
 // round the large sum six times per K step instead of once (measured: ReLU sign flips of the learn step against fp32).
-#include <cudaTypedefs.h>
-
 #include <utility>
 
 #include "avd_common.cuh"
+#include "avd_learn_kernels.cuh"
 #include "avd_umma.cuh"
 
 namespace avd {
@@ -207,41 +206,6 @@ __global__ void __launch_bounds__(NUM_THREADS, PLANES == 3 ? 2 : (STAGES <= 2) ?
     }
 }
 
-
-static PFN_cuTensorMapEncodeTiled encode_fn() {
-    static PFN_cuTensorMapEncodeTiled fn = nullptr;
-    if (!fn) {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<PFN_cuTensorMapEncodeTiled>(p);
-    }
-    return fn;
-}
-
-// 3-D bf16 tensor map {inner, rows, batch} with a {box_inner, box_rows, 1} box and 128-byte swizzle
-static int make_map(CUtensorMap* map, const void* base, uint64_t inner, uint64_t rows, uint64_t batch, uint64_t ld, uint64_t batch_stride,
-                    uint32_t box_inner, uint32_t box_rows) {
-    PFN_cuTensorMapEncodeTiled enc = encode_fn();
-    if (!enc) {
-        set_error("cuTensorMapEncodeTiled is not available from the driver");
-        return AVD_ERR_CUDA;
-    }
-    cuuint64_t dims[3] = {inner, rows, batch};
-    cuuint64_t strides[2] = {ld * 2, batch_stride * 2};
-    if (batch == 1 && strides[1] == 0) strides[1] = ld * 2 * rows;
-    cuuint32_t box[3] = {box_inner, box_rows, 1};
-    cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-        set_error("cuTensorMapEncodeTiled failed with %d (inner=%llu rows=%llu batch=%llu ld=%llu)", (int)r, (unsigned long long)inner,
-                  (unsigned long long)rows, (unsigned long long)batch, (unsigned long long)ld);
-        return AVD_ERR_CUDA;
-    }
-    return AVD_OK;
-}
-
 // planes = 1: plain 16-bit operands; planes = 3: bf16 hi / mid / lo planes, plane p of batch b at A + (p * batch + b) * a_batch
 static int launch_gemm(int layout, int batch, int M, int N, int K, const void* A, int64_t lda, int64_t a_batch, const void* B, int64_t ldb,
                        int64_t b_batch, float* C, int64_t ldc, int64_t c_batch, int splitk, int a_fmt, int b_fmt, int planes, cudaStream_t st) {
@@ -276,13 +240,13 @@ static int launch_gemm(int layout, int batch, int M, int N, int K, const void* A
     if (g.n_fastest) std::swap(grid.x, grid.y);
     const int zmaps = planes * batch;
     if (layout == 0) {
-        if (int rc = make_map(&tmA, A, K, M, zmaps, lda, a_batch, BK, BM)) return rc;
-        if (int rc = make_map(&tmB, B, K, N, zmaps, ldb, b_batch, BK, BN)) return rc;
+        if (int rc = make_tensor_map(&tmA, A, K, M, zmaps, lda, a_batch, BK, BM)) return rc;
+        if (int rc = make_tensor_map(&tmB, B, K, N, zmaps, ldb, b_batch, BK, BN)) return rc;
         if (planes == 3) gemm_bf16_kernel<false, STAGES_TN3, 128, 3><<<grid, NUM_THREADS, smem_bytes(STAGES_TN3, BN, 3), st>>>(tmA, tmB, g);
         else gemm_bf16_kernel<false, STAGES_TN, 128><<<grid, NUM_THREADS, smem_bytes(STAGES_TN), st>>>(tmA, tmB, g);
     } else {
-        if (int rc = make_map(&tmA, A, M, K, zmaps, lda, a_batch, 64, BK)) return rc;
-        if (int rc = make_map(&tmB, B, N, K, zmaps, ldb, b_batch, 64, BK)) return rc;
+        if (int rc = make_tensor_map(&tmA, A, M, K, zmaps, lda, a_batch, 64, BK)) return rc;
+        if (int rc = make_tensor_map(&tmB, B, N, K, zmaps, ldb, b_batch, 64, BK)) return rc;
         if (narrow) gemm_bf16_kernel<true, STAGES_NT, 64><<<grid, NUM_THREADS, smem_bytes(STAGES_NT, 64), st>>>(tmA, tmB, g);
         else gemm_bf16_kernel<true, STAGES_NT, 128><<<grid, NUM_THREADS, smem_bytes(STAGES_NT), st>>>(tmA, tmB, g);
     }
@@ -300,15 +264,11 @@ int gemm_f16kind(int layout, int batch, int M, int N, int K, const void* A, int6
     return launch_gemm(layout, batch, M, N, K, A, lda, a_batch, B, ldb, b_batch, C, ldc, c_batch, splitk, a_fmt, b_fmt, 1, st);
 }
 
-int gemm_bf16x3(int layout, int batch, int M, int N, int K, const void* A, int64_t lda, int64_t a_batch, const void* B, int64_t ldb,
-                int64_t b_batch, float* C, int64_t ldc, int64_t c_batch, int splitk, cudaStream_t st) {
-    AVD_REQUIRE(a_batch > 0 && b_batch > 0, "split operands need positive batch strides (plane p of batch b starts at (p * batch + b) * stride)");
-    return launch_gemm(layout, batch, M, N, K, A, lda, a_batch, B, ldb, b_batch, C, ldc, c_batch, splitk, (int)FMT_BF16, (int)FMT_BF16, 3, st);
-}
-
-int gemm_bf16(int layout, int batch, int M, int N, int K, const void* A, int64_t lda, int64_t a_batch, const void* B, int64_t ldb,
+int gemm_bf16(int planes, int layout, int batch, int M, int N, int K, const void* A, int64_t lda, int64_t a_batch, const void* B, int64_t ldb,
               int64_t b_batch, float* C, int64_t ldc, int64_t c_batch, int splitk, cudaStream_t st) {
-    return gemm_f16kind(layout, batch, M, N, K, A, lda, a_batch, B, ldb, b_batch, C, ldc, c_batch, splitk, (int)FMT_BF16, (int)FMT_BF16, st);
+    AVD_REQUIRE(planes == 1 || (a_batch > 0 && b_batch > 0),
+                "split operands need positive batch strides (plane p of batch b starts at (p * batch + b) * stride)");
+    return launch_gemm(layout, batch, M, N, K, A, lda, a_batch, B, ldb, b_batch, C, ldc, c_batch, splitk, (int)FMT_BF16, (int)FMT_BF16, planes, st);
 }
 
 }  // namespace umma
@@ -323,11 +283,11 @@ extern "C" int avd_gemm_f16kind(int layout, int batch, int M, int N, int K, cons
 
 extern "C" int avd_gemm_bf16(int layout, int batch, int M, int N, int K, const void* A, int64_t lda, int64_t a_batch, const void* B,
                              int64_t ldb, int64_t b_batch, float* C, int64_t ldc, int64_t c_batch, int splitk, void* stream) {
-    return avd::umma::gemm_bf16(layout, batch, M, N, K, A, lda, a_batch, B, ldb, b_batch, C, ldc, c_batch, splitk, (cudaStream_t)stream);
+    return avd::umma::gemm_bf16(1, layout, batch, M, N, K, A, lda, a_batch, B, ldb, b_batch, C, ldc, c_batch, splitk, (cudaStream_t)stream);
 }
 
 extern "C" int avd_gemm_bf16x3(int layout, int batch, int M, int N, int K, const void* A_planes, int64_t lda, int64_t a_batch, const void* B_planes,
                                int64_t ldb, int64_t b_batch, float* C, int64_t ldc, int64_t c_batch, int splitk, void* stream) {
-    return avd::umma::gemm_bf16x3(layout, batch, M, N, K, A_planes, lda, a_batch, B_planes, ldb, b_batch, C, ldc, c_batch, splitk,
-                                  (cudaStream_t)stream);
+    return avd::umma::gemm_bf16(3, layout, batch, M, N, K, A_planes, lda, a_batch, B_planes, ldb, b_batch, C, ldc, c_batch, splitk,
+                                (cudaStream_t)stream);
 }

@@ -50,6 +50,11 @@ __device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarr
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
 // ---- TMA -----------------------------------------------------------------------------------------
+// Host: 3-D bf16 tensor map {inner, rows, batch} with a {box_inner, box_rows, 1} box and 128-byte swizzle; pitch and batch_stride
+// in elements (a single batch may pass batch_stride = 0).  Returns AVD_OK, or AVD_ERR_CUDA with the error text set (avd_lib.cu).
+int make_tensor_map(CUtensorMap* map, const void* base, uint64_t inner, uint64_t rows, uint64_t batch, uint64_t pitch, uint64_t batch_stride,
+                    uint32_t box_inner, uint32_t box_rows);
+
 __device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap* m) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(m)) : "memory");
 }

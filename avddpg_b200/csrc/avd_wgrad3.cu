@@ -21,19 +21,15 @@
 // TMEM: the accumulator is G2^T -- lane = layer-2 unit j, column = feature f (the dz2 tile is the MN-major A operand, the r1 slab
 // the MN-major B operand) -- 256 columns for the state features + 64 for the action branch (N = 64 products instead of a third
 // 128-wide slab), which leaves a ring of four (actor) / three (critic) 64-column z1 entries.
-#include <cudaTypedefs.h>
-
-#include <algorithm>
-
 #include "avd_common.cuh"
 #include "avd_ddpg_layout.cuh"
+#include "avd_learn_kernels.cuh"
 #include "avd_umma.cuh"
 
 namespace avd {
 namespace wgrad3 {
 
 using namespace umma;
-typedef __nv_bfloat16 bf16;
 
 constexpr int TILE_M = 128, L2N = 128, KB = 64, SLAB = 128;
 constexpr int NCONV = 16;                                   // converter warps: four teams of four (one per TMEM lane quadrant), 64 columns each
@@ -344,23 +340,6 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) wgrad3_kernel(const __grid_con
     }
 }
 
-static PFN_cuTensorMapEncodeTiled encode_fn() {
-    static PFN_cuTensorMapEncodeTiled fn = nullptr;
-    if (!fn) {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<PFN_cuTensorMapEncodeTiled>(p);
-    }
-    return fn;
-}
-
-// Persistent CTAs per agent for R rows (shared with the dgrad kernel so that both produce the same number of partial slices)
-int ctas_per_agent(int A, int64_t R) {
-    const int tiles = (int)((R + TILE_M - 1) / TILE_M);
-    return std::max(1, std::min(tiles, sm_count() / std::max(1, A)));
-}
-
 // out: every CTA (agent, cta) stores its partial G2 (row-major [F][128] fp32, rows < F) at out + agent*out_agent_stride +
 // cta*out_cta_stride -- no atomics: the 37 x 4 CTAs of the C2 case would otherwise serialise 7 M atomic adds on 160 k
 // addresses (a quarter of the kernel time).  The caller sums the ctas_per_agent(A, R) slices.  DZ: bf16 [A*R][128].
@@ -369,11 +348,6 @@ int run(bool f16, const avd_net_dims& d, bool critic, int A, int64_t R, const fl
     AVD_REQUIRE(d.l1 == 256 && d.l2 == L2N && d.ns >= 1 && d.ns <= 4 && (!critic || (d.la >= 8 && d.la <= 64)), "unsupported layer sizes for the fused wgrad kernel");
     AVD_REQUIRE(params && s && DZ && out && (!critic || act), "null buffer");
     AVD_REQUIRE(out_agent_stride % 4 == 0 && out_cta_stride % 4 == 0 && ((uintptr_t)out & 15) == 0, "partial G2 slices must be 16-byte aligned");
-    PFN_cuTensorMapEncodeTiled enc = encode_fn();
-    if (!enc) {
-        set_error("cuTensorMapEncodeTiled is not available from the driver");
-        return AVD_ERR_CUDA;
-    }
     static bool attr_set = false;
     if (!attr_set) {
         AVD_CUDA_OK(cudaFuncSetAttribute(wgrad3_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
@@ -381,16 +355,7 @@ int run(bool f16, const avd_net_dims& d, bool critic, int A, int64_t R, const fl
         attr_set = true;
     }
     CUtensorMap tm;
-    cuuint64_t dims[3] = {L2N, (cuuint64_t)R, (cuuint64_t)A};
-    cuuint64_t strides[2] = {L2N * 2, (cuuint64_t)R * L2N * 2};
-    cuuint32_t box[3] = {KB, TILE_M, 1};
-    cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = enc(&tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<bf16*>(DZ), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-        set_error("cuTensorMapEncodeTiled(dz2) failed with %d", (int)r);
-        return AVD_ERR_CUDA;
-    }
+    if (int rc = make_tensor_map(&tm, DZ, L2N, (uint64_t)R, (uint64_t)A, L2N, (uint64_t)R * L2N, KB, TILE_M)) return rc;
     Args g;
     g.d = d; g.critic = critic ? 1 : 0; g.A = A; g.FT = critic ? 3 : 2; g.R = R; g.params = params; g.pstride = pstride; g.s = s; g.s_rs = s_rs; g.act = act;
     g.out = out; g.out_agent_stride = out_agent_stride; g.out_cta_stride = out_cta_stride;

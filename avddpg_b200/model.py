@@ -193,9 +193,8 @@ class _Model:
         np.savez(path if str(path).endswith(".npz") else str(path) + ".npz",
                  **{f"{i:02d}_{n}": w for i, (n, w) in enumerate(zip(self.bank.weight_names, self.get_weights()))})
 
-    def _workspace(self, rows, width):
-        d = self.bank.dims
-        need = rows * width * 4 + (d.l1 + d.la) * d.l2 * 2 + 1024
+    def _workspace(self, rows, critic):
+        need = _lib.load().avd_forward_workspace_bytes(C.byref(self.bank.dims), 1, rows, int(critic), 0)
         if self._ws is None or self._ws.numel() < need:
             self._ws = torch.empty(need, dtype=torch.uint8, device=self.bank.flat.device)
         return self._ws
@@ -207,7 +206,7 @@ class Actor(_Model):
                             dtype=torch.float32, device=self.bank.flat.device).reshape(-1, self.bank.dims.ns).contiguous()
         d, n = self.bank.dims, s.shape[0]
         out = torch.empty(n, 1, dtype=torch.float32, device=s.device)
-        ws = self._workspace(n, d.l1 + d.l2)
+        ws = self._workspace(n, critic=False)
         _lib.check(_lib.load().avd_actor_forward(C.byref(d), 1, n, _lib.ptr(self.bank.flat), _lib.ptr(s), d.ns, 1,
                                                  float(self.high_bound), _lib.ptr(out), _lib.ptr(ws), ws.numel(), 0,
                                                  _lib.current_stream()))
@@ -225,7 +224,7 @@ class Critic(_Model):
                             dtype=torch.float32, device=dev).reshape(-1).contiguous()
         n = s.shape[0]
         q = torch.empty(n, 1, dtype=torch.float32, device=dev)
-        ws = self._workspace(n, d.l1 + d.la + d.l2)
+        ws = self._workspace(n, critic=True)
         _lib.check(_lib.load().avd_critic_forward(C.byref(d), 1, n, _lib.ptr(self.bank.flat), _lib.ptr(s), _lib.ptr(a),
                                                   _lib.ptr(q), _lib.ptr(ws), ws.numel(), 0, _lib.current_stream()))
         return q
