@@ -730,36 +730,64 @@ struct FoldOff {
     int l1;                               // features < l1 use set 0
 };
 
+// b2'[j] = b2[j] + sum_f sh1[f] W2[f][j] of one agent in a fixed order: warp fy sums features fy, fy + 8, ..., then warp 0 adds
+// the eight partial sums in warp order.  Called by all 256 threads of the CTAs of feature slab 0 only: adding per-slab partial sums
+// with atomics made b2', and with it every output of the pass, depend on the order in which CTAs finished (the same weights at two
+// agent slots, or in two calls, gave outputs a few ulp apart).  These CTAs are the tail of the launch, so sh1 is computed once per
+// feature into shared memory and every W2 load of a thread is issued before the first is used.  F <= kFoldMaxF: the fused path
+// (fused3::supported) has F = 256 + la <= 304.
+constexpr int kFoldMaxF = 320;
+__device__ __forceinline__ void fold_bias(const float* __restrict__ P, const FoldOff& o, int F, int l2, int j, int fy, float* __restrict__ b2f) {
+    __shared__ float red[8][32];
+    __shared__ float sh_s[kFoldMaxF];
+    for (int f = threadIdx.x; f < F; f += blockDim.x) {
+        const bool st = f < o.l1;
+        const int c = st ? f : f - o.l1;
+        const float sc = P[(st ? o.g[0] : o.g[1]) + c] / sqrtf(P[(st ? o.var[0] : o.var[1]) + c] + kBnEps);
+        sh_s[f] = P[(st ? o.be[0] : o.be[1]) + c] - P[(st ? o.mu[0] : o.mu[1]) + c] * sc;
+    }
+    float w[kFoldMaxF / 8];
+#pragma unroll
+    for (int k = 0; k < kFoldMaxF / 8; ++k) {
+        const int f = fy + 8 * k;
+        w[k] = (j < l2 && f < F) ? P[o.W2 + (int64_t)f * l2 + j] : 0.0f;
+    }
+    __syncthreads();
+    float acc = 0.0f;
+#pragma unroll
+    for (int k = 0; k < kFoldMaxF / 8; ++k) {
+        const int f = fy + 8 * k;
+        if (f < F) acc += sh_s[f] * w[k];
+    }
+    red[fy][threadIdx.x & 31] = acc;
+    __syncthreads();
+    if (fy == 0 && j < l2) {
+        float t = P[o.b2 + j];
+#pragma unroll
+        for (int k = 0; k < 8; ++k) t += red[k][threadIdx.x];
+        *b2f = t;
+    }
+}
+
 __global__ void __launch_bounds__(256) pack_fold_kernel(const float* __restrict__ params, int64_t pstride, FoldOff o, int F, int l2,
                                                         bf16* __restrict__ W2b, bf16* __restrict__ W2T, float* __restrict__ b2f, int f16) {
     // grid: (l2/32 column slabs, feature slabs of 8, agents); thread (fy, j) owns feature blockIdx.y*8 + fy, column j.
-    // b2f must be zero on entry: every CTA adds its partial sum, the first feature slab also adds b2.
+    // The CTAs of the first feature slab also write b2f (fold_bias).
     const int agent = blockIdx.z;
     const float* P = params + (int64_t)agent * pstride;
     const int j = blockIdx.x * 32 + (threadIdx.x & 31);
     const int fy = threadIdx.x >> 5;
     const int f = blockIdx.y * 8 + fy;
-    __shared__ float red[8][32];
-    float acc = 0.0f;
     if (j < l2 && f < F) {
         const bool st = f < o.l1;
         const int c = st ? f : f - o.l1;
         const float sc = P[(st ? o.g[0] : o.g[1]) + c] / sqrtf(P[(st ? o.var[0] : o.var[1]) + c] + kBnEps);
-        const float sh = P[(st ? o.be[0] : o.be[1]) + c] - P[(st ? o.mu[0] : o.mu[1]) + c] * sc;
         const float w = P[o.W2 + (int64_t)f * l2 + j];
         const bf16 v = to_op16(sc * w, f16);
         if (W2b) W2b[((int64_t)agent * F + f) * l2 + j] = v;
         W2T[((int64_t)agent * l2 + j) * F + f] = v;
-        acc = sh * w;
     }
-    red[fy][threadIdx.x & 31] = acc;
-    __syncthreads();
-    if (fy == 0 && j < l2) {
-        float t = blockIdx.y == 0 ? P[o.b2 + j] : 0.0f;
-#pragma unroll
-        for (int k = 0; k < 8; ++k) t += red[k][threadIdx.x];
-        atomicAdd(b2f + (int64_t)agent * l2 + j, t);
-    }
+    if (blockIdx.y == 0) fold_bias(P, o, F, l2, j, fy, b2f + (int64_t)agent * l2 + j);
 }
 
 // The four networks of a learn step (target actor, target critic, critic, actor) in ONE launch: blockIdx.z = job * A + agent.
@@ -809,13 +837,10 @@ __device__ __forceinline__ void pack_fold4_body(const FoldJobs& jobs, int A, int
     const int j = bx * 32 + (threadIdx.x & 31);
     const int fy = threadIdx.x >> 5;
     const int f = by * 8 + fy;
-    __shared__ float red[8][32];
-    float acc = 0.0f;
     if (j < l2 && f < F) {
         const bool st = f < o.l1;
         const int c = st ? f : f - o.l1;
         const float sc = P[(st ? o.g[0] : o.g[1]) + c] / sqrtf(P[(st ? o.var[0] : o.var[1]) + c] + kBnEps);
-        const float sh = P[(st ? o.be[0] : o.be[1]) + c] - P[(st ? o.mu[0] : o.mu[1]) + c] * sc;
         const float w = P[o.W2 + (int64_t)f * l2 + j];
         // the backward tile carries dq [z2 > 0] without the head weight (avd_fused3.cu): dR = dm (W2' diag(w3'))^T
         if (jb.W2b) {
@@ -823,16 +848,8 @@ __device__ __forceinline__ void pack_fold4_body(const FoldJobs& jobs, int A, int
             jb.W2b[((int64_t)agent * F + f) * l2 + j] = to_op16(sc * w * w3p, f16);
         }
         jb.W2T[((int64_t)agent * l2 + j) * F + f] = to_op16(sc * w, f16);
-        acc = sh * w;
     }
-    red[fy][threadIdx.x & 31] = acc;
-    __syncthreads();
-    if (fy == 0 && j < l2) {
-        float t = by == 0 ? P[o.b2 + j] : 0.0f;
-#pragma unroll
-        for (int k = 0; k < 8; ++k) t += red[k][threadIdx.x];
-        atomicAdd(jb.b2f + (int64_t)agent * l2 + j, t);
-    }
+    if (by == 0) fold_bias(P, o, F, l2, j, fy, jb.b2f + (int64_t)agent * l2 + j);
 }
 
 // xextT[agent][c][r] (bf16, row pitch Rp): x_ext = [ s_hi(4) a_hi 1 0 0 | s_lo(4) a_lo 0 0 0 ] of row r, stored transposed so that a
@@ -1326,13 +1343,12 @@ struct Pass {
         const FoldOff o = fold_off(critic);
         const int F = critic ? d.l1 + d.la : d.l1;
         const int64_t ps = critic ? critic_off(d).total : actor_off(d).total;
-        AVD_CUDA_OK(cudaMemsetAsync(b2f, 0, (size_t)A * d.l2 * sizeof(float), st));
         pack_fold_kernel<<<dim3((unsigned)((d.l2 + 31) / 32), (unsigned)((F + 7) / 8), A), 256, 0, st>>>(params, ps, o, F, d.l2, W2b, W2T, b2f, f16() ? 1 : 0);
         AVD_LAUNCH_OK();
         return AVD_OK;
     }
 
-    // all four networks of a learn step in one launch; the b2f buffers must have been zeroed.
+    // all four networks of a learn step in one launch
     // wscale[i] (fp16 only, nullable): [A] 1 / s of job i's W2b pack.
     int pack_fold4(FoldJobs& jobs, int& Fmax, int njobs, const float* const params[], const bool critic[], bf16* const W2b[], bf16* const W2T[],
                    float* const b2f[], float* const wscale[]) const {
@@ -1714,7 +1730,7 @@ struct StageTimer {
 };
 
 // The preparation launch of the tensor-core learn step: weight half (V table, BN-folded 16-bit packs + folded biases of the four
-// networks; needs the b2f accumulators zeroed) and / or batch half (hi/lo-split [x_hi | 1 | x_lo] operand of the dgrad kernels).
+// networks) and / or batch half (hi/lo-split [x_hi | 1 | x_lo] operand of the dgrad kernels).
 static int learn_prep(const avd_learn_io* io, const Pass& p, const Workspace& w, int job_lo, int job_hi, bool vtab, bool batch, cudaStream_t st) {
     const avd_net_dims d = io->dims;
     const int A = io->A;
@@ -1791,7 +1807,7 @@ static int learn_fused3(const avd_learn_io* io, const Pass& p, const Workspace& 
     const int64_t srs = io->s_stride ? io->s_stride : d.ns;      // row pitch of the state batches
     float* const ws_c = w.wscale;
     float* const ws_a = w.wscale + A;
-    // c_b2f .. ta_b2f (folded biases, accumulated by the fold job), then dbm, ticket, U and sdq are adjacent in the workspace: one
+    // c_b2f .. ta_b2f (folded biases, written by the fold job), then dbm, ticket, U and sdq are adjacent in the workspace: one
     // memset zeroes every accumulator of the step.  (Running the weight half of the preparation on a side stream beside the
     // environment step and the replay gather was measured: -15 us per step with eager launches, nothing under CUDA-graph replay.)
     AVD_CUDA_OK(cudaMemsetAsync(w.c_b2f, 0, (size_t)((char*)(w.sdq + 2 * A) - (char*)w.c_b2f), st));

@@ -10,7 +10,10 @@ unrounded run.  Used to decide which operands need more than bf16 (DESIGN.md §4
                                                    # (the choice of three-way split bf16 operands for precision = 3)
 
 Sites (names follow csrc/avd_fused3.cu / avd_wgrad3.cu / avd_dgrad3.cu):
+    l1    state-branch layer 1 of the fused passes: "bf16x2" = the kernel's hi / lo split (s_hi W_hi + s_lo W_hi + s_hi W_lo
+          + b_hi + b_lo), "bf16" = hi parts only
     r1    relu(z1) A tile of layer 2, all passes                    W2f   folded layer-2 kernel W2' (forward B operand)
+    H     unfused forward: A operand BN(relu(z1))                   W2u   unfused forward: B operand W2 (not folded)
     dm    backward tile dq [z2 > 0] (critic / actor backward)       W2b   W2'' = W2' diag(w3') (dgrad B operand)
     dza   critic-action pass: tile dq w3' [z2 > 0]                  W2a   W2' action rows of the critic-action dgrad
     dz1   staged dz1 chunk (A operand of the layer-1 weight-gradient MMA)
@@ -40,6 +43,8 @@ def rnd(x, fmt):
         m = float(t.abs().max())
         k = 0 if m == 0 else 14 - int(np.ceil(np.log2(m)))
         return (t * 2.0 ** k).to(torch.float16).to(torch.float64).numpy() * 2.0 ** -k
+    if fmt == "fp16sat":   # no scale, round to nearest, saturating at +-65504 (the forward pass: pack_fold_kernel, cvt.rn.satfinite)
+        return t.clamp(-65504.0, 65504.0).to(torch.float16).to(torch.float64).numpy()
     if fmt == "fp32":      # operands only stored in fp32
         return t.to(torch.float64).numpy()
     if fmt == "bf16x2":    # hi + lo split
@@ -86,12 +91,29 @@ class Net:
 
     def z1(self, s, a=None):
         p = self.p
+        W, b = (p["Ws"], p["bs"]) if self.critic else (p["W1"], p["b1"])
+        l1 = self.s.get("l1")
+        if l1 is None:
+            zs = s @ W + b
+        else:                           # hi / lo split of avd_fused3.cu (write_x / W1ext); the lo . lo product is not formed
+            hi = lambda x: rnd(x, "bf16")
+            sh, Wh, bh = hi(s), hi(W), hi(b)
+            zs = sh @ Wh + bh
+            if l1 == "bf16x2":
+                zs = zs + hi(s - sh) @ Wh + sh @ hi(W - Wh) + hi(b - bh)
+            elif l1 != "bf16":
+                raise ValueError(l1)
         if self.critic:
-            return np.concatenate([s @ p["Ws"] + p["bs"], a.reshape(-1, 1) @ p["Wa"] + p["ba"]], axis=1)
-        return s @ p["W1"] + p["b1"]
+            return np.concatenate([zs, a.reshape(-1, 1) @ p["Wa"] + p["ba"]], axis=1)
+        return zs
 
     def forward(self, s, a=None):
         z1 = self.z1(s, a)
+        if "H" in self.s:               # unfused forward: BN applied before the rounding, W2 not folded
+            h1 = rnd(np.maximum(z1, 0) * self.sc1 + self.sh1, self.s["H"])
+            z2 = h1 @ rnd(self.p["W2"], self.s.get("W2u")) + self.p["b2"]
+            q = np.maximum(z2, 0) @ self.w3p + self.b3p
+            return q, dict(z1=z1, h1=h1, z2=z2)
         r1 = rnd(np.maximum(z1, 0), self.s.get("r1"))
         z2 = r1 @ rnd(self.W2p, self.s.get("W2f")) + self.b2p
         q = np.maximum(z2, 0) @ self.w3p + self.b3p
