@@ -11,7 +11,7 @@ import os
 
 AVD_MAX_FOLLOWERS = 16
 RING_RECORD_FLOATS = 10
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 RNG_RESET_VEHICLE, RNG_RESET_PLATOON, RNG_OU, RNG_LEADER_EXOG, RNG_REPLAY, RNG_INIT = range(6)
 
@@ -43,6 +43,10 @@ class Clock(C.Structure):
                 ("reserved", C.c_uint64)]
 
 
+class Runs(C.Structure):
+    _fields_ = [("seed", C.c_void_p), ("platoons_per_run", C.c_int64), ("runs", C.c_int32), ("reserved", C.c_int32)]
+
+
 class EnvIO(C.Structure):
     _fields_ = [
         ("P", C.c_int64), ("platoon_id_base", C.c_int64), ("seed", C.c_uint64),
@@ -55,7 +59,7 @@ class EnvIO(C.Structure):
         ("episode", C.c_void_p), ("step_in_episode", C.c_void_p), ("ep_reward", C.c_void_p),
         ("stats", C.c_void_p), ("clock", C.c_void_p),
         ("gen_exog", C.c_int32), ("auto_reset", C.c_int32), ("clip_actions", C.c_int32), ("ep_hist_window", C.c_int32),
-        ("last_ep_reward", C.c_void_p), ("ep_hist", C.c_void_p),
+        ("last_ep_reward", C.c_void_p), ("ep_hist", C.c_void_p), ("runs", C.c_void_p),
     ]
 
 
@@ -130,6 +134,9 @@ SIGNATURES = {
                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "avd_replay_sample_indices": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int32, C.c_int64, C.c_uint64,
                                             C.c_void_p, C.c_void_p]),
+    "avd_replay_sample_runs": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                         C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "avd_replay_sample_indices_runs": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
     "avd_replay_gather": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p,
                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "avd_replay_fill_synthetic": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_uint64, C.c_void_p]),
@@ -189,7 +196,7 @@ def load():
         fn.restype, fn.argtypes = res, args
     if lib.avd_abi_version() != ABI_VERSION:
         raise AvdError(f"ABI mismatch: library {lib.avd_abi_version()} vs binding {ABI_VERSION}")
-    for which, st in enumerate((EnvParams, EnvIO, Clock, NetDims, LearnIO, PeerComm, FedApplyIO)):
+    for which, st in enumerate((EnvParams, EnvIO, Clock, NetDims, LearnIO, PeerComm, FedApplyIO, Runs)):
         if lib.avd_sizeof(which) != C.sizeof(st):
             raise AvdError(f"struct layout mismatch for {st.__name__}: C {lib.avd_sizeof(which)} vs ctypes {C.sizeof(st)}")
     _lib = lib

@@ -29,6 +29,12 @@ int sm_count();                                  // cached multiprocessor count 
         }                                                                                   \
     } while (0)
 
+// A run table must cover the batch exactly: the kernels index runs->seed with p / platoons_per_run for every platoon p < P.
+#define AVD_REQUIRE_RUNS(r, P)                                                                                               \
+    AVD_REQUIRE((r)->seed && (r)->runs >= 1 && (r)->platoons_per_run >= 1 && (int64_t)(r)->runs * (r)->platoons_per_run == (P), \
+                "run table of %d runs x %lld platoons (seed %p) does not cover the batch of %lld platoons", (int)(r)->runs,  \
+                (long long)(r)->platoons_per_run, (const void*)(r)->seed, (long long)(P))
+
 #define AVD_LAUNCH_OK()                                                                     \
     do {                                                                                    \
         ::avd::count_launch();                                                              \

@@ -42,13 +42,16 @@ __device__ __forceinline__ void finish_episode(const avd_env_io& io, float* ep_r
 // ------------------------------------------------------------------------------------------------
 // reset of one platoon (thread-local): Platoon.reset + Vehicle.reset
 // ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void reset_one_platoon(const avd_env_params& prm, const avd_env_io& io, int64_t p,
+// `runs`: the run table (a kernel parameter), or a null constant in the instantiations that serve one run (they then compile to the
+// code without run tables).
+__device__ __forceinline__ void reset_one_platoon(const avd_env_params& prm, const avd_env_io& io, const avd_runs* runs, int64_t p,
                                                   uint32_t ep_tick, float* __restrict__ x_dst) {
     const int M = prm.M;
     const int64_t P = io.P;
-    const uint64_t gp = (uint64_t)(io.platoon_id_base + p);
+    const StreamKey key = platoon_key(runs, io.seed, (uint64_t)(io.platoon_id_base + p));
+    const uint64_t gp = key.id;
     const bool uni = prm.rand_uniform != 0;
-    const uint4 wp = rng_words(io.seed, gp, ep_tick, AVD_RNG_RESET_PLATOON);
+    const uint4 wp = rng_words(key.seed, gp, ep_tick, AVD_RNG_RESET_PLATOON);
     float fa, fu;
     if (uni) {
         fa = uniform_sym(wp.x, prm.reset_leader_a);
@@ -65,7 +68,7 @@ __device__ __forceinline__ void reset_one_platoon(const avd_env_params& prm, con
     for (int m = 0; m < M; ++m) {
         float e0, e1, a;
         if (prm.reset_mode == 0) {
-            const uint4 wv = rng_words(io.seed, gp * (uint64_t)M + (uint64_t)m, ep_tick, AVD_RNG_RESET_VEHICLE);
+            const uint4 wv = rng_words(key.seed, gp * (uint64_t)M + (uint64_t)m, ep_tick, AVD_RNG_RESET_VEHICLE);
             if (uni) {
                 e0 = uniform_sym(wv.x, prm.reset_ep);
                 e1 = uniform_sym(wv.y, prm.reset_ev);
@@ -95,14 +98,15 @@ __device__ __forceinline__ void reset_one_platoon(const avd_env_params& prm, con
     if (io.step_in_episode) io.step_in_episode[p] = 0;
 }
 
+template <bool RUNS>
 __global__ void __launch_bounds__(256) env_reset_kernel(const __grid_constant__ avd_env_params prm,
                                                         const __grid_constant__ avd_env_io io,
-                                                        const uint8_t* __restrict__ mask) {
+                                                        const uint8_t* __restrict__ mask, const __grid_constant__ avd_runs rt) {
     for (int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < io.P; p += (int64_t)gridDim.x * blockDim.x) {
         if (mask && !mask[p]) continue;
         const uint32_t ep = io.episode ? (uint32_t)io.episode[p] : 0u;
         finish_episode(io, io.ep_reward, prm.M, p, ep, io.step_in_episode ? io.step_in_episode[p] > 0 : false);
-        reset_one_platoon(prm, io, p, ep, io.x_out);
+        reset_one_platoon(prm, io, RUNS ? &rt : nullptr, p, ep, io.x_out);
         if (io.episode) io.episode[p] = (int32_t)(ep + 1u);
     }
 }
@@ -153,12 +157,12 @@ __device__ __forceinline__ FollowerIn load_follower(const StepCtx& c, int64_t v)
 // (Sharing one Philox block + Box-Muller transform between two followers -- z0 / z1 -- was measured in round 2: 5 % slower at M = 4,
 // 3 % faster at M = 8, 10 % slower plain M = 8 launches from the changed register allocation; every follower keeps its own block.)
 __device__ __forceinline__ float step_follower(const avd_env_params& prm, const avd_env_io& io, const StepCtx& c,
-                                               const FollowerIn& f, int m, int M, int64_t p, uint64_t gp, float& w, bool& term) {
+                                               const FollowerIn& f, int m, int M, int64_t p, StreamKey key, float& w, bool& term) {
     const int64_t v = (int64_t)m * c.P + p;
     float u = f.mu;
     if (c.ou_state) {  // noise.py:14-23 with explicit single roundings (bit-exact vs the host restatement)
         float z0, z1;
-        const uint4 wo = rng_words(io.seed, gp * (uint64_t)M + (uint64_t)m, c.tick, AVD_RNG_OU);
+        const uint4 wo = rng_words(key.seed, key.id * (uint64_t)M + (uint64_t)m, c.tick, AVD_RNG_OU);
         normal_pair(wo.x, wo.y, z0, z1);
         const float drift = __fmul_rn(__fmul_rn(prm.ou_theta, __fadd_rn(prm.ou_mean, -f.ou)), prm.ou_dt);
         const float n1 = __fadd_rn(__fadd_rn(f.ou, drift), __fmul_rn(c.ou_c, z0));
@@ -218,9 +222,10 @@ __device__ __forceinline__ float step_follower(const avd_env_params& prm, const 
 // follower) than the plain step, so it trades loads in flight per thread for more resident warps: 4 CTAs per SM (64 registers), and
 // for platoons longer than 4 chunks of 2 followers, which fit 64 registers without spilling.  Measured on 4 Mi platoons (launch
 // time, us; `chunk / CTAs per SM`):      M = 4:  4/3 428   4/4 370   2/4 388   2/5 388        M = 8:  4/3 881   4/4 1002   2/4 829   2/5 959
-template <int MT, bool TRAIN>
+// RUNS: the batch holds several runs (rt, a copy of *io.runs); a separate instantiation because the run-table lookup costs registers.
+template <int MT, bool TRAIN, bool RUNS>
 __global__ void __launch_bounds__(256, MT >= 1 ? (TRAIN ? 4 : 3) : 2)
-    env_step_kernel(const __grid_constant__ avd_env_params prm, const __grid_constant__ avd_env_io io) {
+    env_step_kernel(const __grid_constant__ avd_env_params prm, const __grid_constant__ avd_env_io io, const __grid_constant__ avd_runs rt) {
     const int M = MT ? MT : prm.M;
     StepCtx c;
     c.x_in = io.x_in; c.x_out = io.x_out; c.prev_a = io.prev_a; c.action_mu = io.action_mu; c.ou_state = io.ou_state;
@@ -238,6 +243,7 @@ __global__ void __launch_bounds__(256, MT >= 1 ? (TRAIN ? 4 : 3) : 2)
     c.inv_T = 1.0f / prm.T;
     c.ou_c = __fmul_rn(prm.ou_sigma, __fsqrt_rn(prm.ou_dt));
     const int64_t P = io.P;
+    const avd_runs* runs = RUNS ? &rt : nullptr;
 
     float stat_r[MT ? MT : AVD_MAX_FOLLOWERS];
 #pragma unroll
@@ -245,7 +251,7 @@ __global__ void __launch_bounds__(256, MT >= 1 ? (TRAIN ? 4 : 3) : 2)
     float stat_done = 0.0f;
 
     for (int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < P; p += (int64_t)gridDim.x * blockDim.x) {
-        const uint64_t gp = (uint64_t)(io.platoon_id_base + p);
+        const StreamKey key = platoon_key(runs, io.seed, (uint64_t)(io.platoon_id_base + p));
         constexpr int CH = MT > 4 ? (TRAIN ? 2 : 4) : (MT ? MT : 1);       // followers preloaded at a time
         FollowerIn fin[CH];
         if (MT) {
@@ -257,7 +263,7 @@ __global__ void __launch_bounds__(256, MT >= 1 ? (TRAIN ? 4 : 3) : 2)
         if (io.leader_exog) {
             w = io.leader_exog[p];
         } else if (io.gen_exog) {
-            const uint4 wx = rng_words(io.seed, gp, c.tick, AVD_RNG_LEADER_EXOG);
+            const uint4 wx = rng_words(key.seed, key.id, c.tick, AVD_RNG_LEADER_EXOG);
             w = draw_first(wx.x, wx.y, prm.reset_u, uni);
         } else {
             w = prm.model_a ? io.front_accel[p] : io.front_u[p];
@@ -276,7 +282,7 @@ __global__ void __launch_bounds__(256, MT >= 1 ? (TRAIN ? 4 : 3) : 2)
                 for (int j = 0; j < CH; ++j) {
                     if (m0 + j < MT) {
                         bool term;
-                        const float r = step_follower(prm, io, c, fin[j], m0 + j, MT, p, gp, w, term);
+                        const float r = step_follower(prm, io, c, fin[j], m0 + j, MT, p, key, w, term);
                         any_term |= term;
                         rew_sum += r;
                         stat_r[m0 + j] += r;
@@ -287,7 +293,7 @@ __global__ void __launch_bounds__(256, MT >= 1 ? (TRAIN ? 4 : 3) : 2)
             for (int m = 0; m < M; ++m) {
                 bool term;
                 const FollowerIn f = load_follower(c, (int64_t)m * P + p);
-                const float r = step_follower(prm, io, c, f, m, M, p, gp, w, term);
+                const float r = step_follower(prm, io, c, f, m, M, p, key, w, term);
                 any_term |= term;
                 rew_sum += r;
                 stat_r[m] += r;
@@ -305,7 +311,7 @@ __global__ void __launch_bounds__(256, MT >= 1 ? (TRAIN ? 4 : 3) : 2)
         if (io.auto_reset && (any_term || timeout)) {
             const uint32_t ep = io.episode ? (uint32_t)io.episode[p] : 0u;
             finish_episode(io, c.ep_reward, M, p, ep, true);
-            reset_one_platoon(prm, io, p, ep, io.x_out);
+            reset_one_platoon(prm, io, runs, p, ep, io.x_out);
             if (io.episode) io.episode[p] = (int32_t)(ep + 1u);
         }
     }
@@ -357,6 +363,10 @@ static int check_env_args(const avd_env_params* prm, const avd_env_io* io) {
     AVD_REQUIRE(prm->M >= 1 && prm->M <= AVD_MAX_FOLLOWERS, "M=%d outside 1..%d", prm->M, AVD_MAX_FOLLOWERS);
     AVD_REQUIRE(io->P >= 0, "negative platoon count");
     AVD_REQUIRE(io->P == 0 || io->prev_a, "prev_a buffer is required");
+    if (io->runs) {
+        AVD_REQUIRE(io->platoon_id_base == 0, "a run table indexes the whole batch: platoon_id_base must be 0");
+        AVD_REQUIRE_RUNS(io->runs, io->P);
+    }
     return AVD_OK;
 }
 
@@ -385,7 +395,8 @@ extern "C" int avd_env_reset(const avd_env_params* prm, const avd_env_io* io, co
     if (int rc = check_env_args(prm, io)) return rc;
     if (io->P == 0) return AVD_OK;
     AVD_REQUIRE(io->x_out, "x_out is required");
-    env_reset_kernel<<<grid_for(io->P), 256, 0, (cudaStream_t)stream>>>(*prm, *io, mask);
+    if (io->runs) env_reset_kernel<true><<<grid_for(io->P), 256, 0, (cudaStream_t)stream>>>(*prm, *io, mask, *io->runs);
+    else env_reset_kernel<false><<<grid_for(io->P), 256, 0, (cudaStream_t)stream>>>(*prm, *io, mask, avd_runs{});
     AVD_LAUNCH_OK();
     return AVD_OK;
 }
@@ -403,10 +414,16 @@ extern "C" int avd_env_step(const avd_env_params* prm, const avd_env_io* io, voi
     if (io->P == 0) return AVD_OK;
     cudaStream_t st = (cudaStream_t)stream;
     const bool train = io->ring != nullptr || io->ou_state != nullptr;
-#define AVD_LAUNCH_STEP(MT)                                                                                            \
-    do {                                                                                                               \
-        if (train) env_step_kernel<MT, true><<<resident_grid(env_step_kernel<MT, true>, io->P), 256, 0, st>>>(*prm, *io); \
-        else env_step_kernel<MT, false><<<resident_grid(env_step_kernel<MT, false>, io->P), 256, 0, st>>>(*prm, *io);   \
+    const avd_runs rt = io->runs ? *io->runs : avd_runs{};
+#define AVD_LAUNCH_STEP_R(MT, RUNS)                                                                                                    \
+    do {                                                                                                                               \
+        if (train) env_step_kernel<MT, true, RUNS><<<resident_grid(env_step_kernel<MT, true, RUNS>, io->P), 256, 0, st>>>(*prm, *io, rt); \
+        else env_step_kernel<MT, false, RUNS><<<resident_grid(env_step_kernel<MT, false, RUNS>, io->P), 256, 0, st>>>(*prm, *io, rt);   \
+    } while (0)
+#define AVD_LAUNCH_STEP(MT)                          \
+    do {                                             \
+        if (io->runs) AVD_LAUNCH_STEP_R(MT, true);   \
+        else AVD_LAUNCH_STEP_R(MT, false);           \
     } while (0)
     switch (prm->M) {
         case 1: AVD_LAUNCH_STEP(1); break;
@@ -419,6 +436,7 @@ extern "C" int avd_env_step(const avd_env_params* prm, const avd_env_io* io, voi
         default: AVD_LAUNCH_STEP(0); break;
     }
 #undef AVD_LAUNCH_STEP
+#undef AVD_LAUNCH_STEP_R
     AVD_LAUNCH_OK();
     return AVD_OK;
 }

@@ -90,6 +90,7 @@ extern "C" int64_t avd_sizeof(int which) {
         case 4: return (int64_t)sizeof(avd_learn_io);
         case 5: return (int64_t)sizeof(avd_peer_comm);
         case 6: return (int64_t)sizeof(avd_fed_apply_io);
+        case 7: return (int64_t)sizeof(avd_runs);
         default: return -1;
     }
 }

@@ -25,9 +25,11 @@ __global__ void __launch_bounds__(256) replay_add_kernel(float* __restrict__ rin
     }
 }
 
+// RUNS: every ring's stream is keyed by its run (ring_key); a separate instantiation so the one-run kernels keep their code.
+template <bool RUNS>
 __global__ void __launch_bounds__(256) replay_indices_kernel(int64_t* __restrict__ idx_out, int64_t n_rings, int64_t ring_id_base,
                                                              int32_t batch, int64_t capacity, uint64_t seed,
-                                                             const avd_clock* __restrict__ clock) {
+                                                             const avd_clock* __restrict__ clock, const __grid_constant__ avd_runs rt) {
     const uint64_t count = clock->ring_count;
     const uint64_t range = count < (uint64_t)capacity ? count : (uint64_t)capacity;   // replaybuffer.py:52
     const uint32_t tick = (uint32_t)clock->update_tick;
@@ -35,8 +37,9 @@ __global__ void __launch_bounds__(256) replay_indices_kernel(int64_t* __restrict
     const int64_t total = n_rings * blocks_per_ring;
     for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (int64_t)gridDim.x * blockDim.x) {
         const int64_t ring = t / blocks_per_ring, jb = t - ring * blocks_per_ring;
-        const uint64_t id = (uint64_t)(ring_id_base + ring) * (uint64_t)blocks_per_ring + (uint64_t)jb;
-        const uint4 w = rng_words(seed, id, tick, AVD_RNG_REPLAY);
+        const StreamKey key = ring_key(RUNS ? &rt : nullptr, seed, (uint64_t)(ring_id_base + ring));
+        const uint64_t id = key.id * (uint64_t)blocks_per_ring + (uint64_t)jb;
+        const uint4 w = rng_words(key.seed, id, tick, AVD_RNG_REPLAY);
         longlong4* dst = reinterpret_cast<longlong4*>(idx_out + ring * batch + jb * 4);
         *dst = make_longlong4(index_from_word(w.x, range), index_from_word(w.y, range), index_from_word(w.z, range),
                               index_from_word(w.w, range));
@@ -62,10 +65,11 @@ __global__ void __launch_bounds__(256) replay_gather_kernel(const float* __restr
 
 // index draw + gather fused: thread t owns Philox block jb of ring `ring` (four samples).  All four records (20 x 8 bytes) are requested
 // before the first use, so a thread overlaps four TLB / DRAM latencies instead of one; outputs are 16-byte stores.
+template <bool RUNS>
 __global__ void __launch_bounds__(256) replay_sample_kernel(const float* __restrict__ ring, int64_t n_rings, int64_t ring_id_base, int32_t batch,
                                                             int64_t capacity, uint64_t seed, const avd_clock* __restrict__ clock,
                                                             int64_t* __restrict__ idx_out, float* __restrict__ s, float* __restrict__ a,
-                                                            float* __restrict__ r, float* __restrict__ s2) {
+                                                            float* __restrict__ r, float* __restrict__ s2, const __grid_constant__ avd_runs rt) {
     const uint64_t count = clock->ring_count;
     const uint64_t range = count < (uint64_t)capacity ? count : (uint64_t)capacity;   // replaybuffer.py:52
     const uint32_t tick = (uint32_t)clock->update_tick;
@@ -73,8 +77,9 @@ __global__ void __launch_bounds__(256) replay_sample_kernel(const float* __restr
     const int64_t total = n_rings * blocks_per_ring;
     for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (int64_t)gridDim.x * blockDim.x) {
         const int64_t rg = t / blocks_per_ring, jb = t - rg * blocks_per_ring;
-        const uint64_t id = (uint64_t)(ring_id_base + rg) * (uint64_t)blocks_per_ring + (uint64_t)jb;
-        const uint4 w = rng_words(seed, id, tick, AVD_RNG_REPLAY);
+        const StreamKey key = ring_key(RUNS ? &rt : nullptr, seed, (uint64_t)(ring_id_base + rg));
+        const uint64_t id = key.id * (uint64_t)blocks_per_ring + (uint64_t)jb;
+        const uint4 w = rng_words(key.seed, id, tick, AVD_RNG_REPLAY);
         const int64_t ix[4] = {index_from_word(w.x, range), index_from_word(w.y, range), index_from_word(w.z, range), index_from_word(w.w, range)};
         const int64_t n0 = rg * batch + jb * 4;
         if (idx_out) *reinterpret_cast<longlong4*>(idx_out + n0) = make_longlong4(ix[0], ix[1], ix[2], ix[3]);
@@ -141,16 +146,35 @@ extern "C" int avd_replay_add(float* ring, int64_t capacity, int64_t M, int64_t 
     return AVD_OK;
 }
 
-extern "C" int avd_replay_sample_indices(int64_t* idx_out, int64_t n_rings, int64_t ring_id_base, int32_t batch,
-                                         int64_t capacity, uint64_t seed, const avd_clock* clock, void* stream) {
+static int replay_sample_indices(int64_t* idx_out, int64_t n_rings, int64_t ring_id_base, int32_t batch, int64_t capacity, uint64_t seed,
+                                 const avd_runs* runs, const avd_clock* clock, void* stream) {
     AVD_REQUIRE(idx_out && clock, "null buffer");
     AVD_REQUIRE(batch > 0 && batch % 4 == 0, "batch must be a positive multiple of 4 (got %d)", batch);
     AVD_REQUIRE(capacity > 0 && n_rings >= 0, "bad sizes");
     if (n_rings == 0) return AVD_OK;
-    replay_indices_kernel<<<grid_for(n_rings * (batch / 4)), 256, 0, (cudaStream_t)stream>>>(idx_out, n_rings, ring_id_base, batch,
-                                                                                             capacity, seed, clock);
+    if (runs)
+        replay_indices_kernel<true><<<grid_for(n_rings * (batch / 4)), 256, 0, (cudaStream_t)stream>>>(idx_out, n_rings, 0, batch, capacity, 0,
+                                                                                                       clock, *runs);
+    else
+        replay_indices_kernel<false><<<grid_for(n_rings * (batch / 4)), 256, 0, (cudaStream_t)stream>>>(idx_out, n_rings, ring_id_base, batch,
+                                                                                                        capacity, seed, clock, avd_runs{});
     AVD_LAUNCH_OK();
     return AVD_OK;
+}
+
+extern "C" int avd_replay_sample_indices(int64_t* idx_out, int64_t n_rings, int64_t ring_id_base, int32_t batch,
+                                         int64_t capacity, uint64_t seed, const avd_clock* clock, void* stream) {
+    return replay_sample_indices(idx_out, n_rings, ring_id_base, batch, capacity, seed, nullptr, clock, stream);
+}
+
+extern "C" int avd_replay_sample_indices_runs(int64_t* idx_out, int64_t n_rings, int32_t batch, int64_t capacity, const avd_runs* runs,
+                                              const avd_clock* clock, void* stream) {
+    AVD_REQUIRE(runs, "null run table");
+    AVD_REQUIRE(runs->seed && runs->runs >= 1 && runs->platoons_per_run >= 1 &&
+                    n_rings % ((int64_t)runs->runs * runs->platoons_per_run) == 0,
+                "%lld rings are not M x (%d runs x %lld platoons), or the table has no seeds", (long long)n_rings, (int)runs->runs,
+                (long long)runs->platoons_per_run);
+    return replay_sample_indices(idx_out, n_rings, 0, batch, capacity, 0, runs, clock, stream);
 }
 
 extern "C" int avd_replay_gather(const float* ring, int64_t capacity, int64_t M, int64_t P, const int64_t* idx, int32_t batch,
@@ -163,18 +187,34 @@ extern "C" int avd_replay_gather(const float* ring, int64_t capacity, int64_t M,
     return AVD_OK;
 }
 
-extern "C" int avd_replay_sample(const float* ring, int64_t capacity, int64_t M, int64_t P, int64_t ring_id_base, int32_t batch, uint64_t seed,
-                                 const avd_clock* clock, int64_t* idx_out, float* s, float* a, float* r, float* s2, void* stream) {
+static int replay_sample(const float* ring, int64_t capacity, int64_t M, int64_t P, int64_t ring_id_base, int32_t batch, uint64_t seed,
+                         const avd_runs* runs, const avd_clock* clock, int64_t* idx_out, float* s, float* a, float* r, float* s2, void* stream) {
     AVD_REQUIRE(ring && clock && s && a && r && s2, "null buffer");
     AVD_REQUIRE(batch > 0 && batch % 4 == 0, "batch must be a positive multiple of 4 (got %d)", batch);
     AVD_REQUIRE(capacity > 0 && M > 0 && P >= 0, "bad sizes");
     AVD_REQUIRE(((uintptr_t)a & 15) == 0 && ((uintptr_t)r & 15) == 0 && ((uintptr_t)s & 15) == 0 && ((uintptr_t)s2 & 15) == 0 &&
                 (!idx_out || ((uintptr_t)idx_out & 31) == 0), "sample outputs must be 16-byte (indices: 32-byte) aligned");
     if (P == 0) return AVD_OK;
-    replay_sample_kernel<<<grid_for(M * P * (batch / 4)), 256, 0, (cudaStream_t)stream>>>(ring, M * P, ring_id_base, batch, capacity, seed, clock, idx_out, s, a,
-                                                                                        r, s2);
+    if (runs)
+        replay_sample_kernel<true><<<grid_for(M * P * (batch / 4)), 256, 0, (cudaStream_t)stream>>>(ring, M * P, 0, batch, capacity, 0, clock, idx_out, s,
+                                                                                                    a, r, s2, *runs);
+    else
+        replay_sample_kernel<false><<<grid_for(M * P * (batch / 4)), 256, 0, (cudaStream_t)stream>>>(ring, M * P, ring_id_base, batch, capacity, seed, clock,
+                                                                                                     idx_out, s, a, r, s2, avd_runs{});
     AVD_LAUNCH_OK();
     return AVD_OK;
+}
+
+extern "C" int avd_replay_sample(const float* ring, int64_t capacity, int64_t M, int64_t P, int64_t ring_id_base, int32_t batch, uint64_t seed,
+                                 const avd_clock* clock, int64_t* idx_out, float* s, float* a, float* r, float* s2, void* stream) {
+    return replay_sample(ring, capacity, M, P, ring_id_base, batch, seed, nullptr, clock, idx_out, s, a, r, s2, stream);
+}
+
+extern "C" int avd_replay_sample_runs(const float* ring, int64_t capacity, int64_t M, int64_t P, int32_t batch, const avd_runs* runs,
+                                      const avd_clock* clock, int64_t* idx_out, float* s, float* a, float* r, float* s2, void* stream) {
+    AVD_REQUIRE(runs, "null run table");
+    AVD_REQUIRE_RUNS(runs, P);
+    return replay_sample(ring, capacity, M, P, 0, batch, 0, runs, clock, idx_out, s, a, r, s2, stream);
 }
 
 extern "C" int avd_replay_fill_synthetic(float* ring, int64_t capacity, int64_t M, int64_t P, uint64_t seed, void* stream) {

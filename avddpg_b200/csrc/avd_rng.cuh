@@ -9,6 +9,8 @@
 #pragma once
 #include <stdint.h>
 
+#include "../../include/avddpg_b200.h"
+
 namespace avd {
 
 constexpr uint32_t kPhiloxM0 = 0xD2511F53u;
@@ -31,6 +33,28 @@ __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
 __device__ __forceinline__ uint4 rng_words(uint64_t seed, uint64_t id, uint32_t tick, uint32_t purpose) {
     return philox4x32_10(make_uint4((uint32_t)id, (uint32_t)(id >> 32), tick, purpose),
                          make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
+}
+
+// Stream key of platoon `p` (with runs: a platoon index of the whole batch) and of replay ring `ring` = m*P + p.
+// Without a run table that is (seed, p) and ring id m*P + p; with one, platoon p belongs to run s = p / Pr and the key is
+// (runs->seed[s], p mod Pr), ring id m*Pr + p mod Pr: the keys of the stand-alone run with random_seed = seed[s].  `runs` points
+// at a kernel parameter the host entry has checked (AVD_REQUIRE_RUNS: P = runs * Pr), so s < runs.  The env kernels evaluate
+// it once per platoon, the replay kernels once per Philox block (four samples of a ring).
+struct StreamKey {
+    uint64_t seed, id;
+};
+
+__device__ __forceinline__ StreamKey platoon_key(const avd_runs* runs, uint64_t seed, uint64_t p) {
+    if (!runs) return {seed, p};
+    const uint64_t pr = (uint64_t)runs->platoons_per_run, s = p / pr;
+    return {runs->seed[s], p - s * pr};
+}
+
+__device__ __forceinline__ StreamKey ring_key(const avd_runs* runs, uint64_t seed, uint64_t ring) {
+    if (!runs) return {seed, ring};
+    const uint64_t m = ring / ((uint64_t)runs->runs * (uint64_t)runs->platoons_per_run);
+    const StreamKey k = platoon_key(runs, seed, ring - m * ((uint64_t)runs->runs * (uint64_t)runs->platoons_per_run));
+    return {k.seed, m * (uint64_t)runs->platoons_per_run + k.id};
 }
 
 // uint32 -> (0,1): ((x >> 9) + 0.5) * 2^-23, exact in binary32.

@@ -46,6 +46,36 @@ class DeviceClock:
         return {"step_tick": s, "ring_count": r, "update_tick": u}
 
 
+class RunTable:
+    """S independent training runs that share one batch of P = S * platoons_per_run platoons (avd_runs: a host struct the library
+    checks and hands to its kernels by value, over a device array of the seeds, so a captured CUDA graph replays it).  Run s owns
+    platoons [s * Pr, (s + 1) * Pr) and draws every random stream of the stand-alone run with random_seed = seeds[s]: its platoon
+    p' is keyed (seeds[s], p') and its ring m * Pr + p' likewise."""
+
+    def __init__(self, seeds, platoons_per_run: int, device):
+        seeds = [int(k) for k in seeds]
+        if not seeds:
+            raise ValueError("a run table needs at least one seed")
+        bad = [k for k in seeds if not 0 <= k < 1 << 64]
+        if bad:
+            raise ValueError(f"seeds must be unsigned 64-bit integers, got {bad}")
+        if int(platoons_per_run) < 1:
+            raise ValueError("platoons_per_run must be positive")
+        self.seeds, self.S, self.Pr = seeds, len(seeds), int(platoons_per_run)
+        # uint64 bit patterns in an int64 tensor (the kernels read them as uint64_t)
+        self.seed_t = torch.tensor([k - (1 << 64) if k >= 1 << 63 else k for k in seeds], dtype=torch.int64, device=device)
+        self.table = _lib.Runs()
+        self.table.seed, self.table.platoons_per_run, self.table.runs = self.seed_t.data_ptr(), self.Pr, self.S
+
+    @property
+    def ptr(self):
+        return C.c_void_p(C.addressof(self.table))
+
+    @property
+    def P(self) -> int:
+        return self.S * self.Pr
+
+
 class BatchedPlatoons:
     """P platoons x M followers on one GPU.
 
@@ -60,7 +90,10 @@ class BatchedPlatoons:
                  seed: Optional[int] = None, rand_states: bool = True, evaluator_states_enabled: bool = False,
                  track_kinematics: bool = True, ring=None, clock: Optional[DeviceClock] = None,
                  steps_per_episode: Optional[int] = None, auto_reset: bool = False, collect_stats: bool = False,
-                 track_episodes: bool = True, store_actions: bool = True, reward_history: int = 0):
+                 track_episodes: bool = True, store_actions: bool = True, reward_history: int = 0,
+                 runs: Optional[RunTable] = None):
+        """runs: the platoons are runs.S independent runs of runs.Pr platoons each (see RunTable); seed and platoon_id_base are
+        then unused."""
         self.lib = _lib.load()
         _lib.require_device()
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
@@ -71,6 +104,9 @@ class BatchedPlatoons:
         self.num_states = int(self.prm.num_states)
         self.centralized = bool(self.prm.centralized)
         self.seed = int(getattr(config, "random_seed", 1) if seed is None else seed)
+        if runs is not None and (runs.P != self.P or platoon_id_base != 0):
+            raise ValueError(f"a run table of {runs.S} x {runs.Pr} platoons needs P = {runs.P} and platoon_id_base = 0")
+        self.runs = runs
         P, M, dev = self.P, self.M, self.device
         f32 = dict(dtype=torch.float32, device=dev)
         self._x = torch.zeros(2, 4, M, P, **f32)
@@ -111,6 +147,7 @@ class BatchedPlatoons:
             setattr(io, name, None if t is None else t.data_ptr())
         io.reward, io.done = self._reward.data_ptr(), self._done.data_ptr()
         io.clock = self.clock.t.data_ptr()
+        io.runs = None if runs is None else C.addressof(runs.table)
         if ring is not None:
             if ring.M != M or ring.P != P:
                 raise ValueError("replay ring shape does not match the platoon batch")

@@ -110,9 +110,9 @@ class NetBank:
         """Gradients in ``trainable_variables`` order (views into the flat gradient vector)."""
         return [self.view(n, agent, self.grad) for n in self.trainable_names]
 
-    def init_reference(self, generator: torch.Generator):
+    def init_reference(self, generator: torch.Generator, agents: Optional[torch.Tensor] = None):
         """Initialisers of agent/model.py:19-25 / 53-60; every agent starts from agent 0's weights
-        (workers/trainer.py:121-131)."""
+        (workers/trainer.py:121-131).  agents: index tensor of the agents to initialise (default: all)."""
         d = self.dims
 
         def uni(shape, bound):
@@ -130,11 +130,21 @@ class NetBank:
             vals["W2"] = uni((d.l1 + d.la, d.l2), 1 / math.sqrt(d.l2))
             vals["W3"] = uni((d.l2, 1), 3e-4)
             ones = ["gs", "vars", "ga", "vara", "g2", "var2"]
-        self.flat.zero_()
+        if agents is None:
+            self.flat.zero_()
+            for name, v in vals.items():
+                self.view(name).copy_(v.to(self.flat.device).unsqueeze(0).expand(self.A, *v.shape))
+            for name in ones:
+                self.view(name).fill_(1.0)
+            return
+        row = torch.zeros(self.total, dtype=torch.float32)
         for name, v in vals.items():
-            self.view(name).copy_(v.to(self.flat.device).unsqueeze(0).expand(self.A, *v.shape))
+            off, shape = self.offsets[name]
+            row[off: off + v.numel()] = v.reshape(-1)
         for name in ones:
-            self.view(name).fill_(1.0)
+            off, shape = self.offsets[name]
+            row[off: off + int(np.prod(shape))] = 1.0
+        self.flat[agents.to(self.flat.device)] = row.to(self.flat.device)
 
     def set_weights(self, agent: Optional[int], arrays):
         """Keras ``set_weights`` (list in `.weights` order); agent=None sets every agent."""

@@ -21,7 +21,9 @@ from .environment import DeviceClock
 
 class ReplayRings:
     def __init__(self, capacity: int, M: int, P: int, batch_size: int = 64, *, seed: int = 1, ring_id_base: int = 0,
-                 clock: Optional[DeviceClock] = None, device=None):
+                 clock: Optional[DeviceClock] = None, device=None, runs=None):
+        """runs: an environment.RunTable; ring m*P + p is then keyed like ring m*Pr + p mod Pr of run p // Pr (seed and
+        ring_id_base are unused)."""
         if capacity <= 0 or batch_size <= 0 or batch_size % 4:
             raise ValueError("capacity must be > 0 and batch_size a positive multiple of 4")
         self.lib = _lib.load()
@@ -30,6 +32,9 @@ class ReplayRings:
         self.capacity, self.M, self.P, self.batch_size = int(capacity), int(M), int(P), int(batch_size)
         self.n_rings = self.M * self.P
         self.seed, self.ring_id_base = int(seed), int(ring_id_base)
+        if runs is not None and (runs.P != self.P or self.ring_id_base != 0):
+            raise ValueError(f"a run table of {runs.S} x {runs.Pr} platoons needs P = {runs.P} and ring_id_base = 0")
+        self.runs = runs
         self.data = torch.empty(self.capacity, self.M, self.P, _lib.RING_RECORD_FLOATS, dtype=torch.float32, device=self.device)
         self.clock = clock if clock is not None else DeviceClock(self.device)
         self.idx = self.s = self.a = self.r = self.s2 = None      # sample buffers: allocated on first use
@@ -57,6 +62,10 @@ class ReplayRings:
 
     def sample_indices(self):
         self._alloc_sample_buffers()
+        if self.runs is not None:
+            _lib.check(self.lib.avd_replay_sample_indices_runs(_lib.ptr(self.idx), self.n_rings, self.batch_size, self.capacity, self.runs.ptr,
+                                                               self.clock.ptr, _lib.current_stream()))
+            return self.idx
         _lib.check(self.lib.avd_replay_sample_indices(_lib.ptr(self.idx), self.n_rings, self.ring_id_base, self.batch_size,
                                                       self.capacity, self.seed, self.clock.ptr, _lib.current_stream()))
         return self.idx
@@ -73,9 +82,15 @@ class ReplayRings:
         """ReplayBuffer.sample for every ring in one launch (avd_replay_sample: index draw + gathers fused, identical to
         sample_indices() + gather()); keep_indices also writes the draws to self.idx."""
         self._alloc_sample_buffers()
-        _lib.check(self.lib.avd_replay_sample(_lib.ptr(self.data), self.capacity, self.M, self.P, self.ring_id_base, self.batch_size, self.seed,
-                                              self.clock.ptr, _lib.ptr(self.idx) if keep_indices else None, _lib.ptr(self.s), _lib.ptr(self.a),
-                                              _lib.ptr(self.r), _lib.ptr(self.s2), _lib.current_stream()))
+        idx = _lib.ptr(self.idx) if keep_indices else None
+        if self.runs is not None:
+            _lib.check(self.lib.avd_replay_sample_runs(_lib.ptr(self.data), self.capacity, self.M, self.P, self.batch_size, self.runs.ptr,
+                                                       self.clock.ptr, idx, _lib.ptr(self.s), _lib.ptr(self.a), _lib.ptr(self.r),
+                                                       _lib.ptr(self.s2), _lib.current_stream()))
+        else:
+            _lib.check(self.lib.avd_replay_sample(_lib.ptr(self.data), self.capacity, self.M, self.P, self.ring_id_base, self.batch_size,
+                                                  self.seed, self.clock.ptr, idx, _lib.ptr(self.s), _lib.ptr(self.a), _lib.ptr(self.r),
+                                                  _lib.ptr(self.s2), _lib.current_stream()))
         if advance_clock:
             self.clock.advance(update=1)
         return self.s, self.a, self.r, self.s2

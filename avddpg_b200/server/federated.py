@@ -149,13 +149,15 @@ def shard_platoons(num_platoons: int, rank: int, world: int):
 
 class FederatedAggregator:
     def __init__(self, population, conf, process_group=None, world_size: Optional[int] = None,
-                 reference_weights_quirk: bool = True, transport: str = "auto"):
+                 reference_weights_quirk: bool = True, transport: str = "auto", runs: int = 1):
         """population: DDPGPopulation (A = G*M agents of THIS rank).  process_group: a torch.distributed group
         (NCCL on GPUs) or None for single-process.  reference_weights_quirk: weights mode applies system 0's
         average to every agent, as workers/trainer.py:442-456 does (`[...][0]`).  transport: "peer" = the NVLink-native
         one-kernel exchange over symmetric memory (NVLS in-switch reduction when available; "p2p" forces plain peer loads),
         "nccl" = all_reduce + finalize,
-        "auto" = peer when the group spans several CUDA ranks and symmetric memory can be set up ON EVERY RANK, else nccl."""
+        "auto" = peer when the group spans several CUDA ranks and symmetric memory can be set up ON EVERY RANK, else nccl.
+        runs: the population's groups are `runs` independent runs of G / runs groups (DDPGPopulation seeds); interfrl then averages
+        each follower over the groups of its own run."""
         self.pop, self.conf, self.pg = population, conf, process_group
         self.lib = _lib.load()
         if conf.fed_method not in ("interfrl", "intrafrl"):
@@ -167,9 +169,15 @@ class FederatedAggregator:
             import torch.distributed as dist
             self.world = dist.get_world_size(process_group)
         G, M = population.G, population.M
-        # member row of (system s, member x) = s*stride_s + x*stride_x in the [A, n] banks (a = m*G + g)
+        self.runs = int(runs)
+        if self.runs > 1 and conf.aggregation_method == conf.weights:
+            raise NotImplementedError("weights-mode FRL over several runs: its reference quirk broadcasts system 0 to every agent, "
+                                      "which would have to be per run")
+        # member row of (system s, member x) = s*stride_s + x*stride_x in the [A, n] banks (a = m*G + g).  interfrl over runs: system
+        # (m, run) = m*runs + run has the run's Gr groups as members, row (m*runs + run)*Gr + g' = m*G + run*Gr + g'.
         if self.inter:
-            self.n_systems, self.n_members, self.stride_s, self.stride_x = M, G, G, 1
+            Gr = G // self.runs
+            self.n_systems, self.n_members, self.stride_s, self.stride_x = M * self.runs, Gr, Gr, 1
         else:
             self.n_systems, self.n_members, self.stride_s, self.stride_x = G, M, 1, G
         dev = population.device
@@ -261,30 +269,32 @@ class FederatedAggregator:
         self.rounds += 1
         return buf
 
-    def aggregate_gradients(self, weights=None, apply: bool = True, write_back: bool = True):
+    def aggregate_gradients(self, weights=None, apply: bool = True, write_back: bool = True, apply_mask=None):
         """train_all_models_federated_gradients (trainer.py:400-431): average actor/critic gradients per system, then every member
         applies them with its own Adam and soft-updates its targets.  On CUDA with `apply` this is TWO launches: avd_fed_reduce2 and
         the fused consumer avd_fed_apply_gradients (barrier -> in-switch reduction -> division -> Adam -> Polyak -> step counters);
         `write_back` also stores the averaged gradients into every member's .grad row (what the unfused path leaves there).
-        The NCCL transport, `apply=False` and host tensors take reduce -> all_reduce -> finalize -> broadcast (-> Adam / Polyak)."""
+        The NCCL transport, `apply=False` and host tensors take reduce -> all_reduce -> finalize -> broadcast (-> Adam / Polyak).
+        apply_mask: [A] uint8, the agents that take this round (default: self.apply_mask); the others keep weights and gradients."""
         pop = self.pop
+        mask = self.apply_mask if apply_mask is None else apply_mask
         na, nc = pop.actor.n_train, pop.critic.n_train
         fused = apply and self.device.type == "cuda" and (self._use_peer() or not (self.inter and self.world > 1))
         if fused:
             part, pitch = self._reduce(pop.actor.grad, na, pop.critic.grad, nc, na, nc, weights)
-            self._apply_fused(part, pitch, write_back)
+            self._apply_fused(part, pitch, write_back, mask)
             self.last_weight_sums = self.wsum
             self.rounds += 1
             return None
         buf = self._reduce_exchange(pop.actor.grad, na, pop.critic.grad, nc, na, nc, weights)
         _lib.check(self.lib.avd_fed_broadcast2(_lib.ptr(pop.actor.grad), na, na, _lib.ptr(pop.critic.grad), nc, nc, _lib.ptr(buf), buf.shape[1],
-                                               self.n_systems, self.n_members, self.stride_s, self.stride_x, _lib.ptr(self.apply_mask),
+                                               self.n_systems, self.n_members, self.stride_s, self.stride_x, _lib.ptr(mask),
                                                _lib.current_stream()))
         if apply:
-            pop.apply_gradients_and_soft_update(self.apply_mask)
+            pop.apply_gradients_and_soft_update(mask)
         return buf
 
-    def _apply_fused(self, part, pitch, write_back):
+    def _apply_fused(self, part, pitch, write_back, mask):
         pop, conf = self.pop, self.conf
         if self._apply_io is None:
             io = _lib.FedApplyIO()
@@ -293,12 +303,12 @@ class FederatedAggregator:
             io.actor, io.t_actor, io.actor_m, io.actor_v, io.actor_step = a.flat.data_ptr(), pop.t_actor.flat.data_ptr(), a.m.data_ptr(), a.v.data_ptr(), a.step.data_ptr()
             io.critic, io.t_critic, io.critic_m, io.critic_v, io.critic_step = c.flat.data_ptr(), pop.t_critic.flat.data_ptr(), c.m.data_ptr(), c.v.data_ptr(), c.step.data_ptr()
             io.actor_total, io.actor_train, io.critic_total, io.critic_train = a.total, a.n_train, c.total, c.n_train
-            io.apply_mask = None if self.apply_mask is None else self.apply_mask.data_ptr()
             io.wsum_out = self.wsum.data_ptr()
             io.actor_lr, io.critic_lr, io.beta1, io.beta2, io.eps, io.tau = float(conf.actor_lr), float(conf.critic_lr), 0.9, 0.999, 1e-7, float(conf.tau)
             self._apply_io = io
         io = self._apply_io
         io.pitch = pitch
+        io.apply_mask = None if mask is None else mask.data_ptr()
         io.actor_grad_out = pop.actor.grad.data_ptr() if write_back else None
         io.critic_grad_out = pop.critic.grad.data_ptr() if write_back else None
         if self._use_peer():

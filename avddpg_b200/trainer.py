@@ -16,7 +16,7 @@ single-agent model objects from avddpg_b200.model.
 from __future__ import annotations
 
 import ctypes as C
-from typing import Optional
+from typing import Optional, Sequence
 
 import numpy as np
 import torch
@@ -27,7 +27,9 @@ from .model import NetBank, dims_from_config
 
 class DDPGPopulation:
     def __init__(self, num_groups: int, num_followers: int, config, *, num_states: int = 4, rows_per_agent: int = 64,
-                 device=None, seed: Optional[int] = None, precision: int = 0):
+                 device=None, seed: Optional[int] = None, precision: int = 0, seeds: Optional[Sequence[int]] = None):
+        """seeds: the G groups are len(seeds) independent runs of G / len(seeds) groups each; run s starts from the weights the
+        stand-alone population with seed seeds[s] draws (its agents m*G + s*Gr + g', see run_agents)."""
         self.lib = _lib.load()
         _lib.require_device()
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
@@ -39,14 +41,30 @@ class DDPGPopulation:
         self.critic = NetBank("critic", self.dims, self.A, dev, with_optimizer=True)
         self.t_actor = NetBank("actor", self.dims, self.A, dev)
         self.t_critic = NetBank("critic", self.dims, self.A, dev)
-        gen = torch.Generator().manual_seed(int(getattr(config, "random_seed", 1) if seed is None else seed))
-        self.actor.init_reference(gen)
-        self.critic.init_reference(gen)
+        if seeds is None:
+            self.S = 1
+            gen = torch.Generator().manual_seed(int(getattr(config, "random_seed", 1) if seed is None else seed))
+            self.actor.init_reference(gen)
+            self.critic.init_reference(gen)
+        else:
+            self.S = len(seeds)
+            if self.S < 1 or self.G % self.S:
+                raise ValueError(f"{self.G} groups cannot be split into {self.S} runs")
+            for s, k in enumerate(seeds):
+                gen = torch.Generator().manual_seed(int(k))      # the actor, then the critic: the stand-alone draw order
+                agents = self.run_agents(s)
+                self.actor.init_reference(gen, agents)
+                self.critic.init_reference(gen, agents)
         self.sync_targets()
         self.loss = torch.zeros(self.A, 2, dtype=torch.float32, device=dev)
         self._ws = None
         self._act_ws = None
         self.io = _lib.LearnIO()
+
+    def run_agents(self, s: int) -> torch.Tensor:
+        """Agent indices of run s, in the stand-alone run's agent order m*Gr + g' (agent m*G + s*Gr + g' here)."""
+        Gr = self.G // self.S
+        return (torch.arange(self.M).unsqueeze(1) * self.G + s * Gr + torch.arange(Gr).unsqueeze(0)).reshape(-1)
 
     def sync_targets(self):
         """target.set_weights(online.get_weights())  (trainer.py:130-131)."""
@@ -143,27 +161,44 @@ class BatchedTrainer:
     on the device; the host only launches kernels (optionally a captured CUDA graph of the whole step).
     Per-platoon episode handling replaces the reference's "any platoon terminal ends the episode for all"
     (trainer.py:268-269): a platoon that terminates or reaches steps_per_episode is reset inside the env kernel.
+
+    seeds=[k_0, ..., k_{S-1}] hosts S independent runs of num_groups x envs_per_group platoons each: run s behaves like the
+    stand-alone trainer with random_seed = k_s (its draws, initial weights, FRL systems, episodes and reward log) and owns groups
+    [s*Gr, (s+1)*Gr) of the G = S*Gr here (Gr = num_groups), so its platoons and rings are contiguous.  Single GPU only.
     """
 
     def __init__(self, conf, num_groups: int, envs_per_group: int = 1, *, ring_capacity=None, rank: int = 0, world: int = 1,
-                 process_group=None, precision: int = 0, seed=None, track_kinematics: bool = False, fed_transport: str = "auto"):
-        from .environment import BatchedPlatoons
+                 process_group=None, precision: int = 0, seed=None, track_kinematics: bool = False, fed_transport: str = "auto",
+                 seeds=None):
+        from .environment import BatchedPlatoons, RunTable
         from .replaybuffer import ReplayRings
-        self.conf, self.G, self.E, self.M = conf, int(num_groups), int(envs_per_group), int(conf.pl_size)
+        self.S = 1 if seeds is None else len(seeds)
+        self.conf, self.Gr, self.E, self.M = conf, int(num_groups), int(envs_per_group), int(conf.pl_size)
+        self.G = self.Gr * self.S
         self.P = self.G * self.E
         self.rank, self.world = rank, world
+        self.seeds, self.runs = None, None
+        if seeds is not None:
+            if world > 1 or process_group is not None:
+                raise ValueError("seeds: the runs of a batch live on one GPU (world must be 1)")
+            if is_fed_enabled(conf) and is_model_weight_updates_enabled(conf):
+                # run()'s per-run loop has gradient rounds only, so even one seed would silently train unlike its stand-alone run
+                raise NotImplementedError("weights-mode FRL is not available for trainers built with seeds")
+            self.runs = RunTable(seeds, self.Gr * self.E, torch.device("cuda", torch.cuda.current_device()))
+            self.seeds = self.runs.seeds
         seed = int(getattr(conf, "random_seed", 1) if seed is None else seed)
         cap = int(conf.buffer_size if ring_capacity is None else ring_capacity)
-        self.rings = ReplayRings(cap, self.M, self.P, int(conf.batch_size), seed=seed, ring_id_base=rank * self.M * self.P)
+        self.rings = ReplayRings(cap, self.M, self.P, int(conf.batch_size), seed=seed, ring_id_base=rank * self.M * self.P, runs=self.runs)
         self.env = BatchedPlatoons(self.P, self.M, conf, platoon_id_base=rank * self.P, seed=seed, ring=self.rings,
                                    clock=self.rings.clock, auto_reset=True, collect_stats=True, track_kinematics=track_kinematics,
-                                   reward_history=int(conf.weighted_window) if is_fed_enabled(conf) and conf.weighted_average_enabled else 0)
+                                   reward_history=int(conf.weighted_window) if is_fed_enabled(conf) and conf.weighted_average_enabled else 0,
+                                   runs=self.runs)
         self.pop = DDPGPopulation(self.G, self.M, conf, num_states=self.env.num_states, rows_per_agent=self.E * int(conf.batch_size),
-                                  seed=seed, precision=precision)
+                                  seed=seed, precision=precision, seeds=self.seeds)
         self.fed = None
         if is_fed_enabled(conf):
             from .server.federated import FederatedAggregator
-            self.fed = FederatedAggregator(self.pop, conf, process_group=process_group, transport=fed_transport)
+            self.fed = FederatedAggregator(self.pop, conf, process_group=process_group, transport=fed_transport, runs=self.S)
         self.buffer_counter = 0          # == ReplayBuffer.buffer_counter of every ring
         self.step_in_run = 0             # bookkeeping only
         # What the FRL scheduling predicates see (workers/trainer.py:232, 251: `ep`, `i`).  run() counts real episodes and zeroes
@@ -229,33 +264,67 @@ class BatchedTrainer:
         self.fed_weights = self._fed_w
         return self._fed_w
 
-    def frl_weight_lists(self):
+    def frl_weight_lists(self, run: Optional[int] = None):
         """(fed_weights[g][m], fed_weight_sums[g][m]) of the last federated round as nested lists of np.float32, the layout
         update_reward_list records (trainer.py:521-528), or (None, None) when the round was unweighted.  fed_weight_sums is the sum
-        over ALL members of the system -- over every rank's platoons for interfrl (it travels through the exchange)."""
+        over ALL members of the system -- over every rank's platoons for interfrl (it travels through the exchange).
+        run: only the groups of that run (trainers built with seeds)."""
         if self.fed is None or self.fed_weights is None or self.fed.last_weight_sums is None:
             return None, None
-        w = self.fed_weights.cpu().numpy().astype(np.float32)            # [S][X]
-        sums = self.fed.last_weight_sums.cpu().numpy().astype(np.float32)  # [S]
-        if self.fed.inter:      # systems = followers m, members = groups g
-            return ([[w[m, g] for m in range(self.M)] for g in range(self.G)], [[sums[m] for m in range(self.M)] for g in range(self.G)])
-        return ([[w[g, m] for m in range(self.M)] for g in range(self.G)], [[sums[g] for m in range(self.M)] for g in range(self.G)])
+        w = self.fed_weights.cpu().numpy().astype(np.float32)            # [systems][members]
+        sums = self.fed.last_weight_sums.cpu().numpy().astype(np.float32)  # [systems]
+        groups = range(self.G) if run is None else range(run * self.Gr, (run + 1) * self.Gr)
+        if self.fed.inter:      # systems = (follower m, run k) = m*S + k, members = the run's groups g'
+            Gr, S = self.Gr, self.S
+            return ([[w[m * S + g // Gr, g % Gr] for m in range(self.M)] for g in groups],
+                    [[sums[m * S + g // Gr] for m in range(self.M)] for g in groups])
+        return ([[w[g, m] for m in range(self.M)] for g in groups], [[sums[g] for m in range(self.M)] for g in groups])
 
-    def episodic_rewards(self):
+    def episodic_rewards(self, run: Optional[int] = None):
         """Cumulative reward of the current episode per agent, [G][M] nested lists of np.float32 (the reference's
-        all_episodic_reward_counters, trainer.py:249, 321); with E environments per group: the mean over the group's platoons."""
+        all_episodic_reward_counters, trainer.py:249, 321); with E environments per group: the mean over the group's platoons.
+        run: only the groups of that run, [Gr][M] (trainers built with seeds)."""
         r = self.env.ep_reward.reshape(self.M, self.G, self.E).mean(dim=2).t().contiguous().cpu().numpy().astype(np.float32)
-        return [[r[g, m] for m in range(self.M)] for g in range(self.G)]
+        groups = range(self.G) if run is None else range(run * self.Gr, (run + 1) * self.Gr)
+        return [[r[g, m] for m in range(self.M)] for g in groups]
 
-    def run(self, episodes: int, reward_log=None, *, global_break: bool = True, learn: bool = True, any_terminal_group=None):
+    def reward_logs(self):
+        """One results.RewardLog per run, each on a copy of the configuration that carries the run's seed, so that generate_csvs
+        writes its files as ..._seed{k_s}.csv (the files the reference's accumr aggregates)."""
+        import copy
+        from .results import RewardLog
+        logs = []
+        for k in (self.seeds if self.seeds is not None else [int(getattr(self.conf, "random_seed", 1))]):
+            conf = copy.copy(self.conf)
+            conf.random_seed = k
+            logs.append(RewardLog(conf, num_platoons=self.Gr, num_models=self.M))
+        return logs
+
+    def run_weights(self, s: int, group: int = 0):
+        """Run s's weights: (actors, critics) with actors[m] / critics[m] the Keras `.weights` arrays of follower m of the run's group
+        `group` -- what results.save_weights writes, or what a G = 1 DDPGPopulation takes (set_weights) for evaluator.run."""
+        if not 0 <= s < self.S or not 0 <= group < self.Gr:
+            raise IndexError(f"run {s} / group {group} outside {self.S} runs of {self.Gr} groups")
+        agents = [m * self.G + s * self.Gr + group for m in range(self.M)]
+        return [self.pop.actor.get_weights(a) for a in agents], [self.pop.critic.get_weights(a) for a in agents]
+
+    def run(self, episodes: int, reward_log=None, *, global_break: bool = True, learn: bool = True, any_terminal_group=None,
+            reward_logs=None):
         """The episode loop of Trainer.run (workers/trainer.py:232-273) for the whole population: every episode resets ALL
         platoons (246-249), runs up to conf.steps_per_episode steps (251), ends early for everybody when ANY platoon reports a
         terminal state (268-269; `global_break=False` lets the other platoons finish) and appends the episodic rewards to
-        `reward_log` (an avddpg_b200.results.RewardLog; trainer.py:273, 510-517).  In-kernel auto-reset is switched off for the
+        `reward_log` (an avddpg_b200.results.RewardLog; trainer.py:273, 510-517).  A trainer built with seeds runs this loop per run
+        (see _run_runs) and takes `reward_logs`, one RewardLog per run (reward_logs()).  In-kernel auto-reset is switched off for the
         duration, so episodes line up across platoons exactly like the reference's; one D2H read of the done flags per step is
         the price (the free-running `step()` loop used by the benchmark never synchronises).  `any_terminal_group`: a
         torch.distributed group over which "any platoon terminal" is agreed (one 1-word all_reduce(MAX) per step) so that platoons
         sharded over several GPUs still end their episodes together (SURVEY.md section 8e: opt-in).  Returns the number of env steps."""
+        if self.runs is not None:
+            if reward_log is not None or any_terminal_group is not None:
+                raise ValueError("a trainer with runs takes reward_logs (one per run) and no any_terminal_group")
+            return self._run_runs(episodes, reward_logs, global_break, learn)
+        if reward_logs is not None:
+            raise ValueError("reward_logs is for trainers built with seeds; pass reward_log")
         env, conf = self.env, self.conf
         saved = env.auto_reset
         env.auto_reset = False
@@ -286,6 +355,101 @@ class BatchedTrainer:
             env.auto_reset = saved
             self._in_run = False
         return steps
+
+    def _run_runs(self, episodes: int, reward_logs, global_break: bool, learn: bool):
+        """run() for S runs: each run keeps its own episode index and step-in-episode counter, ends its episode when one of ITS
+        platoons is terminal (global_break) or after steps_per_episode steps, then logs its rewards and resets only its own
+        platoons.  FRL predicates and the weighting window are evaluated per run.  A run that has finished its episodes is frozen
+        (its agents take no further update) while the others go on, so its weights end where the stand-alone run's do."""
+        env, conf, S = self.env, self.conf, self.S
+        if reward_logs is not None and len(reward_logs) != S:
+            raise ValueError(f"{len(reward_logs)} reward logs for {S} runs")
+        spe, Pr = int(conf.steps_per_episode), self.Gr * self.E
+        saved = env.auto_reset
+        env.auto_reset = False
+        self._in_run = True
+        self._run_ep, self._run_i = [self.episode] * S, [0] * S
+        left = [int(episodes)] * S
+        self.run_episode_steps = [[] for _ in range(S)]     # [run][episode]: env steps of each episode of this call
+        steps = 0
+        try:
+            if any(left):
+                env.reset()
+            while any(left):
+                active = [n > 0 for n in left]
+                self._step_runs(learn, active)
+                steps += 1
+                term = (env._done & 1).view(S, Pr).any(dim=1).tolist() if global_break else [False] * S
+                ending = []
+                for k in range(S):
+                    if active[k]:
+                        self._run_i[k] += 1
+                        if term[k] or self._run_i[k] >= spe:
+                            ending.append(k)
+                for k in ending:
+                    if reward_logs is not None:
+                        fw, fws = self.frl_weight_lists(k) if is_weighted_fed_enabled(conf, self._run_ep[k]) else (None, None)
+                        reward_logs[k].update_reward_list(self.episodic_rewards(k), fw, fws)
+                    self.run_episode_steps[k].append(self._run_i[k])
+                    self._run_ep[k] += 1
+                    self._run_i[k] = 0
+                    left[k] -= 1
+                restart = [k for k in ending if left[k] > 0]
+                if restart:
+                    env.reset(self._run_mask(restart, per="platoon"))
+            self.episode += int(episodes)
+        finally:
+            env.auto_reset = saved
+            self._in_run = False
+        return steps
+
+    def _run_mask(self, runs, per: str = "agent") -> torch.Tensor:
+        """uint8 device mask over agents [A] (a = m*G + k*Gr + g') or platoons [P] (p = k*Pr + p') of the listed runs."""
+        f = torch.zeros(self.S, dtype=torch.uint8)
+        f[list(runs)] = 1
+        if per == "platoon":
+            m = f.repeat_interleave(self.Gr * self.E)
+        else:
+            m = f.view(1, self.S, 1).expand(self.M, self.S, self.Gr).reshape(-1)
+        return m.to(self.pop.device)
+
+    def _step_runs(self, learn: bool, active):
+        """step() with per-run FRL predicates (run k at episode _run_ep[k], step _run_i[k]); runs not in `active` are frozen.  Runs on
+        an FRL step skip the local update (trainer.py:345) and take the federated round if it is a gradients round; the others take
+        their local Adam / Polyak step through the learn call's apply mask."""
+        env, pop, rings, conf, S = self.env, self.pop, self.rings, self.conf, self.S
+        pop.act(env.native_state, env.action_mu, self.E)
+        env.step_native(explore=True, gen_exog=True, advance_clock=False)
+        rings.clock.advance(step=1, ring=1)
+        self.buffer_counter += 1
+        if learn and self.buffer_counter > conf.batch_size:
+            s, a, r, s2 = rings.sample(advance_clock=True)
+            fed_step = [active[k] and self.fed is not None and is_valid_update_step(conf, self._run_i[k]) for k in range(S)]
+            grads = [fed_step[k] and is_valid_step_for_federated_training_with_gradients(conf, self._run_ep[k], self._run_i[k])
+                     for k in range(S)]
+            local = [k for k in range(S) if active[k] and not fed_step[k]]
+            pop.learn(s, a, r, s2, apply_updates=bool(local), apply_mask=self._run_mask(local))
+            if any(grads):
+                mask = self._run_mask([k for k in range(S) if grads[k]])
+                if self.fed.apply_mask is not None:
+                    mask = mask & self.fed.apply_mask
+                self.fed.aggregate_gradients(self._frl_weights_runs(), write_back=False, apply_mask=mask)
+        self.step_in_run += 1
+
+    def _frl_weights_runs(self):
+        """_frl_weights with per-run weighting windows: the FedAvg weights of every run past its window, 1 for the others (a plain
+        mean).  None while no run is past its window."""
+        conf = self.conf
+        plain = [k for k in range(self.S) if not is_weighted_fed_enabled(conf, self._run_ep[k])]
+        if len(plain) == self.S:
+            return None
+        w = self._frl_weights(self._run_ep[[k for k in range(self.S) if k not in plain][0]])
+        for k in plain:
+            if self.fed.inter:      # [M*S][Gr]: system m*S + k
+                w.view(self.M, self.S, self.Gr)[:, k, :] = 1.0
+            else:                   # [G][M]: systems k*Gr .. (k+1)*Gr - 1
+                w.view(self.S, self.Gr, self.M)[k] = 1.0
+        return w
 
     def capture(self, warmup: int = 3):
         """Capture one full step (learn included) into a CUDA graph; afterwards `replay()` costs one launch.  The host-side FRL

@@ -31,7 +31,7 @@ extern "C" {
 
 #define AVD_MAX_FOLLOWERS 16
 #define AVD_RING_RECORD_FLOATS 10
-#define AVD_ABI_VERSION 3
+#define AVD_ABI_VERSION 4
 
 typedef enum avd_status {
     AVD_OK = 0,
@@ -83,6 +83,19 @@ typedef struct avd_clock {
     uint64_t reserved;
 } avd_clock;
 
+/* ---- a batch of independent training runs.  The batch's P platoons are `runs` contiguous blocks of `platoons_per_run`:
+ * platoon p belongs to run s = p / platoons_per_run and draws the streams of platoon p mod platoons_per_run under seed[s]; ring
+ * m*P + p draws those of ring m*platoons_per_run + p mod platoons_per_run.  These are the keys a stand-alone run with
+ * random_seed = seed[s] uses, so run s of the batch reproduces it.  The struct itself is host memory: every entry that takes
+ * one checks runs * platoons_per_run == P and passes it to its kernels by value, so a captured CUDA graph replays it; the
+ * seeds it points to live in device memory.                                                                              */
+typedef struct avd_runs {
+    const uint64_t* seed;      /* [runs] DEVICE pointer: random_seed of every run                             */
+    int64_t platoons_per_run;  /* >= 1                                                                       */
+    int32_t runs;              /* >= 1                                                                       */
+    int32_t reserved;
+} avd_runs;
+
 /* ---- buffers of one shard of platoons (all device pointers; nullable ones are marked) */
 typedef struct avd_env_io {
     int64_t P;                 /* platoons in this shard                                             */
@@ -121,6 +134,9 @@ typedef struct avd_env_io {
      * all_ep_reward_lists[p][m][-weighted_window:] (trainer.py:385-398, 510-517) without leaving the device.              */
     float* last_ep_reward;     /* [M][P] nullable: cumulative reward of the last FINISHED episode              */
     float* ep_hist;            /* [ep_hist_window][M][P] nullable: ring of the last finished episodes' rewards */
+    const avd_runs* runs;      /* nullable HOST pointer: the platoons are several runs with their own seeds (seed is then
+                                  unused, platoon_id_base must be 0, runs->runs * runs->platoons_per_run must equal P);
+                                  NULL: one run keyed by (seed, platoon_id_base + p)                                         */
 } avd_env_io;
 
 /* ---- library ------------------------------------------------------------------------------- */
@@ -130,7 +146,7 @@ const char* avd_last_error(void);
  * callers difference it around a region, e.g. bench.py's "gpu_launches" */
 int64_t avd_kernel_launches(void);
 /* sizeof of the ABI structs as compiled (0 avd_env_params, 1 avd_env_io, 2 avd_clock, 3 avd_net_dims, 4 avd_learn_io,
- * 5 avd_peer_comm, 6 avd_fed_apply_io): bindings assert their own layout against these at load time. */
+ * 5 avd_peer_comm, 6 avd_fed_apply_io, 7 avd_runs): bindings assert their own layout against these at load time. */
 int64_t avd_sizeof(int which);
 /* SM count, compute capability major*10+minor of the current device; AVD_ERR_NO_DEVICE if none */
 int avd_device_info(int* sm_count, int* cc, int64_t* total_mem);
@@ -196,6 +212,13 @@ int avd_replay_gather(const float* ring, int64_t capacity, int64_t M, int64_t P,
 int avd_replay_sample(const float* ring, int64_t capacity, int64_t M, int64_t P, int64_t ring_id_base, int32_t batch, uint64_t seed,
                       const avd_clock* clock, int64_t* idx_out, float* s, float* a, float* r, float* s2, void* stream);
 
+/* The two entries above for a batch of runs (avd_runs, a host pointer): the same kernels, with every ring's Philox stream keyed by
+ * its run's seed and its ring id inside the run instead of (seed, ring_id_base + ring).  P (for the index draw: n_rings / M) must be
+ * runs * platoons_per_run; AVD_ERR_INVALID_ARG otherwise.                                                                          */
+int avd_replay_sample_indices_runs(int64_t* idx_out, int64_t n_rings, int32_t batch, int64_t capacity, const avd_runs* runs,
+                                   const avd_clock* clock, void* stream);
+int avd_replay_sample_runs(const float* ring, int64_t capacity, int64_t M, int64_t P, int32_t batch, const avd_runs* runs,
+                           const avd_clock* clock, int64_t* idx_out, float* s, float* a, float* r, float* s2, void* stream);
 
 /* Fill the whole ring with synthetic transitions (benchmark warm start: steady-state sampling
  * range without running `capacity` env steps).                                                    */
