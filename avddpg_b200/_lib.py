@@ -11,7 +11,7 @@ import os
 
 AVD_MAX_FOLLOWERS = 16
 RING_RECORD_FLOATS = 10
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 RNG_RESET_VEHICLE, RNG_RESET_PLATOON, RNG_OU, RNG_LEADER_EXOG, RNG_REPLAY, RNG_INIT = range(6)
 
@@ -44,7 +44,8 @@ class Clock(C.Structure):
 
 
 class Runs(C.Structure):
-    _fields_ = [("seed", C.c_void_p), ("platoons_per_run", C.c_int64), ("runs", C.c_int32), ("reserved", C.c_int32)]
+    _fields_ = [("seed", C.c_void_p), ("platoons_per_run", C.c_int64), ("runs", C.c_int32), ("reserved", C.c_int32),
+                ("ou_sigma", C.c_void_p), ("ou_theta", C.c_void_p)]
 
 
 class EnvIO(C.Structure):
@@ -79,7 +80,7 @@ class LearnIO(C.Structure):
         ("actor_t", C.c_void_p), ("critic_t", C.c_void_p),
         ("apply_mask", C.c_void_p), ("loss", C.c_void_p),
         ("workspace", C.c_void_p), ("workspace_bytes", C.c_int64),
-        ("precision", C.c_int32), ("s_stride", C.c_int32),
+        ("precision", C.c_int32), ("s_stride", C.c_int32), ("agent_hp", C.c_void_p),
     ]
 
 
@@ -102,6 +103,7 @@ class FedApplyIO(C.Structure):
         ("critic_grad_out", C.c_void_p), ("critic_total", C.c_int64), ("critic_train", C.c_int64),
         ("apply_mask", C.c_void_p), ("wsum_out", C.c_void_p),
         ("actor_lr", C.c_float), ("critic_lr", C.c_float), ("beta1", C.c_float), ("beta2", C.c_float), ("eps", C.c_float), ("tau", C.c_float),
+        ("agent_hp", C.c_void_p),
     ]
 
 
@@ -155,7 +157,8 @@ SIGNATURES = {
                                  C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "avd_adam_polyak_apply2": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
                                          C.c_float, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
-                                         C.c_int64, C.c_float, C.c_void_p, C.c_int32, C.c_float, C.c_float, C.c_float, C.c_float, C.c_void_p]),
+                                         C.c_int64, C.c_float, C.c_void_p, C.c_int32, C.c_float, C.c_float, C.c_float, C.c_float, C.c_void_p,
+                                         C.c_void_p]),
     "avd_fed_reduce2": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_int32, C.c_int32,
                                   C.c_int64, C.c_int64, C.c_void_p, C.c_void_p]),
     "avd_fed_broadcast2": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64, C.c_int32,

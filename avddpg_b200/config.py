@@ -8,7 +8,9 @@ of the reference Config are out of scope and not reproduced.
 """
 from __future__ import annotations
 
+import copy
 import ctypes as C
+import math
 
 from . import _lib
 
@@ -113,3 +115,40 @@ def env_params_from_config(conf, M: int, rand_states: bool = True, evaluator_sta
                                                   float(_get(conf, "timegap")), float(_get(conf, "dyn_coeff")),
                                                   float(_get(conf, "pl_leader_tau"))))
     return p
+
+
+# Config fields a run of a batched sweep may override (BatchedTrainer(..., seeds=..., overrides=...)): the scalars the learn step
+# and the OU noise read.  Every other field would change shapes or the environment and is shared by all runs of a batch.
+SWEEP_KEYS = ("actor_lr", "critic_lr", "gamma", "tau", "std_dev", "theta")
+
+
+def run_configs(conf, seeds, overrides=None) -> list:
+    """Effective configuration of every run of a batch: a copy of `conf` with random_seed = seeds[s] and the fields of overrides[s]
+    set.  overrides: None, or one dict per seed whose keys are among SWEEP_KEYS and whose values are finite numbers; a missing key
+    keeps conf's value.  Raises ValueError for any other key, a non-finite or non-numeric value, or a length mismatch.  Host only."""
+    if overrides is not None:
+        if seeds is None:
+            raise ValueError("overrides needs seeds: one dict per run")
+        overrides = list(overrides)
+        if len(overrides) != len(seeds):
+            raise ValueError(f"{len(overrides)} overrides for {len(seeds)} seeds")
+    out = []
+    for s, k in enumerate(seeds):
+        c = copy.copy(conf)
+        c.random_seed = k
+        d = {} if overrides is None else overrides[s]
+        if not isinstance(d, dict):
+            raise ValueError(f"overrides[{s}] must be a dict, got {type(d).__name__}")
+        bad = sorted(set(d) - set(SWEEP_KEYS))
+        if bad:
+            raise ValueError(f"overrides[{s}]: {bad} cannot differ between the runs of a batch (allowed: {', '.join(SWEEP_KEYS)})")
+        for key, v in d.items():
+            try:
+                f = float(v)
+            except (TypeError, ValueError):
+                raise ValueError(f"overrides[{s}][{key!r}] = {v!r} is not a number") from None
+            if isinstance(v, bool) or not math.isfinite(f):
+                raise ValueError(f"overrides[{s}][{key!r}] = {v!r} is not a finite number")
+            setattr(c, key, f)
+        out.append(c)
+    return out

@@ -305,7 +305,10 @@ __global__ void __launch_bounds__(256) action_grad_kernel(avd_net_dims d, const 
 // ------------------------------------------------------------------------------------------------
 // heads: everything after the l2-wide GEMM.  One warp per row, lane owns columns lane, lane+32, ...
 // ------------------------------------------------------------------------------------------------
-enum HeadMode { HEAD_ACTOR_FWD = 0, HEAD_CRITIC_TARGET = 1, HEAD_CRITIC_Q = 2, HEAD_CRITIC_BWD = 3, HEAD_CRITIC_BWD_ACTION = 4, HEAD_ACTOR_BWD = 5 };
+// HEAD_CRITIC_TARGET_HP: the TD target with every agent's own gamma (HeadArgs.hp); a mode of its own so that HEAD_CRITIC_TARGET
+// compiles to the kernel it was before.
+enum HeadMode { HEAD_ACTOR_FWD = 0, HEAD_CRITIC_TARGET = 1, HEAD_CRITIC_Q = 2, HEAD_CRITIC_BWD = 3, HEAD_CRITIC_BWD_ACTION = 4, HEAD_ACTOR_BWD = 5,
+                HEAD_CRITIC_TARGET_HP = 6 };
 
 struct HeadArgs {
     const float* params;   // [A][pstride]
@@ -314,6 +317,7 @@ struct HeadArgs {
     const float* Z;        // [A*R][L2] raw GEMM output (bias not yet added)
     int64_t R;
     float high, gamma;
+    const float* hp;       // TARGET_HP: [A][4] per-agent (gamma, ...); gamma of agent a = hp[4 a] instead of `gamma`
     const float* rew;      // TARGET
     const float* y;        // CRITIC_BWD
     const float* dpi;      // ACTOR_BWD
@@ -365,8 +369,9 @@ __global__ void __launch_bounds__(256) head_kernel(HeadArgs h) {
         const float pre = warp_sum(part) + b3;
         if (MODE == HEAD_ACTOR_FWD) {
             if (lane == 0) h.out[n] = h.high * tanhf(pre);
-        } else if (MODE == HEAD_CRITIC_TARGET) {
-            if (lane == 0) h.out[n] = h.rew[n] + h.gamma * pre;   // trainer.py:494 (no terminal mask)
+        } else if (MODE == HEAD_CRITIC_TARGET || MODE == HEAD_CRITIC_TARGET_HP) {
+            const float gamma = MODE == HEAD_CRITIC_TARGET_HP ? h.hp[4 * agent] : h.gamma;
+            if (lane == 0) h.out[n] = h.rew[n] + gamma * pre;      // trainer.py:494 (no terminal mask)
         } else if (MODE == HEAD_CRITIC_Q) {
             if (lane == 0) h.out[n] = pre;
         } else {
@@ -540,14 +545,20 @@ struct AdamNet {
 };
 struct AdamNets { AdamNet n[2]; };
 
-__global__ void __launch_bounds__(256) adam_polyak2_kernel(AdamNets nets, const uint8_t* __restrict__ mask, float b1, float b2, float eps, float tau) {
+// HP: per-agent learning rates and tau from hp[A][4] = (gamma, actor_lr, critic_lr, tau) (avd_learn_io.agent_hp), same arithmetic; a
+// template parameter so that the launch without a table compiles to the kernel it was before.
+template <bool HP>
+__global__ void __launch_bounds__(256) adam_polyak2_kernel(AdamNets nets, const uint8_t* __restrict__ mask, float b1, float b2, float eps, float tau,
+                                                           const float* __restrict__ hp) {
     pdl_wait();                  // launched with programmatic dependent launch (avd_common.cuh): every CTA waits before it reads or exits
     pdl_launch_dependents();
     const AdamNet& nt = nets.n[blockIdx.z];
     const int agent = blockIdx.y;
     if (mask && !mask[agent]) return;
+    const float lr = HP ? hp[4 * agent + (blockIdx.z == 0 ? 2 : 1)] : nt.lr;      // n[0] is the critic
+    if (HP) tau = hp[4 * agent + 3];
     const float t = (float)(nt.step[agent] + 1);
-    const float lr_t = nt.lr * sqrtf(1.0f - powf(b2, t)) / (1.0f - powf(b1, t));
+    const float lr_t = lr * sqrtf(1.0f - powf(b2, t)) / (1.0f - powf(b1, t));
     float* P = nt.params + (int64_t)agent * nt.pstride;
     float* T = nt.target + (int64_t)agent * nt.pstride;
     const float* G = nt.grads + (int64_t)agent * nt.gstride;
@@ -1577,7 +1588,7 @@ extern "C" int avd_adam_polyak_apply2(float* actor, float* t_actor, int64_t acto
                                       float* actor_m, float* actor_v, int32_t* actor_step, int64_t actor_train, float actor_lr, float* critic,
                                       float* t_critic, int64_t critic_total, const float* critic_grad, int64_t critic_gstride, float* critic_m,
                                       float* critic_v, int32_t* critic_step, int64_t critic_train, float critic_lr, const uint8_t* apply_mask,
-                                      int32_t A, float beta1, float beta2, float eps, float tau, void* stream) {
+                                      int32_t A, float beta1, float beta2, float eps, float tau, const float* agent_hp, void* stream) {
     AVD_REQUIRE(actor && t_actor && actor_grad && actor_m && actor_v && actor_step && critic && t_critic && critic_grad && critic_m && critic_v &&
                     critic_step,
                 "null buffer");
@@ -1588,7 +1599,9 @@ extern "C" int avd_adam_polyak_apply2(float* actor, float* t_actor, int64_t acto
     nets.n[0] = AdamNet{critic, t_critic, critic_grad, critic_m, critic_v, critic_step, critic_total, critic_gstride, critic_train, critic_total, critic_lr};
     nets.n[1] = AdamNet{actor, t_actor, actor_grad, actor_m, actor_v, actor_step, actor_total, actor_gstride, actor_train, actor_total, actor_lr};
     const int64_t blocks = std::min<int64_t>((std::max(critic_total, actor_total) + 255) / 256, 1024);
-    AVD_CUDA_OK(launch_pdl(adam_polyak2_kernel, dim3((unsigned)blocks, (unsigned)A, 2), dim3(256), 0, st, nets, apply_mask, beta1, beta2, eps, tau));
+    const dim3 grid((unsigned)blocks, (unsigned)A, 2);
+    if (agent_hp) AVD_CUDA_OK(launch_pdl(adam_polyak2_kernel<true>, grid, dim3(256), 0, st, nets, apply_mask, beta1, beta2, eps, tau, agent_hp));
+    else AVD_CUDA_OK(launch_pdl(adam_polyak2_kernel<false>, grid, dim3(256), 0, st, nets, apply_mask, beta1, beta2, eps, tau, agent_hp));
     AVD_LAUNCH_OK();
     AVD_CUDA_OK(launch_pdl(step_increment2_kernel, dim3((unsigned)((A + 127) / 128)), dim3(128), 0, st, actor_step, critic_step, apply_mask, (int)A));
     AVD_LAUNCH_OK();
@@ -1684,7 +1697,7 @@ static int apply_local_updates(const avd_learn_io* io, void* stream) {
     AVD_TRY(avd_adam_polyak_apply2(io->actor, io->t_actor, ao.total, io->actor_grad, ao.n_train, io->actor_m, io->actor_v, io->actor_t, ao.n_train,
                                    io->actor_lr, io->critic, io->t_critic, co.total, io->critic_grad, co.n_train, io->critic_m, io->critic_v,
                                    io->critic_t, co.n_train, io->critic_lr, io->apply_mask, A, io->adam_beta1, io->adam_beta2, io->adam_eps,
-                                   io->tau, stream));
+                                   io->tau, io->agent_hp, stream));
     return AVD_OK;
 }
 
@@ -1828,7 +1841,7 @@ static int learn_fused3(const avd_learn_io* io, const Pass& p, const Workspace& 
     tm.mark("t_actor");
     {
         fused3::RunArgs f = p.fused_args(fused3::MODE_TARGET, io->t_critic, w.tcW2T, w.tc_b2f, io->s2, srs);
-        f.act = w.a2; f.rew = io->r; f.gamma = io->gamma; f.out = w.y;
+        f.act = w.a2; f.rew = io->r; f.gamma = io->gamma; f.hp = io->agent_hp; f.out = w.y;
         AVD_TRY(fused3::run(f, st));
     }
     tm.mark("t_critic");
@@ -1951,8 +1964,9 @@ extern "C" int avd_ddpg_learn(const avd_learn_io* io, void* stream) {
     AVD_TRY(p.forward(w.H, F, io->t_critic, co.total, co.W2, w.tcW2T, w.Z));
     {
         HeadArgs h = critic_head(d, io->t_critic, w.Z, R);
-        h.rew = io->r; h.gamma = io->gamma; h.out = w.y;
-        AVD_TRY(launch_head<HEAD_CRITIC_TARGET>(h, d.l2, A, st));
+        h.rew = io->r; h.gamma = io->gamma; h.hp = io->agent_hp; h.out = w.y;
+        if (io->agent_hp) AVD_TRY(launch_head<HEAD_CRITIC_TARGET_HP>(h, d.l2, A, st));
+        else AVD_TRY(launch_head<HEAD_CRITIC_TARGET>(h, d.l2, A, st));
     }
     // ---- critic loss gradient on (s, a)                                             trainer.py:495-498
     AVD_TRY(p.layer1(true, io->critic, io->s, srs, 1, io->a, w.H));

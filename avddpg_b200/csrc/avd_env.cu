@@ -156,16 +156,18 @@ __device__ __forceinline__ FollowerIn load_follower(const StepCtx& c, int64_t v)
 // input on entry and the next follower's on exit.  Returns the (negated) reward; sets `term`.
 // (Sharing one Philox block + Box-Muller transform between two followers -- z0 / z1 -- was measured in round 2: 5 % slower at M = 4,
 // 3 % faster at M = 8, 10 % slower plain M = 8 launches from the changed register allocation; every follower keeps its own block.)
+// ou_theta / ou_c: the platoon's OU theta and sigma * sqrt(dt) (its run's values when the batch holds several runs).
 __device__ __forceinline__ float step_follower(const avd_env_params& prm, const avd_env_io& io, const StepCtx& c,
-                                               const FollowerIn& f, int m, int M, int64_t p, StreamKey key, float& w, bool& term) {
+                                               const FollowerIn& f, int m, int M, int64_t p, StreamKey key, float ou_theta, float ou_c,
+                                               float& w, bool& term) {
     const int64_t v = (int64_t)m * c.P + p;
     float u = f.mu;
     if (c.ou_state) {  // noise.py:14-23 with explicit single roundings (bit-exact vs the host restatement)
         float z0, z1;
         const uint4 wo = rng_words(key.seed, key.id * (uint64_t)M + (uint64_t)m, c.tick, AVD_RNG_OU);
         normal_pair(wo.x, wo.y, z0, z1);
-        const float drift = __fmul_rn(__fmul_rn(prm.ou_theta, __fadd_rn(prm.ou_mean, -f.ou)), prm.ou_dt);
-        const float n1 = __fadd_rn(__fadd_rn(f.ou, drift), __fmul_rn(c.ou_c, z0));
+        const float drift = __fmul_rn(__fmul_rn(ou_theta, __fadd_rn(prm.ou_mean, -f.ou)), prm.ou_dt);
+        const float n1 = __fadd_rn(__fadd_rn(f.ou, drift), __fmul_rn(ou_c, z0));
         c.ou_state[v] = n1;
         u = __fadd_rn(u, n1);
     }
@@ -223,6 +225,7 @@ __device__ __forceinline__ float step_follower(const avd_env_params& prm, const 
 // for platoons longer than 4 chunks of 2 followers, which fit 64 registers without spilling.  Measured on 4 Mi platoons (launch
 // time, us; `chunk / CTAs per SM`):      M = 4:  4/3 428   4/4 370   2/4 388   2/5 388        M = 8:  4/3 881   4/4 1002   2/4 829   2/5 959
 // RUNS: the batch holds several runs (rt, a copy of *io.runs); a separate instantiation because the run-table lookup costs registers.
+// Only these instantiations read the optional per-run OU parameters (rt.ou_sigma / rt.ou_theta).
 template <int MT, bool TRAIN, bool RUNS>
 __global__ void __launch_bounds__(256, MT >= 1 ? (TRAIN ? 4 : 3) : 2)
     env_step_kernel(const __grid_constant__ avd_env_params prm, const __grid_constant__ avd_env_io io, const __grid_constant__ avd_runs rt) {
@@ -252,6 +255,12 @@ __global__ void __launch_bounds__(256, MT >= 1 ? (TRAIN ? 4 : 3) : 2)
 
     for (int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < P; p += (int64_t)gridDim.x * blockDim.x) {
         const StreamKey key = platoon_key(runs, io.seed, (uint64_t)(io.platoon_id_base + p));
+        float ou_theta = prm.ou_theta, ou_c = c.ou_c;
+        if (RUNS && TRAIN) {      // (a plain step has no OU noise)
+            const uint64_t run = (uint64_t)p / (uint64_t)rt.platoons_per_run;
+            if (rt.ou_theta) ou_theta = rt.ou_theta[run];
+            if (rt.ou_sigma) ou_c = __fmul_rn(rt.ou_sigma[run], __fsqrt_rn(prm.ou_dt));
+        }
         constexpr int CH = MT > 4 ? (TRAIN ? 2 : 4) : (MT ? MT : 1);       // followers preloaded at a time
         FollowerIn fin[CH];
         if (MT) {
@@ -282,7 +291,7 @@ __global__ void __launch_bounds__(256, MT >= 1 ? (TRAIN ? 4 : 3) : 2)
                 for (int j = 0; j < CH; ++j) {
                     if (m0 + j < MT) {
                         bool term;
-                        const float r = step_follower(prm, io, c, fin[j], m0 + j, MT, p, key, w, term);
+                        const float r = step_follower(prm, io, c, fin[j], m0 + j, MT, p, key, ou_theta, ou_c, w, term);
                         any_term |= term;
                         rew_sum += r;
                         stat_r[m0 + j] += r;
@@ -293,7 +302,7 @@ __global__ void __launch_bounds__(256, MT >= 1 ? (TRAIN ? 4 : 3) : 2)
             for (int m = 0; m < M; ++m) {
                 bool term;
                 const FollowerIn f = load_follower(c, (int64_t)m * P + p);
-                const float r = step_follower(prm, io, c, f, m, M, p, key, w, term);
+                const float r = step_follower(prm, io, c, f, m, M, p, key, ou_theta, ou_c, w, term);
                 any_term |= term;
                 rew_sum += r;
                 stat_r[m] += r;

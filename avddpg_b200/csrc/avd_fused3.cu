@@ -64,6 +64,7 @@ struct Args {
     const float* act;           // [A*R] critic passes
     const float* rew;           // MODE_TARGET
     float gamma, high;
+    const float* hp;            // MODE_TARGET, nullable: gamma of agent a = hp[4 a] instead of `gamma`
     const float* y;             // MODE_CRITIC_BWD: TD targets
     float* out;                 // forward modes: [A*R]; MODE_CRITIC_ACTION: d loss / d action; MODE_CRITIC_BWD: q (nullable)
     uint32_t* mask_out;         // backward modes / MODE_ACTOR_SAVE: [A*R][mask_words] sign bits of z1 (column j of word w at bit 31-j)
@@ -310,6 +311,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) fused3_kernel(const __grid_con
         const int row = q * 32 + lane;
         const uint32_t tlane = (uint32_t)(q * 32) << 16;
         const float invR = 1.0f / (float)g.R;
+        const float gamma = (MODE == MODE_TARGET && g.hp) ? g.hp[4 * agent] : g.gamma;     // one agent per CTA
         float sdq_acc = 0.0f, loss_acc = 0.0f;
         uint32_t zneg = 0u;                  // backward modes: sign bits of z2 + b2' of this thread's 32 columns (column j at bit 31 - j), pass 1 -> pass 2
 
@@ -504,7 +506,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) fused3_kernel(const __grid_con
                     o = g.high * t;
                     if (SAVE && valid) g.dact_out[nrow] = g.high * (1.0f - t * t);       // through high * tanh(.)    model.py:36-37
                 }
-                else if (MODE == MODE_TARGET) o = yv + g.gamma * qv;                 // trainer.py:494 (no terminal mask)
+                else if (MODE == MODE_TARGET) o = yv + gamma * qv;                   // trainer.py:494 (no terminal mask)
                 else if (ACTION) {                                                   // d(-mean q)/d a   trainer.py:503-506
                     const float* pg = part2 + buf * 4 * TILE_M + row;
                     o = -invR * (pg[0] + pg[TILE_M] + pg[2 * TILE_M] + pg[3 * TILE_M]);
@@ -635,7 +637,7 @@ int run(const RunArgs& a, cudaStream_t st) {
         if (int rc = make_tensor_map(&tmDZ, a.DZ_out, L2N, (uint64_t)R, (uint64_t)A, L2N, (uint64_t)R * L2N, KB, TILE_M)) return rc;
     Args g;
     g.d = d; g.A = A; g.R = R; g.params = a.params; g.pstride = a.pstride; g.b2f = a.b2f; g.s = a.s; g.s_rs = a.s_rs; g.s_cs = a.s_cs; g.act = a.act;
-    g.rew = a.rew; g.gamma = a.gamma; g.high = a.high; g.y = a.y; g.out = a.out; g.mask_out = a.mask_out; g.mask_words = 2 * ((F + KB - 1) / KB);
+    g.rew = a.rew; g.gamma = a.gamma; g.hp = a.hp; g.high = a.high; g.y = a.y; g.out = a.out; g.mask_out = a.mask_out; g.mask_words = 2 * ((F + KB - 1) / KB);
     g.vtab = a.vtab; g.dm_scale = a.dm_scale; g.sdq = a.sdq; g.loss = a.loss; g.mask2_out = a.mask2_out; g.dact_out = a.dact_out;
     g.tiles_per_agent = (int)((R + TILE_M - 1) / TILE_M);
     g.ctas_per_agent = ctas_per_agent(A, R);

@@ -42,6 +42,7 @@ struct RunArgs {
     const float* act = nullptr;     // [A*R] critic passes
     const float* rew = nullptr;     // MODE_TARGET
     float gamma = 0.f, high = 0.f;
+    const float* hp = nullptr;      // MODE_TARGET, nullable: [A][4] per-agent (gamma, ...) (avd_learn_io.agent_hp) in place of gamma
     const float* y = nullptr;       // MODE_CRITIC_BWD: TD targets
     const float* vtab = nullptr;    // MODE_CRITIC_ACTION: [A][vtab_floats()] from critic_vtab_kernel
     float* out = nullptr;           // forward modes: [A*R]; MODE_CRITIC_ACTION: d loss / d action; MODE_CRITIC_BWD: q (nullable)

@@ -144,16 +144,24 @@ struct ApplyArgs {
     const uint8_t* mask;                   // [A] nullable: agents with 0 keep their weights
     float b1, b2, eps, tau;
     float* wsum_out;                       // [systems] nullable: the reduced divisor
+    const float* hp;                       // [A][4] (gamma, actor_lr, critic_lr, tau) per agent; read by the HP instantiation only
 };
 
+// HP: every agent takes its learning rates and tau from a.hp (same arithmetic as with the scalars); the table then holds [3][A]
+// floats -- the two lr_t rows and tau -- instead of [2][A], which lowers the largest A from 25,600 to 17,066 (200 KB).
+template <bool HP>
 __global__ void __launch_bounds__(256) fed_apply_kernel(ApplyArgs a) {
-    extern __shared__ float lr_tab[];      // [2][A]: lr * sqrt(1 - b2^t) / (1 - b1^t) per net and agent, t = step + 1
+    extern __shared__ float lr_tab[];      // [2][A]: lr * sqrt(1 - b2^t) / (1 - b1^t) per net and agent, t = step + 1;  HP: + [A] tau
     const PeerCore& g = a.core;
     for (int i = threadIdx.x; i < 2 * a.A; i += blockDim.x) {
         const ApplyNet& nt = a.net[i / a.A];
         const float t = (float)(nt.step[i % a.A] + 1);
-        lr_tab[i] = nt.lr * sqrtf(1.0f - powf(a.b2, t)) / (1.0f - powf(a.b1, t));
+        const float lr = HP ? a.hp[4 * (i % a.A) + (i < a.A ? 1 : 2)] : nt.lr;      // net[0] is the actor
+        lr_tab[i] = lr * sqrtf(1.0f - powf(a.b2, t)) / (1.0f - powf(a.b1, t));
     }
+    const float* tau_tab = lr_tab + 2 * a.A;
+    if (HP)
+        for (int i = threadIdx.x; i < a.A; i += blockDim.x) lr_tab[2 * a.A + i] = a.hp[4 * i + 3];
     peer_barrier(g);                       // ends with __syncthreads(): the table is complete
     const int64_t na = a.net[0].n_train;
     const float omt = 1.0f - a.tau;
@@ -194,7 +202,8 @@ __global__ void __launch_bounds__(256) fed_apply_kernel(ApplyArgs a) {
                 *Vv = vi;
                 const float p = *Pp - lr_tab[k * a.A + (int)ag] * mi / (sqrtf(vi) + a.eps);
                 *Pp = p;
-                *Tt = p * a.tau + *Tt * omt;
+                if (HP) *Tt = p * tau_tab[ag] + *Tt * (1.0f - tau_tab[ag]);
+                else *Tt = p * a.tau + *Tt * omt;
             }
         }
     }
@@ -207,7 +216,8 @@ __global__ void __launch_bounds__(256) fed_apply_kernel(ApplyArgs a) {
         const ApplyNet& nt = a.net[r < tail0 ? 0 : 1];
         const int64_t idx = nt.n_train + (r < tail0 ? r : r - tail0);
         float* Tt = nt.target + ag * nt.total + idx;
-        *Tt = nt.params[ag * nt.total + idx] * a.tau + *Tt * omt;
+        if (HP) *Tt = nt.params[ag * nt.total + idx] * tau_tab[ag] + *Tt * (1.0f - tau_tab[ag]);
+        else *Tt = nt.params[ag * nt.total + idx] * a.tau + *Tt * omt;
     }
     if (peer_round_done(g)) {              // every CTA has built its lr table: the step counters may advance now
         for (int i = threadIdx.x; i < a.A; i += blockDim.x)
@@ -264,17 +274,19 @@ extern "C" int avd_fed_apply_gradients(const avd_fed_apply_io* io, void* stream)
     a.net[0] = ApplyNet{io->actor, io->t_actor, io->actor_m, io->actor_v, io->actor_step, io->actor_grad_out, io->actor_total, io->actor_train, io->actor_lr};
     a.net[1] = ApplyNet{io->critic, io->t_critic, io->critic_m, io->critic_v, io->critic_step, io->critic_grad_out, io->critic_total, io->critic_train, io->critic_lr};
     a.n_members = io->n_members; a.A = io->A; a.stride_s = io->member_stride_s; a.stride_x = io->member_stride_x; a.mask = io->apply_mask;
-    a.b1 = io->beta1; a.b2 = io->beta2; a.eps = io->eps; a.tau = io->tau; a.wsum_out = io->wsum_out;
-    const size_t smem = (size_t)2 * io->A * sizeof(float);
-    AVD_REQUIRE(smem <= 200 * 1024, "too many agents per rank for the fused federated consumer (%d)", io->A);
-    static size_t smem_set = 48 * 1024;
-    if (smem > smem_set) {
-        AVD_CUDA_OK(cudaFuncSetAttribute(fed_apply_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        smem_set = smem;
+    a.b1 = io->beta1; a.b2 = io->beta2; a.eps = io->eps; a.tau = io->tau; a.wsum_out = io->wsum_out; a.hp = io->agent_hp;
+    const bool hp = io->agent_hp != nullptr;
+    const size_t smem = (size_t)(hp ? 3 : 2) * io->A * sizeof(float);
+    AVD_REQUIRE(smem <= 200 * 1024, "too many agents per rank for the fused federated consumer (%d%s)", io->A, hp ? " with a per-agent table" : "");
+    static size_t smem_set[2] = {48 * 1024, 0};      // with a table: set the limit on first use (the kernel also has static shared memory)
+    if (smem > smem_set[hp]) {
+        AVD_CUDA_OK(cudaFuncSetAttribute(hp ? fed_apply_kernel<true> : fed_apply_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        smem_set[hp] = smem;
     }
     const int64_t work = (int64_t)io->n_systems * (io->pitch / 4);
     const int grid = (int)std::min<int64_t>((work + 255) / 256, 2 * sm_count());
-    fed_apply_kernel<<<grid, 256, smem, (cudaStream_t)stream>>>(a);
+    if (hp) fed_apply_kernel<true><<<grid, 256, smem, (cudaStream_t)stream>>>(a);
+    else fed_apply_kernel<false><<<grid, 256, smem, (cudaStream_t)stream>>>(a);
     AVD_LAUNCH_OK();
     return AVD_OK;
 }

@@ -50,9 +50,10 @@ class RunTable:
     """S independent training runs that share one batch of P = S * platoons_per_run platoons (avd_runs: a host struct the library
     checks and hands to its kernels by value, over a device array of the seeds, so a captured CUDA graph replays it).  Run s owns
     platoons [s * Pr, (s + 1) * Pr) and draws every random stream of the stand-alone run with random_seed = seeds[s]: its platoon
-    p' is keyed (seeds[s], p') and its ring m * Pr + p' likewise."""
+    p' is keyed (seeds[s], p') and its ring m * Pr + p' likewise.  ou_sigma / ou_theta: optional per-run OU std_dev / theta (one value
+    per seed) in place of the configuration's, for a hyperparameter sweep; None keeps the configuration's value for every run."""
 
-    def __init__(self, seeds, platoons_per_run: int, device):
+    def __init__(self, seeds, platoons_per_run: int, device, ou_sigma=None, ou_theta=None):
         seeds = [int(k) for k in seeds]
         if not seeds:
             raise ValueError("a run table needs at least one seed")
@@ -66,6 +67,18 @@ class RunTable:
         self.seed_t = torch.tensor([k - (1 << 64) if k >= 1 << 63 else k for k in seeds], dtype=torch.int64, device=device)
         self.table = _lib.Runs()
         self.table.seed, self.table.platoons_per_run, self.table.runs = self.seed_t.data_ptr(), self.Pr, self.S
+        self.ou_sigma = self._per_run("ou_sigma", ou_sigma, device)
+        self.ou_theta = self._per_run("ou_theta", ou_theta, device)
+        self.table.ou_sigma = None if self.ou_sigma is None else self.ou_sigma.data_ptr()
+        self.table.ou_theta = None if self.ou_theta is None else self.ou_theta.data_ptr()
+
+    def _per_run(self, name, values, device):
+        if values is None:
+            return None
+        values = [float(v) for v in values]
+        if len(values) != self.S:
+            raise ValueError(f"{name}: {len(values)} values for {self.S} runs")
+        return torch.tensor(values, dtype=torch.float32, device=device)
 
     @property
     def ptr(self):

@@ -157,7 +157,8 @@ class FederatedAggregator:
         "nccl" = all_reduce + finalize,
         "auto" = peer when the group spans several CUDA ranks and symmetric memory can be set up ON EVERY RANK, else nccl.
         runs: the population's groups are `runs` independent runs of G / runs groups (DDPGPopulation seeds); interfrl then averages
-        each follower over the groups of its own run."""
+        each follower over the groups of its own run.  A population with per-run overrides (DDPGPopulation.hp) applies every round
+        with each agent's own learning rates and tau."""
         self.pop, self.conf, self.pg = population, conf, process_group
         self.lib = _lib.load()
         if conf.fed_method not in ("interfrl", "intrafrl"):
@@ -304,6 +305,7 @@ class FederatedAggregator:
             io.critic, io.t_critic, io.critic_m, io.critic_v, io.critic_step = c.flat.data_ptr(), pop.t_critic.flat.data_ptr(), c.m.data_ptr(), c.v.data_ptr(), c.step.data_ptr()
             io.actor_total, io.actor_train, io.critic_total, io.critic_train = a.total, a.n_train, c.total, c.n_train
             io.wsum_out = self.wsum.data_ptr()
+            io.agent_hp = None if pop.hp is None else pop.hp.data_ptr()      # per-run learning rates and tau (DDPGPopulation overrides)
             io.actor_lr, io.critic_lr, io.beta1, io.beta2, io.eps, io.tau = float(conf.actor_lr), float(conf.critic_lr), 0.9, 0.999, 1e-7, float(conf.tau)
             self._apply_io = io
         io = self._apply_io

@@ -15,6 +15,7 @@ single-agent model objects from avddpg_b200.model.
 """
 from __future__ import annotations
 
+import copy
 import ctypes as C
 from typing import Optional, Sequence
 
@@ -27,9 +28,13 @@ from .model import NetBank, dims_from_config
 
 class DDPGPopulation:
     def __init__(self, num_groups: int, num_followers: int, config, *, num_states: int = 4, rows_per_agent: int = 64,
-                 device=None, seed: Optional[int] = None, precision: int = 0, seeds: Optional[Sequence[int]] = None):
+                 device=None, seed: Optional[int] = None, precision: int = 0, seeds: Optional[Sequence[int]] = None,
+                 overrides: Optional[Sequence[dict]] = None):
         """seeds: the G groups are len(seeds) independent runs of G / len(seeds) groups each; run s starts from the weights the
-        stand-alone population with seed seeds[s] draws (its agents m*G + s*Gr + g', see run_agents)."""
+        stand-alone population with seed seeds[s] draws (its agents m*G + s*Gr + g', see run_agents).
+        overrides: one dict per seed (config.run_configs): run s learns with its own gamma, actor_lr, critic_lr and tau.  They go into
+        the per-agent table `hp` [A, 4] = (gamma, actor_lr, critic_lr, tau), which learn() and apply_gradients_and_soft_update()
+        (and so FederatedAggregator) use in place of the config scalars; without overrides `hp` is None."""
         self.lib = _lib.load()
         _lib.require_device()
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
@@ -56,6 +61,13 @@ class DDPGPopulation:
                 self.actor.init_reference(gen, agents)
                 self.critic.init_reference(gen, agents)
         self.sync_targets()
+        self.hp = None
+        if overrides is not None:
+            from .config import run_configs
+            confs = run_configs(config, seeds, overrides)
+            rows = [[float(c.gamma), float(c.actor_lr), float(c.critic_lr), float(c.tau)] for c in confs]
+            Gr = self.G // self.S
+            self.hp = torch.tensor([rows[(a % self.G) // Gr] for a in range(self.A)], dtype=torch.float32, device=dev)
         self.loss = torch.zeros(self.A, 2, dtype=torch.float32, device=dev)
         self._ws = None
         self._act_ws = None
@@ -122,11 +134,13 @@ class DDPGPopulation:
         io.loss = self.loss.data_ptr()
         io.workspace, io.workspace_bytes = ws.data_ptr(), ws.numel()
         io.precision, io.s_stride = self.precision, 4         # the replay gather writes 4 state words per row; dims.ns of them are read
+        io.agent_hp = None if self.hp is None else self.hp.data_ptr()
         _lib.check(self.lib.avd_ddpg_learn(C.byref(io), _lib.current_stream()))
         return self.critic.grad, self.actor.grad
 
     def apply_gradients(self, apply_mask: Optional[torch.Tensor] = None):
         """optimizer.apply_gradients for both nets with whatever is in .grad (trainer.py:348-349 / 420-425)."""
+        self._refuse_table("apply_gradients")
         conf = self.config
         for bank, lr in ((self.critic, conf.critic_lr), (self.actor, conf.actor_lr)):
             _lib.check(self.lib.avd_adam_apply(_lib.ptr(bank.flat), bank.total, _lib.ptr(bank.grad), bank.n_train, _lib.ptr(bank.m),
@@ -140,10 +154,16 @@ class DDPGPopulation:
             _lib.ptr(a.flat), _lib.ptr(self.t_actor.flat), a.total, _lib.ptr(a.grad), a.n_train, _lib.ptr(a.m), _lib.ptr(a.v), _lib.ptr(a.step),
             a.n_train, float(conf.actor_lr), _lib.ptr(c.flat), _lib.ptr(self.t_critic.flat), c.total, _lib.ptr(c.grad), c.n_train, _lib.ptr(c.m),
             _lib.ptr(c.v), _lib.ptr(c.step), c.n_train, float(conf.critic_lr), _lib.ptr(apply_mask), self.A, 0.9, 0.999, 1e-7, float(conf.tau),
-            _lib.current_stream()))
+            _lib.ptr(self.hp), _lib.current_stream()))
+
+    def _refuse_table(self, what):
+        if self.hp is not None:
+            raise NotImplementedError(f"{what} applies the config's scalars; a population with per-run overrides updates through "
+                                      "learn() or apply_gradients_and_soft_update()")
 
     def soft_update(self, apply_mask: Optional[torch.Tensor] = None):
         """ddpgagent.update_target + set_weights for every agent (trainer.py:352-356)."""
+        self._refuse_table("soft_update")
         for tgt, onl in ((self.t_critic, self.critic), (self.t_actor, self.actor)):
             _lib.check(self.lib.avd_polyak_update(_lib.ptr(tgt.flat), _lib.ptr(onl.flat), _lib.ptr(apply_mask), self.A, onl.total,
                                                   float(self.config.tau), _lib.current_stream()))
@@ -165,13 +185,24 @@ class BatchedTrainer:
     seeds=[k_0, ..., k_{S-1}] hosts S independent runs of num_groups x envs_per_group platoons each: run s behaves like the
     stand-alone trainer with random_seed = k_s (its draws, initial weights, FRL systems, episodes and reward log) and owns groups
     [s*Gr, (s+1)*Gr) of the G = S*Gr here (Gr = num_groups), so its platoons and rings are contiguous.  Single GPU only.
+
+    overrides=[d_0, ..., d_{S-1}] (with seeds, one dict per run) makes the batch a hyperparameter sweep: run s reproduces the stand-alone
+    trainer built from run_config(s), a copy of conf with random_seed = k_s and the fields of d_s set.  The keys may be actor_lr,
+    critic_lr, gamma, tau, std_dev and theta (config.SWEEP_KEYS); seeds may repeat.  Two runs that share a seed write CSV files of the
+    same names (reward_logs()), so give their logs different output directories.
     """
 
     def __init__(self, conf, num_groups: int, envs_per_group: int = 1, *, ring_capacity=None, rank: int = 0, world: int = 1,
                  process_group=None, precision: int = 0, seed=None, track_kinematics: bool = False, fed_transport: str = "auto",
-                 seeds=None):
+                 seeds=None, overrides=None):
+        from .config import run_configs
         from .environment import BatchedPlatoons, RunTable
         from .replaybuffer import ReplayRings
+        # validated before anything is allocated; without seeds: the one run of conf
+        if seeds is None and overrides is not None:
+            raise ValueError("overrides needs seeds: one dict per run")
+        self._run_confs = run_configs(conf, [int(getattr(conf, "random_seed", 1))] if seeds is None else seeds, overrides)
+        self.overrides = None if overrides is None else [dict(d) for d in overrides]
         self.S = 1 if seeds is None else len(seeds)
         self.conf, self.Gr, self.E, self.M = conf, int(num_groups), int(envs_per_group), int(conf.pl_size)
         self.G = self.Gr * self.S
@@ -184,7 +215,9 @@ class BatchedTrainer:
             if is_fed_enabled(conf) and is_model_weight_updates_enabled(conf):
                 # run()'s per-run loop has gradient rounds only, so even one seed would silently train unlike its stand-alone run
                 raise NotImplementedError("weights-mode FRL is not available for trainers built with seeds")
-            self.runs = RunTable(seeds, self.Gr * self.E, torch.device("cuda", torch.cuda.current_device()))
+            ou = {} if overrides is None else dict(ou_sigma=[float(c.std_dev) for c in self._run_confs],
+                                                   ou_theta=[float(c.theta) for c in self._run_confs])
+            self.runs = RunTable(seeds, self.Gr * self.E, torch.device("cuda", torch.cuda.current_device()), **ou)
             self.seeds = self.runs.seeds
         seed = int(getattr(conf, "random_seed", 1) if seed is None else seed)
         cap = int(conf.buffer_size if ring_capacity is None else ring_capacity)
@@ -194,7 +227,7 @@ class BatchedTrainer:
                                    reward_history=int(conf.weighted_window) if is_fed_enabled(conf) and conf.weighted_average_enabled else 0,
                                    runs=self.runs)
         self.pop = DDPGPopulation(self.G, self.M, conf, num_states=self.env.num_states, rows_per_agent=self.E * int(conf.batch_size),
-                                  seed=seed, precision=precision, seeds=self.seeds)
+                                  seed=seed, precision=precision, seeds=self.seeds, overrides=self.overrides)
         self.fed = None
         if is_fed_enabled(conf):
             from .server.federated import FederatedAggregator
@@ -288,17 +321,18 @@ class BatchedTrainer:
         groups = range(self.G) if run is None else range(run * self.Gr, (run + 1) * self.Gr)
         return [[r[g, m] for m in range(self.M)] for g in groups]
 
+    def run_config(self, s: int):
+        """Run s's effective configuration: a copy of conf with the run's random_seed and overrides applied."""
+        if not 0 <= s < self.S:
+            raise IndexError(f"run {s} outside {self.S} runs")
+        return copy.copy(self._run_confs[s])
+
     def reward_logs(self):
-        """One results.RewardLog per run, each on a copy of the configuration that carries the run's seed, so that generate_csvs
-        writes its files as ..._seed{k_s}.csv (the files the reference's accumr aggregates)."""
-        import copy
+        """One results.RewardLog per run, each on the run's configuration (run_config), so that generate_csvs writes its files as
+        ..._seed{k_s}.csv (the files the reference's accumr aggregates).  Runs that share a seed (a sweep over overrides) produce
+        files of the same names: write their logs into different directories."""
         from .results import RewardLog
-        logs = []
-        for k in (self.seeds if self.seeds is not None else [int(getattr(self.conf, "random_seed", 1))]):
-            conf = copy.copy(self.conf)
-            conf.random_seed = k
-            logs.append(RewardLog(conf, num_platoons=self.Gr, num_models=self.M))
-        return logs
+        return [RewardLog(self.run_config(s), num_platoons=self.Gr, num_models=self.M) for s in range(self.S)]
 
     def run_weights(self, s: int, group: int = 0):
         """Run s's weights: (actors, critics) with actors[m] / critics[m] the Keras `.weights` arrays of follower m of the run's group

@@ -31,7 +31,7 @@ extern "C" {
 
 #define AVD_MAX_FOLLOWERS 16
 #define AVD_RING_RECORD_FLOATS 10
-#define AVD_ABI_VERSION 4
+#define AVD_ABI_VERSION 5
 
 typedef enum avd_status {
     AVD_OK = 0,
@@ -88,12 +88,14 @@ typedef struct avd_clock {
  * m*P + p draws those of ring m*platoons_per_run + p mod platoons_per_run.  These are the keys a stand-alone run with
  * random_seed = seed[s] uses, so run s of the batch reproduces it.  The struct itself is host memory: every entry that takes
  * one checks runs * platoons_per_run == P and passes it to its kernels by value, so a captured CUDA graph replays it; the
- * seeds it points to live in device memory.                                                                              */
+ * seeds (and the optional per-run OU parameters) it points to live in device memory.                                     */
 typedef struct avd_runs {
     const uint64_t* seed;      /* [runs] DEVICE pointer: random_seed of every run                             */
     int64_t platoons_per_run;  /* >= 1                                                                       */
     int32_t runs;              /* >= 1                                                                       */
     int32_t reserved;
+    const float* ou_sigma;     /* [runs] nullable DEVICE pointer: OU std_dev of every run (NULL: avd_env_params.ou_sigma)  */
+    const float* ou_theta;     /* [runs] nullable DEVICE pointer: OU theta of every run (NULL: avd_env_params.ou_theta)    */
 } avd_runs;
 
 /* ---- buffers of one shard of platoons (all device pointers; nullable ones are marked) */
@@ -266,6 +268,8 @@ typedef struct avd_learn_io {
     int32_t precision;          /* 0: fp32 SIMT kernels (parity mode); 1: bf16 tcgen05 tensor-core GEMMs; 2: fp16 tcgen05;
                                    3: tcgen05 on three-way split bf16 operands, fp32-accurate (avd_gemm_bf16x3; DESIGN.md 4) */
     int32_t s_stride;           /* row pitch of s / s2 in floats: 4 for the replay gather output (avd_replay_gather), 0 = dims.ns */
+    const float* agent_hp;      /* [A][4] nullable DEVICE pointer: (gamma, actor_lr, critic_lr, tau) of every agent, used in place of
+                                   the scalars above with the same arithmetic (a sweep of hyperparameters in one batch); NULL: the scalars */
 } avd_learn_io;
 
 /* sizes of the flat parameter vectors: out4 = {actor_trainable, actor_total, critic_trainable, critic_total} */
@@ -301,12 +305,13 @@ int avd_adam_apply(float* params, int64_t param_stride, const float* grads, int6
 
 /* avd_adam_apply for both nets followed by avd_polyak_update of both targets (trainer.py:348-356), fused: one pass per net
  * applies Adam to the trainable prefix and the Polyak update to ALL weights, then both step counters advance.  Per-agent
- * gradient vectors have stride *_gstride (0 = one shared vector for every agent, as after FedAvg).                          */
+ * gradient vectors have stride *_gstride (0 = one shared vector for every agent, as after FedAvg).  agent_hp: nullable [A][4]
+ * device table laid out as avd_learn_io.agent_hp; agent a then takes its actor_lr, critic_lr and tau from row a.              */
 int avd_adam_polyak_apply2(float* actor, float* t_actor, int64_t actor_total, const float* actor_grad, int64_t actor_gstride,
                            float* actor_m, float* actor_v, int32_t* actor_step, int64_t actor_train, float actor_lr, float* critic,
                            float* t_critic, int64_t critic_total, const float* critic_grad, int64_t critic_gstride, float* critic_m,
                            float* critic_v, int32_t* critic_step, int64_t critic_train, float critic_lr, const uint8_t* apply_mask,
-                           int32_t A, float beta1, float beta2, float eps, float tau, void* stream);
+                           int32_t A, float beta1, float beta2, float eps, float tau, const float* agent_hp, void* stream);
 
 /* ddpgagent.update_target (agent/ddpgagent.py:44-55): target = tau*online + (1-tau)*target over n floats
  * per agent (ALL weights incl. BN statistics).                                                          */
@@ -390,6 +395,8 @@ typedef struct avd_fed_apply_io {
     const uint8_t* apply_mask;    /* [A] nullable                                                      */
     float* wsum_out;
     float actor_lr, critic_lr, beta1, beta2, eps, tau;
+    const float* agent_hp;        /* [A][4] nullable: per-agent (gamma, actor_lr, critic_lr, tau) as avd_learn_io.agent_hp; the
+                                     learning rates and tau are read.  A <= 25,600 without it, A <= 17,066 with it (shared memory) */
 } avd_fed_apply_io;
 int avd_fed_apply_gradients(const avd_fed_apply_io* io, void* stream);
 
