@@ -107,6 +107,30 @@ class FedApplyIO(C.Structure):
     ]
 
 
+class EpisodeState(C.Structure):
+    _fields_ = [("buffer_counter", C.c_int64), ("steps", C.c_int64), ("rounds", C.c_int64), ("learn_from", C.c_int64),
+                ("flags", C.c_int32), ("reserved", C.c_int32)]
+
+
+EPISODE_ARM, EPISODE_STEP, EPISODE_WEIGHTS = range(3)
+EPISODE_CONTINUE, EPISODE_ROUND, EPISODE_HAVE_WEIGHTS, EPISODE_HAVE_SUMS, EPISODE_LOCAL = 1, 2, 4, 8, 16
+
+
+class EpisodeIO(C.Structure):
+    _fields_ = [
+        ("mode", C.c_int32), ("runs", C.c_int32), ("platoons_per_run", C.c_int32), ("groups_per_run", C.c_int32), ("M", C.c_int32),
+        ("steps_per_episode", C.c_int32), ("global_break", C.c_int32), ("learn", C.c_int32), ("fed", C.c_int32), ("fed_gradients", C.c_int32),
+        ("fed_update_delay_steps", C.c_int32), ("fed_update_count", C.c_int32), ("fed_cutoff_episode", C.c_int32), ("weighted", C.c_int32),
+        ("weighted_window", C.c_int32), ("log_slots", C.c_int32), ("n_cont_handles", C.c_int32), ("has_round_handle", C.c_int32),
+        ("cont_handle", C.c_uint64 * 2), ("round_handle", C.c_uint64), ("has_local_handle", C.c_int32), ("reserved", C.c_int32),
+        ("local_handle", C.c_uint64), ("state", C.c_void_p),
+        ("left", C.c_void_p), ("ep", C.c_void_p), ("i", C.c_void_p), ("nrec", C.c_void_p), ("done", C.c_void_p), ("ep_reward", C.c_void_p),
+        ("reset_mask", C.c_void_p), ("learn_mask", C.c_void_p), ("round_mask", C.c_void_p), ("fed_apply_mask", C.c_void_p),
+        ("fed_w", C.c_void_p), ("round_w", C.c_void_p), ("wsum", C.c_void_p), ("log_reward", C.c_void_p), ("log_w", C.c_void_p),
+        ("log_wsum", C.c_void_p), ("log_len", C.c_void_p), ("log_weighted", C.c_void_p), ("log_pitch", C.c_int64),
+    ]
+
+
 class AvdError(RuntimeError):
     pass
 
@@ -170,6 +194,14 @@ SIGNATURES = {
     "avd_fed_apply_gradients": (C.c_int, [C.POINTER(FedApplyIO), C.c_void_p]),
     "avd_fed_broadcast": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_int64, C.c_int64,
                                     C.c_void_p, C.c_int64, C.c_void_p]),
+    "avd_episode_control": (C.c_int, [C.POINTER(EpisodeIO), C.c_void_p]),
+    "avd_loop_graph_create": (C.c_int, [C.POINTER(C.c_void_p), C.c_int32, C.POINTER(C.c_uint64)]),
+    "avd_loop_graph_capture_begin": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "avd_loop_graph_cond_begin": (C.c_int, [C.c_void_p, C.c_uint64, C.c_int32, C.c_void_p, C.c_void_p]),
+    "avd_loop_graph_cond_end": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "avd_loop_graph_capture_end": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "avd_loop_graph_launch": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "avd_loop_graph_destroy": (C.c_int, [C.c_void_p]),
     "avd_gemm_bf16": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64,
                                 C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p]),
     "avd_gemm_f16kind": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64,
@@ -199,7 +231,8 @@ def load():
         fn.restype, fn.argtypes = res, args
     if lib.avd_abi_version() != ABI_VERSION:
         raise AvdError(f"ABI mismatch: library {lib.avd_abi_version()} vs binding {ABI_VERSION}")
-    for which, st in enumerate((EnvParams, EnvIO, Clock, NetDims, LearnIO, PeerComm, FedApplyIO, Runs)):
+    for which, st in enumerate((EnvParams, EnvIO, Clock, NetDims, LearnIO, PeerComm, FedApplyIO, Runs, EpisodeIO,
+                                     EpisodeState)):
         if lib.avd_sizeof(which) != C.sizeof(st):
             raise AvdError(f"struct layout mismatch for {st.__name__}: C {lib.avd_sizeof(which)} vs ctypes {C.sizeof(st)}")
     _lib = lib

@@ -1774,31 +1774,47 @@ static int learn_prep(const avd_learn_io* io, const Pass& p, const Workspace& w,
     return AVD_OK;
 }
 
-// Side stream of the learn step (one per device, created on first use): the critic's unfold kernel -- 1216 small CTAs that need the
-// gradients of BOTH critic products but feed nothing before the optimiser -- runs there while the actor's forward pass occupies the
-// tensor pipe on the caller's stream (a 128-thread unfold CTA fits beside a persistent 220 KB CTA on the same SM).  Fork / join by
-// events, so a CUDA-graph capture of the caller's stream records the branch.
+// Side stream of the learn step (created on first use): the critic's unfold kernel -- 1216 small CTAs that need the gradients of
+// BOTH critic products but feed nothing before the optimiser -- runs there while the actor's forward pass occupies the tensor pipe on
+// the caller's stream (a 128-thread unfold CTA fits beside a persistent 220 KB CTA on the same SM).  Fork / join by events, so a
+// CUDA-graph capture of the caller's stream records the branch.  Every caller shares the first side stream, except that a side stream
+// joined into one capture stays in it until that capture ends: a caller that captures while it is so taken (the bodies of a
+// conditional graph are captured concurrently) takes another idle one, or one created for it; with none, it runs unbranched.
 struct SideStream {
+    cudaStream_t caller = nullptr;
     cudaStream_t s = nullptr;
     cudaEvent_t fork = nullptr, join = nullptr, fork2 = nullptr, join2 = nullptr, fork0 = nullptr, join0 = nullptr;
 };
+static bool side_idle(const SideStream& x) {
+    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+    return cudaStreamIsCapturing(x.s, &cs) == cudaSuccess && cs == cudaStreamCaptureStatusNone;
+}
 static SideStream* side_stream(cudaStream_t caller) {
-    static SideStream tab[64];
+    constexpr int kSlots = 8;
+    static SideStream tab[64][kSlots];
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return nullptr;
-    SideStream& x = tab[dev];
-    if (!x.s) {
-        // never create the stream / events while the caller's stream is being captured (a first call inside a capture runs unbranched)
-        cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-        if (cudaStreamIsCapturing(caller, &cs) != cudaSuccess || cs != cudaStreamCaptureStatusNone) return nullptr;
-        if (cudaStreamCreateWithFlags(&x.s, cudaStreamNonBlocking) != cudaSuccess || cudaEventCreateWithFlags(&x.fork, cudaEventDisableTiming) != cudaSuccess ||
-            cudaEventCreateWithFlags(&x.join, cudaEventDisableTiming) != cudaSuccess || cudaEventCreateWithFlags(&x.fork2, cudaEventDisableTiming) != cudaSuccess ||
-            cudaEventCreateWithFlags(&x.join2, cudaEventDisableTiming) != cudaSuccess || cudaEventCreateWithFlags(&x.fork0, cudaEventDisableTiming) != cudaSuccess ||
-            cudaEventCreateWithFlags(&x.join0, cudaEventDisableTiming) != cudaSuccess) {
-            x.s = nullptr;
-            return nullptr;
-        }
+    SideStream* t = tab[dev];
+    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+    if (cudaStreamIsCapturing(caller, &cs) != cudaSuccess) return nullptr;
+    const bool capturing = cs != cudaStreamCaptureStatusNone;
+    int n = 0;
+    while (n < kSlots && t[n].s) ++n;
+    if (n > 0 && !capturing) return &t[0];
+    for (int k = 0; k < n; ++k)
+        if (t[k].caller == caller || side_idle(t[k])) return &t[k];
+    // the first side stream is created outside a capture; further ones only for a capturing caller that found none idle
+    if (n == kSlots || (n == 0 && capturing)) return nullptr;
+    SideStream& x = t[n];
+    if (cudaStreamCreateWithFlags(&x.s, cudaStreamNonBlocking) != cudaSuccess || cudaEventCreateWithFlags(&x.fork, cudaEventDisableTiming) != cudaSuccess ||
+        cudaEventCreateWithFlags(&x.join, cudaEventDisableTiming) != cudaSuccess || cudaEventCreateWithFlags(&x.fork2, cudaEventDisableTiming) != cudaSuccess ||
+        cudaEventCreateWithFlags(&x.join2, cudaEventDisableTiming) != cudaSuccess || cudaEventCreateWithFlags(&x.fork0, cudaEventDisableTiming) != cudaSuccess ||
+        cudaEventCreateWithFlags(&x.join0, cudaEventDisableTiming) != cudaSuccess) {
+        cudaGetLastError();
+        x.s = nullptr;
+        return nullptr;
     }
+    x.caller = caller;
     return &x;
 }
 

@@ -91,6 +91,8 @@ extern "C" int64_t avd_sizeof(int which) {
         case 5: return (int64_t)sizeof(avd_peer_comm);
         case 6: return (int64_t)sizeof(avd_fed_apply_io);
         case 7: return (int64_t)sizeof(avd_runs);
+        case 8: return (int64_t)sizeof(avd_episode_io);
+        case 9: return (int64_t)sizeof(avd_episode_state);
         default: return -1;
     }
 }

@@ -243,6 +243,7 @@ class BatchedTrainer:
         self.fed_weights = None          # [systems][members] device tensor of the current episode's FedAvg weights, or None
         self._fed_w = None
         self.graph = None
+        self._dev = None                 # _DeviceEpisodes of run() on the device (trainers built with seeds)
         self.env.reset()
 
     @property
@@ -306,6 +307,9 @@ class BatchedTrainer:
             return None, None
         w = self.fed_weights.cpu().numpy().astype(np.float32)            # [systems][members]
         sums = self.fed.last_weight_sums.cpu().numpy().astype(np.float32)  # [systems]
+        return self._weight_lists(w, sums, run)
+
+    def _weight_lists(self, w, sums, run):
         groups = range(self.G) if run is None else range(run * self.Gr, (run + 1) * self.Gr)
         if self.fed.inter:      # systems = (follower m, run k) = m*S + k, members = the run's groups g'
             Gr, S = self.Gr, self.S
@@ -348,15 +352,15 @@ class BatchedTrainer:
         platoons (246-249), runs up to conf.steps_per_episode steps (251), ends early for everybody when ANY platoon reports a
         terminal state (268-269; `global_break=False` lets the other platoons finish) and appends the episodic rewards to
         `reward_log` (an avddpg_b200.results.RewardLog; trainer.py:273, 510-517).  A trainer built with seeds runs this loop per run
-        (see _run_runs) and takes `reward_logs`, one RewardLog per run (reward_logs()).  In-kernel auto-reset is switched off for the
-        duration, so episodes line up across platoons exactly like the reference's; one D2H read of the done flags per step is
-        the price (the free-running `step()` loop used by the benchmark never synchronises).  `any_terminal_group`: a
+        on the device (see _run_device) and takes `reward_logs`, one RewardLog per run (reward_logs()).  In-kernel auto-reset is
+        switched off for the duration, so episodes line up across platoons exactly like the reference's; without seeds one D2H read
+        of the done flags per step is the price (the free-running `step()` loop used by the benchmark never synchronises).  `any_terminal_group`: a
         torch.distributed group over which "any platoon terminal" is agreed (one 1-word all_reduce(MAX) per step) so that platoons
         sharded over several GPUs still end their episodes together (SURVEY.md section 8e: opt-in).  Returns the number of env steps."""
         if self.runs is not None:
             if reward_log is not None or any_terminal_group is not None:
                 raise ValueError("a trainer with runs takes reward_logs (one per run) and no any_terminal_group")
-            return self._run_runs(episodes, reward_logs, global_break, learn)
+            return self._run_device(episodes, reward_logs, global_break, learn)
         if reward_logs is not None:
             raise ValueError("reward_logs is for trainers built with seeds; pass reward_log")
         env, conf = self.env, self.conf
@@ -391,7 +395,7 @@ class BatchedTrainer:
         return steps
 
     def _run_runs(self, episodes: int, reward_logs, global_break: bool, learn: bool):
-        """run() for S runs: each run keeps its own episode index and step-in-episode counter, ends its episode when one of ITS
+        """The host reference of _run_device (one D2H read of the done flags and host-built masks per step).  run() for S runs: each run keeps its own episode index and step-in-episode counter, ends its episode when one of ITS
         platoons is terminal (global_break) or after steps_per_episode steps, then logs its rewards and resets only its own
         platoons.  FRL predicates and the weighting window are evaluated per run.  A run that has finished its episodes is frozen
         (its agents take no further update) while the others go on, so its weights end where the stand-alone run's do."""
@@ -485,6 +489,218 @@ class BatchedTrainer:
                 w.view(self.S, self.Gr, self.M)[k] = 1.0
         return w
 
+    # ------------------------------------------------------------------ the per-run episode loop on the device
+    RUN_LOG_SLOTS = 64          # episode records per run one graph launch of _run_device can log before the host drains them
+
+    def _run_device(self, episodes: int, reward_logs, global_break: bool, learn: bool):
+        """_run_runs with the loop on the device, bit-identical to it: after every step the episode controller (avd_episode_control)
+        ends episodes, logs them and writes the next step's masks, and a conditional CUDA graph repeats the step while runs have
+        episodes left.  Each graph launch runs until every run is done, a run's log is full (run_log_slots records) or, without
+        learning yet, the rings reach batch_size transitions; then the host synchronises once, drains the log into the reward logs
+        and, if needed, launches again.  The graphs (with and without learning, per starting state buffer) are built on first use
+        by capturing the same library calls _step_runs makes, and cached."""
+        env, conf, S = self.env, self.conf, self.S
+        if reward_logs is not None and len(reward_logs) != S:
+            raise ValueError(f"{len(reward_logs)} reward logs for {S} runs")
+        episodes = int(episodes)
+        self._run_ep, self._run_i = [self.episode] * S, [0] * S
+        self.run_episode_steps = [[] for _ in range(S)]
+        if episodes <= 0:
+            self.episode += episodes
+            return 0
+        L = self._device_episodes()
+        bs, lib = int(conf.batch_size), self.pop.lib
+        saved = env.auto_reset
+        env.auto_reset = False
+        self._in_run = True
+        steps = rounds = 0
+        try:
+            env.reset()
+            flags = (_lib.EPISODE_HAVE_WEIGHTS if self.fed_weights is not None else 0) | \
+                    (_lib.EPISODE_HAVE_SUMS if self.fed is not None and self.fed.last_weight_sums is not None else 0)
+            L.ctr.copy_(torch.tensor([[episodes] * S, [self.episode] * S, [0] * S, [0] * S], dtype=torch.int32))
+            L.state.copy_(torch.tensor([self.buffer_counter, 0, 0, 0, flags], dtype=torch.int64))
+            while True:
+                learning = learn and self.buffer_counter >= bs
+                L.state[3].fill_(bs if learn and not learning else _NEVER)
+                g = self._loop_graph(learning, global_break)
+                _lib.check(lib.avd_loop_graph_launch(g, _lib.current_stream()))
+                st, ctr = L.state.tolist(), L.ctr.tolist()          # the one synchronisation per launch
+                taken = st[1] - steps
+                steps, rounds = st[1], st[2]
+                self.buffer_counter = st[0]
+                self.step_in_run += taken
+                env._cur ^= taken & 1
+                self._drain_episode_log(ctr[3], reward_logs)
+                if not any(n > 0 for n in ctr[0]):
+                    break
+                if taken == 0 and not any(ctr[3]):
+                    raise RuntimeError("device episode loop made no progress")
+                L.ctr[3].zero_()
+            self._run_ep, self._run_i = ctr[1], ctr[2]
+            self.episode += episodes
+            if self.fed is not None:
+                self.fed.rounds += rounds
+                if st[4] & _lib.EPISODE_HAVE_SUMS:
+                    self.fed.last_weight_sums = self.fed.wsum
+                if st[4] & _lib.EPISODE_HAVE_WEIGHTS:
+                    self.fed_weights = self._fed_w
+        finally:
+            env.auto_reset = saved
+            self._in_run = False
+        return steps
+
+    def _drain_episode_log(self, nrec, reward_logs):
+        """The records of one launch, in each run's order: run_episode_steps and reward_logs[k].update_reward_list with the same values
+        _run_runs passes (episodic_rewards' expression on the logged ep_reward rows, frl_weight_lists' layout)."""
+        L, M, G, E, Gr = self._dev, self.M, self.G, self.E, self.Gr
+        J = max(nrec)
+        if J == 0:
+            return
+        lens, wrec = L.log_len[:J].tolist(), L.log_weighted[:J].tolist()
+        if reward_logs is not None:
+            n = M * self.P
+            rew = torch.stack([L.log_reward[j, :n].reshape(M, G, E).mean(dim=2).t().contiguous() for j in range(J)])
+            rew = rew.cpu().numpy().astype(np.float32)
+            if L.log_w is not None:
+                w, ws = L.log_w[:J].cpu().numpy().astype(np.float32), L.log_wsum[:J].cpu().numpy().astype(np.float32)
+        for k in range(self.S):
+            for j in range(nrec[k]):
+                self.run_episode_steps[k].append(lens[j][k])
+                if reward_logs is not None:
+                    fw, fws = self._weight_lists(w[j], ws[j], k) if wrec[j][k] else (None, None)
+                    reward_logs[k].update_reward_list([[rew[j, g, m] for m in range(M)] for g in range(k * Gr, (k + 1) * Gr)], fw, fws)
+
+    def _device_episodes(self):
+        slots = max(1, int(self.RUN_LOG_SLOTS))
+        if self._dev is None or self._dev.slots != slots:
+            self._free_loop_graphs()
+            self._dev = _DeviceEpisodes(self, slots)
+        return self._dev
+
+    def _episode_control(self, mode, learning=False, cont_handles=(), step_handles=(None, None)):
+        """One avd_episode_control launch; step_handles: the (round, local) IF handles of the next step, or None each."""
+        io = _lib.EpisodeIO.from_buffer_copy(self._dev.io)
+        io.mode, io.learn, io.n_cont_handles = mode, int(learning), len(cont_handles)
+        for j, h in enumerate(cont_handles):
+            io.cont_handle[j] = h
+        (rh, lh) = step_handles
+        io.has_round_handle, io.round_handle = int(rh is not None), rh or 0
+        io.has_local_handle, io.local_handle = int(lh is not None), lh or 0
+        _lib.check(self.pop.lib.avd_episode_control(C.byref(io), _lib.current_stream()))
+
+    def _loop_graph(self, learning: bool, global_break: bool):
+        """The cached loop graph for the current state buffer:
+            ARM -> WHILE (continue) { step A -> controller -> reset(mask)
+                                      IF (continue) { step B -> controller -> reset(mask) } }
+        with a learning step = act -> env step -> sample -> learn (gradients) -> IF (local) {Adam / Polyak} -> IF (round) {FRL round}.
+        Step B reads the buffer step A writes, so every iteration ends on the buffer it started from; a launch that ends after step A
+        leaves the other buffer current, and the next launch takes the graph built for that one."""
+        L, env, lib = self._dev, self.env, self.pop.lib
+        L.io.global_break = int(global_break)
+        key = (learning, global_break, env._cur)
+        if key in L.graphs:
+            return L.graphs[key]
+        rounds = learning and L.rounds
+        self._warm_loop(learning)
+        n = 2 + (2 if learning else 0) + (2 if rounds else 0)
+        hs = (C.c_uint64 * 6)()
+        g = C.c_void_p()
+        _lib.check(lib.avd_loop_graph_create(C.byref(g), n, hs))
+        h_while, h_b = int(hs[0]), int(hs[1])
+        la, lb = (int(hs[2]), int(hs[3])) if learning else (None, None)
+        ra, rb = (int(hs[4]), int(hs[5])) if rounds else (None, None)
+        st = L.streams
+        fed = self.fed
+        saved = (self.buffer_counter, self.step_in_run, env._cur, env._launches,
+                 None if fed is None else (fed.rounds, fed.last_weight_sums))
+
+        def body():
+            self._device_step(g, learning, (ra, la), st[2])
+            self._episode_control(_lib.EPISODE_STEP, learning, (h_while, h_b), (rb, lb))
+            env.reset(L.reset_mask)
+
+            def step_b():
+                self._device_step(g, learning, (rb, lb), st[3])
+                self._episode_control(_lib.EPISODE_STEP, learning, (h_while,), (ra, la))
+                env.reset(L.reset_mask)
+            self._graph_cond(g, h_b, 0, st[2], step_b)
+
+        try:
+            _lib.check(lib.avd_loop_graph_capture_begin(g, st[0].cuda_stream))
+            with torch.cuda.stream(st[0]):
+                self._episode_control(_lib.EPISODE_ARM, learning, (h_while,), (ra, la))
+                self._graph_cond(g, h_while, 1, st[1], body)
+            _lib.check(lib.avd_loop_graph_capture_end(g, st[0].cuda_stream))
+        except BaseException:
+            lib.avd_loop_graph_destroy(g)
+            raise
+        finally:      # capturing executes nothing on the device
+            self.buffer_counter, self.step_in_run, env._cur, env._launches = saved[:4]
+            if fed is not None:
+                fed.rounds, fed.last_weight_sums = saved[4]
+        L.graphs[key] = g
+        return g
+
+    def _graph_cond(self, g, handle, kind, child, body):
+        """body()'s launches, enqueued on the current stream's position, inside an IF (kind 0) / WHILE (1) node on `handle`."""
+        lib = self.pop.lib
+        _lib.check(lib.avd_loop_graph_cond_begin(g, handle, kind, torch.cuda.current_stream().cuda_stream, child.cuda_stream))
+        with torch.cuda.stream(child):
+            body()
+        _lib.check(lib.avd_loop_graph_cond_end(g, child.cuda_stream))
+
+    def _device_step(self, g, learning: bool, handles, child):
+        """_step_runs with its masks read from the device (the controller wrote them): the local Adam / Polyak step (the same launch
+        learn() makes with apply_updates) and the FRL round each behind an IF node, so a step without them costs nothing for them."""
+        env, pop, rings, L = self.env, self.pop, self.rings, self._dev
+        pop.act(env.native_state, env.action_mu, self.E)
+        env.step_native(explore=True, gen_exog=True, advance_clock=False)
+        rings.clock.advance(step=1, ring=1)
+        self.buffer_counter += 1
+        if learning:
+            s, a, r, s2 = rings.sample(advance_clock=True)
+            pop.learn(s, a, r, s2, apply_updates=False)
+            round_handle, local_handle = handles
+            self._graph_cond(g, local_handle, 0, child, lambda: pop.apply_gradients_and_soft_update(L.learn_mask))
+            if L.rounds:
+                self._graph_cond(g, round_handle, 0, child, self._device_round)
+        self.step_in_run += 1
+
+    def _device_round(self):
+        """The gradients round of _step_runs on the device masks: with weighting, _frl_weights_runs' weights (the runs before their
+        window take 1, which avd_fed_reduce2 sums exactly like its NULL weights)."""
+        L, conf, env = self._dev, self.conf, self.env
+        w = None
+        if L.round_w is not None:
+            _lib.check(self.pop.lib.avd_fed_weights_from_history(_lib.ptr(env.ep_hist), int(conf.weighted_window), self.M, self.G, self.E,
+                                                                 _lib.ptr(L.round_w), 0 if self.fed.inter else 1, _lib.current_stream()))
+            self._episode_control(_lib.EPISODE_WEIGHTS)
+            w = L.round_w
+        self.fed.aggregate_gradients(w, write_back=False, apply_mask=L.round_mask)
+
+    def _warm_loop(self, learning: bool):
+        """Allocate everything a captured step uses (nothing may allocate during capture) and create the learn step's side stream."""
+        pop, rings = self.pop, self.rings
+        pop.act(self.env.native_state, self.env.action_mu, self.E)     # the first step overwrites action_mu
+        if learning:
+            rings._alloc_sample_buffers()
+            pop.learn(rings.s, rings.a, rings.r, rings.s2, apply_updates=False)     # gradients and losses: every learn step rewrites them
+            if self.fed is not None:
+                self.fed._buffer(pop.actor.n_train, pop.critic.n_train)
+
+    def _free_loop_graphs(self):
+        if self._dev is not None:
+            for g in self._dev.graphs.values():
+                self.pop.lib.avd_loop_graph_destroy(g)
+            self._dev.graphs.clear()
+
+    def __del__(self):
+        try:
+            self._free_loop_graphs()
+        except Exception:       # noqa: BLE001 -- interpreter shutdown: the library may already be gone
+            pass
+
     def capture(self, warmup: int = 3):
         """Capture one full step (learn included) into a CUDA graph; afterwards `replay()` costs one launch.  The host-side FRL
         schedule is frozen into the graph, so capture is refused unless every step takes the same branch (fed_update_delay_steps == 1
@@ -526,6 +742,55 @@ class BatchedTrainer:
         spe = int(self.conf.steps_per_episode)
         if not self._in_run and self.step_in_episode >= spe:
             self.step_in_episode, self.episode = self.step_in_episode - spe, self.episode + 1
+
+
+_NEVER = (1 << 63) - 1      # avd_episode_state.learn_from when no prefix stop applies
+
+
+class _DeviceEpisodes:
+    """Device state of BatchedTrainer._run_device: the episode controller's counters, masks and log (avd_episode_io) and the
+    cached loop graphs."""
+
+    def __init__(self, tr: "BatchedTrainer", slots: int):
+        dev, conf, fed = tr.pop.device, tr.conf, tr.fed
+        S, P, A, M = tr.S, tr.P, tr.pop.A, tr.M
+        u8, i32, f32 = (dict(dtype=t, device=dev) for t in (torch.uint8, torch.int32, torch.float32))
+        self.slots = slots
+        self.state = torch.zeros(5, dtype=torch.int64, device=dev)            # avd_episode_state (flags in the low half of word 4)
+        self.ctr = torch.zeros(4, S, **i32)                                    # left, ep, i, nrec
+        self.reset_mask, self.learn_mask = torch.zeros(P, **u8), torch.zeros(A, **u8)
+        self.round_mask = None if fed is None else torch.zeros(A, **u8)
+        self.rounds = fed is not None and is_fed_enabled(conf) and bool(conf.fed_enabled) and is_gradient_updates_enabled(conf)
+        weighted = fed is not None and bool(conf.weighted_average_enabled)
+        if weighted and tr._fed_w is None:
+            tr._fed_w = torch.zeros(fed.n_systems, fed.n_members, **f32)
+        self.round_w = torch.zeros(fed.n_systems, fed.n_members, **f32) if weighted else None
+        pitch = (M * P + 127) // 128 * 128      # every record starts 512-byte aligned, like env.ep_reward (same reduction in mean())
+        self.log_reward = torch.zeros(slots, pitch, **f32)
+        self.log_w = torch.zeros(slots, fed.n_systems, fed.n_members, **f32) if weighted else None
+        self.log_wsum = torch.zeros(slots, fed.n_systems, **f32) if weighted else None
+        self.log_len, self.log_weighted = torch.zeros(slots, S, **i32), torch.zeros(slots, S, **i32)
+        self.streams = [torch.cuda.Stream() for _ in range(4)]                # capture: top level, loop body, step B / round, round in B
+        self.graphs = {}
+        io = self.io = _lib.EpisodeIO()
+        io.runs, io.platoons_per_run, io.groups_per_run, io.M = S, tr.Gr * tr.E, tr.Gr, M
+        io.steps_per_episode, io.global_break = int(conf.steps_per_episode), 1
+        io.fed = 0 if fed is None else (1 if fed.inter else 2)
+        io.fed_gradients = int(self.rounds)
+        if fed is not None:
+            io.fed_update_delay_steps, io.fed_update_count = int(conf.fed_update_delay_steps), int(conf.fed_update_count)
+            io.fed_cutoff_episode = max(-(1 << 31), min(int(conf.fed_cutoff_episode), (1 << 31) - 1))
+        io.weighted, io.weighted_window = int(bool(conf.weighted_average_enabled)), int(conf.weighted_window)
+        io.log_slots = slots
+        io.state = self.state.data_ptr()
+        io.left, io.ep, io.i, io.nrec = (self.ctr[j].data_ptr() for j in range(4))
+        io.done, io.ep_reward = tr.env._done.data_ptr(), tr.env.ep_reward.data_ptr()
+        io.reset_mask, io.learn_mask = self.reset_mask.data_ptr(), self.learn_mask.data_ptr()
+        ptr = lambda t: None if t is None else t.data_ptr()
+        io.round_mask, io.fed_apply_mask = ptr(self.round_mask), ptr(None if fed is None else fed.apply_mask)
+        io.fed_w, io.round_w, io.wsum = ptr(tr._fed_w if weighted else None), ptr(self.round_w), ptr(None if fed is None else fed.wsum)
+        io.log_reward, io.log_w, io.log_wsum = self.log_reward.data_ptr(), ptr(self.log_w), ptr(self.log_wsum)
+        io.log_len, io.log_weighted, io.log_pitch = self.log_len.data_ptr(), self.log_weighted.data_ptr(), pitch
 
 
 class HostStepPipeline:

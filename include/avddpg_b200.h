@@ -148,7 +148,7 @@ const char* avd_last_error(void);
  * callers difference it around a region, e.g. bench.py's "gpu_launches" */
 int64_t avd_kernel_launches(void);
 /* sizeof of the ABI structs as compiled (0 avd_env_params, 1 avd_env_io, 2 avd_clock, 3 avd_net_dims, 4 avd_learn_io,
- * 5 avd_peer_comm, 6 avd_fed_apply_io, 7 avd_runs): bindings assert their own layout against these at load time. */
+ * 5 avd_peer_comm, 6 avd_fed_apply_io, 7 avd_runs, 8 avd_episode_io, 9 avd_episode_state): bindings assert their own layout against these at load time. */
 int64_t avd_sizeof(int which);
 /* SM count, compute capability major*10+minor of the current device; AVD_ERR_NO_DEVICE if none */
 int avd_device_info(int* sm_count, int* cc, int64_t* total_mem);
@@ -404,6 +404,91 @@ int avd_fed_apply_gradients(const avd_fed_apply_io* io, void* stream);
 int avd_fed_broadcast(float* out, int64_t out_pitch, const float* in, int64_t in_pitch, int32_t n_systems,
                       int32_t n_members, int64_t member_stride_s, int64_t member_stride_x, const uint8_t* apply_mask,
                       int64_t n, void* stream);
+
+/* ---- per-run episode loop on the device (BatchedTrainer.run of a trainer built with seeds) ---------------------------------
+ * The episode controller runs once per training step, after the step's learn / FRL launches and before the platoon reset, and does
+ * for every run k of a batch of `runs` x `platoons_per_run` platoons what the host loop does (workers/trainer.py:251-273 per run):
+ * with global_break, bit 0 of done[] over the run's platoons; i[k] += 1; the episode ends when a platoon is terminal or i[k] reaches
+ * steps_per_episode; then a log record is appended (the run's raw ep_reward columns, the episode length and, once the run is past its
+ * weighting window, the run's FedAvg weights and weight sums), ep[k] += 1, i[k] = 0, left[k] -= 1, and the run's platoons are marked
+ * in reset_mask[P] if episodes are left.  Finally the masks of the NEXT step are written from the FRL predicates of (ep[k], i[k])
+ * (trainer.py:631-695): learn_mask[A] (local Adam / Polyak update: run active and not on an FRL step) and round_mask[A] (gradients
+ * round, ANDed with fed_apply_mask).  Runs with no episodes left are frozen (all masks 0).  Agent a = m*G + k*Gr + g', platoon
+ * p = k*platoons_per_run + p'.  All counters and masks are device memory, so the entry works eagerly as well as inside a graph.  */
+enum {
+    AVD_EPISODE_ARM = 0,       /* end nothing: write the masks and flags of the next step from the counters as they are              */
+    AVD_EPISODE_STEP = 1,      /* after a step: advance the counters, end episodes, log, then write the next step's masks            */
+    AVD_EPISODE_WEIGHTS = 2    /* inside a weighted gradients round, after avd_fed_weights_from_history(out = round_w): rows of runs
+                                  before their weighting window become 1 (a plain mean); unless every run is such a run, round_w is
+                                  also copied to fed_w (the weights the log records) and AVD_EPISODE_HAVE_WEIGHTS is set            */
+};
+enum {                         /* avd_episode_state.flags                                                                              */
+    AVD_EPISODE_CONTINUE = 1,  /* some run has episodes left, no such run has a full log, buffer_counter < learn_from               */
+    AVD_EPISODE_ROUND = 2,     /* the next step takes a gradients round (some run's round_mask row is set)                          */
+    AVD_EPISODE_HAVE_WEIGHTS = 4, /* a weighted round has happened: fed_w holds FedAvg weights                                        */
+    AVD_EPISODE_HAVE_SUMS = 8, /* a round has happened: wsum holds weight sums                                                        */
+    AVD_EPISODE_LOCAL = 16     /* the next step takes a local update (some run's learn_mask row is set)                             */
+};
+typedef struct avd_episode_state {   /* DEVICE memory */
+    int64_t buffer_counter;    /* transitions added per ring (BatchedTrainer.buffer_counter); += 1 per STEP                        */
+    int64_t steps;             /* STEP launches since the caller zeroed it                                                          */
+    int64_t rounds;            /* gradients rounds taken since the caller zeroed it (counted by the STEP after the round)         */
+    int64_t learn_from;        /* CONTINUE needs buffer_counter < learn_from (a prefix without learning stops at batch_size)       */
+    int32_t flags;             /* AVD_EPISODE_*                                                                                      */
+    int32_t reserved;
+} avd_episode_state;
+typedef struct avd_episode_io {
+    int32_t mode;              /* AVD_EPISODE_ARM / STEP / WEIGHTS                                                                  */
+    int32_t runs, platoons_per_run, groups_per_run, M;
+    int32_t steps_per_episode;
+    int32_t global_break;      /* 1: a terminal platoon ends its run's episode                                                      */
+    int32_t learn;             /* 1: the steps learn, so a set AVD_EPISODE_ROUND flag means the step took a round                  */
+    int32_t fed;               /* 0 no FRL, 1 interfrl (systems m*runs + k, members g'), 2 intrafrl (systems g, members m)          */
+    int32_t fed_gradients;     /* FRL enabled with aggregation_method gradients                                                     */
+    int32_t fed_update_delay_steps, fed_update_count, fed_cutoff_episode;   /* >= 1, >= 1, any                                     */
+    int32_t weighted;          /* weighted_average_enabled                                                                          */
+    int32_t weighted_window;
+    int32_t log_slots;         /* records per run the log holds                                                                     */
+    int32_t n_cont_handles;    /* 0..2: conditional handles set to CONTINUE at the end of an ARM / STEP launch (0 outside a graph) */
+    int32_t has_round_handle;  /* 1: round_handle is set to CONTINUE && ROUND                                                       */
+    uint64_t cont_handle[2];   /* cudaGraphConditionalHandle values                                                                 */
+    uint64_t round_handle;
+    int32_t has_local_handle;  /* 1: local_handle is set to CONTINUE && LOCAL                                                       */
+    int32_t reserved;
+    uint64_t local_handle;
+    avd_episode_state* state;
+    int32_t *left, *ep, *i, *nrec;          /* [runs] episodes left, episode index, step in episode, log records held               */
+    const uint8_t* done;       /* [P] avd_env_io.done                                                                               */
+    const float* ep_reward;    /* [M][P] avd_env_io.ep_reward                                                                       */
+    uint8_t* reset_mask;       /* [P]                                                                                               */
+    uint8_t* learn_mask;       /* [A]                                                                                               */
+    uint8_t* round_mask;       /* [A] nullable without FRL                                                                          */
+    const uint8_t* fed_apply_mask; /* [A] nullable (intrafrl directional averaging)                                                 */
+    float* fed_w;              /* [systems][members] nullable without weighting: the last weighted round's FedAvg weights           */
+    float* round_w;            /* [systems][members] WEIGHTS: this round's weights                                                  */
+    const float* wsum;         /* [systems] nullable without FRL: weight sums of the last round (avd_fed_apply_io.wsum_out)          */
+    float* log_reward;         /* [log_slots][log_pitch >= M*P]: record j of run k in the run's columns of [M][P] row j            */
+    float* log_w;              /* [log_slots][systems][members] nullable without weighting                                          */
+    float* log_wsum;           /* [log_slots][systems]          nullable without weighting                                          */
+    int32_t* log_len;          /* [log_slots][runs] episode length                                                                  */
+    int32_t* log_weighted;     /* [log_slots][runs] 1: the record holds weights                                                     */
+    int64_t log_pitch;         /* floats from one log_reward record to the next                                                     */
+} avd_episode_io;
+int avd_episode_control(const avd_episode_io* io, void* stream);
+
+/* A CUDA graph with conditional nodes, built by stream capture: capture_begin captures `stream` into the graph's top level;
+ * cond_begin adds an IF (type 0) or WHILE (type 1) node on `handle` at the current position of the capturing `parent` stream and
+ * captures `child` (an idle stream) into its body until cond_end; capture_end ends the top-level capture and instantiates.  The
+ * handles (created with the graph, no default value) are set by kernels in the graph: avd_episode_control.  A failed build leaves
+ * no stream capturing once avd_loop_graph_destroy has run.                                                                       */
+typedef struct avd_loop_graph avd_loop_graph;
+int avd_loop_graph_create(avd_loop_graph** out, int32_t n_handles, uint64_t* handles_out);
+int avd_loop_graph_capture_begin(avd_loop_graph* g, void* stream);
+int avd_loop_graph_cond_begin(avd_loop_graph* g, uint64_t handle, int32_t type, void* parent, void* child);
+int avd_loop_graph_cond_end(avd_loop_graph* g, void* child);
+int avd_loop_graph_capture_end(avd_loop_graph* g, void* stream);
+int avd_loop_graph_launch(avd_loop_graph* g, void* stream);   /* counts as one launch in avd_kernel_launches */
+int avd_loop_graph_destroy(avd_loop_graph* g);
 
 /* ---- tensor-core GEMM (tcgen05 + TMEM + TMA), the building block of precision = 1 ------------------
  * C[b] (fp32, M x N, row pitch ldc) = / += op(A[b]) op(B[b]) with bf16 operands and fp32 accumulation.
